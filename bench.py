@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- rollout-steps/s of the batched MPC rollout hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload mppi_ode_1m|...]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload mppi_ode_1m|...] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 Own arm ("ours"): one step = one MPPI tick (sample -> rollout -> cost -> softmin update) over the configured rollout
@@ -14,8 +14,10 @@ in-kernel Philox noise, sharded by sample over the N GPUs ("strong" scaling: the
              < 1 byte of HBM traffic per rollout-step), algorithmic 80 FLOP per rollout-step (DESIGN.md).
   cpu_baseline : the oracle port of the reference's MPPI (torch-CPU fp32, all host threads) on a bounded sample.
 Reference arm (--impl reference): the reference's UNMODIFIED optimizer file through controller_mpc and the oracle/refharness shims
-where the checkout (/root/reference) exists, the oracle port on the GPU box where it does not (cpu_baseline.kind says which), timed on
-the host cores, K steps of a bounded sample each; under torchrun rank 0 alone runs it.
+where CTK_REFERENCE names a checkout of the original Control_Toolkit, the oracle port where it does not (cpu_baseline.kind says which),
+timed on the host cores, K steps of a bounded sample each; under torchrun rank 0 alone runs it.
+--dump-outputs DIR (own arm): after the K timed ticks, rank 0 writes what the last of them computed to DIR/<name>.npy (see
+timed_path_outputs).  Inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -188,9 +190,9 @@ def cpu_mppi_rate(workload, n_sample, ticks, warm=1):
 
 
 def cpu_reference_rate(workload, n_sample, ticks, warm=1):
-    """rollout-steps/s of the reference's UNMODIFIED optimizer file (imported from /root/reference through the test-only shims of
-    oracle/refharness: SI_Toolkit stand-in with the pinned spec predictor / cost, torch-CPU fp32).  Only where the reference checkout
-    exists (the build container); the GPU box has no /root/reference and times the oracle port instead."""
+    """rollout-steps/s of the reference's UNMODIFIED optimizer file (imported from that checkout through the test-only shims of
+    oracle/refharness: SI_Toolkit stand-in with the pinned spec predictor / cost, torch-CPU fp32).  Only where CTK_REFERENCE names a
+    checkout of the original Control_Toolkit; without one the reference arm times the oracle port instead."""
     import copy
     import logging
     import torch
@@ -265,6 +267,41 @@ def run_reference_arm(args):
 
 
 # ------------------------------------------------------------------------------------------------------------------
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_LOG_ROWS = 4096  # rollouts of the logged controls / trajectories written with logging on (the whole log is GBs at 10^6 rollouts)
+
+
+def timed_path_outputs(opt, u_dev, logging_on) -> dict:
+    """What the last timed tick computed, as a caller of the tick receives it: the control u, the optimizer state the next tick
+    starts from (get_state(): MPPI u_nom, CEM mean and stdev, RPGD the population and its Adam moments) and, with logging on, the
+    cost of every rollout plus the logged controls and trajectories of a fixed, seeded sample of DUMP_LOG_ROWS rollouts.  u and the
+    state are the same on every shard; the logs are this rank's shard of the population (rank 0's when several GPUs run).  The logs
+    come to the host whole, as optimizer.step hands them over, once, after the timed passes."""
+    nu = int(opt.num_control_inputs)
+    out = {"u": u_dev[:nu].cpu().numpy()}
+    for k, v in opt.get_state().items():
+        v = np.asarray(v)
+        out[f"state_{k}"] = v if v.dtype == np.float32 else v.astype(np.float64)
+    if logging_on:
+        n = opt._n_local
+        opt._collect_rollout_logs(n)
+        rows = np.sort(np.random.default_rng(0).choice(n, min(n, DUMP_LOG_ROWS), replace=False))
+        out["J_logged"] = np.array(opt.logging_values["J_logged"], np.float32)
+        out["log_rows"] = rows.astype(np.float64)
+        for k in ("Q_logged", "rollout_trajectories_logged"):
+            out[f"{k}_rows"] = np.array(opt.logging_values[k][rows], np.float32)
+    return out
+
+
+def write_outputs(directory, arrays: dict) -> None:
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"outputs to dump take {total} bytes, more than the {DUMP_LIMIT_BYTES} allowed")
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -286,7 +323,7 @@ def run_ours(args):
                                   mlp_engine=args.mlp_engine, logging=logging_on)
     opt = ctrl.optimizer
     plan.attach(opt, lib)  # handle runs on torch's current stream (events + NCCL ordering)
-    K, W = max(args.steps, 1), max(args.warmup, 3)  # timing rule: at least three untimed warm-up ticks (the line reports the W used)
+    K, W = args.steps, max(args.warmup, 3)  # timing rule: at least three untimed warm-up ticks (the line reports the W used)
     states = torch.from_numpy(synthetic_states(K + W, 0)).to(dev)
     u_dev = torch.zeros(4, dtype=torch.float32, device=dev)
     flush = torch.empty(256 * 1024 * 1024, dtype=torch.uint8, device=dev)  # > 126 MB L2
@@ -329,6 +366,8 @@ def run_ours(args):
     barrier()
     wall = time.perf_counter() - wall0
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, timed_path_outputs(opt, u_dev, logging_on))
     per_tick_ms = [a.elapsed_time(b) for a, b in ev]
     launches = opt.gpu_launches - launches0 - n_align[0]  # kernels of the K timed ticks
     # ---- second pass, same ticks: CUDA events around the rollout kernel only (roofline.achieved); kept out of the pass
@@ -361,18 +400,17 @@ def run_ours(args):
     #      difference to ms_per_step is the event-pair / launch gap and the cold prologue, not work. ----
     pipelined_ms = None
     if fused:
-        Kp = max(K, 50)
-        st_rep = states[W:W + K].repeat((Kp + K - 1) // K, 1)[:Kp].contiguous()
-        u_rep = torch.zeros(Kp, 2, dtype=torch.float32, device=dev)
-        L.check(lib.ctk_step_device_n(opt._h, C.c_void_p(st_rep.data_ptr()), 6, C.c_void_p(u_rep.data_ptr()), 2, min(Kp, 10)))  # warm
+        st_rep = states[W:W + K].contiguous()
+        u_rep = torch.zeros(K, 2, dtype=torch.float32, device=dev)
+        L.check(lib.ctk_step_device_n(opt._h, C.c_void_p(st_rep.data_ptr()), 6, C.c_void_p(u_rep.data_ptr()), 2, min(K, 10)))  # warm
         barrier()
         align()
         p0, p1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         p0.record()
-        L.check(lib.ctk_step_device_n(opt._h, C.c_void_p(st_rep.data_ptr()), 6, C.c_void_p(u_rep.data_ptr()), 2, Kp))
+        L.check(lib.ctk_step_device_n(opt._h, C.c_void_p(st_rep.data_ptr()), 6, C.c_void_p(u_rep.data_ptr()), 2, K))
         p1.record()
         barrier()
-        pm = torch.tensor([p0.elapsed_time(p1) / Kp], dtype=torch.float64, device=dev)
+        pm = torch.tensor([p0.elapsed_time(p1) / K], dtype=torch.float64, device=dev)
         if world > 1:
             dist.all_reduce(pm, op=dist.ReduceOp.MAX)
         pipelined_ms = float(pm.item())
@@ -518,7 +556,7 @@ def run_ours(args):
                         "p50_step_latency_ms": statistics.median(lat) * 1e3, "api": api_name},
                 "pipelined": (None if pipelined_ms is None else
                               {"value": N * H * passes / (pipelined_ms * 1e-3), "unit": "rollout-steps/s", "ms_per_step": pipelined_ms,
-                               "ticks": max(K, 50), "how": "ticks back to back inside ONE CUDA-event pair (ctk_step_device_n), no per-tick L2 flush, "
+                               "ticks": K, "how": "ticks back to back inside ONE CUDA-event pair (ctk_step_device_n), no per-tick L2 flush, "
                                                            "max over ranks; consecutive ticks overlap through programmatic dependent launch"}),
                 "gpu_launches": int(launches), "roofline": roofline, "cpu_baseline": cpu, "clocks": clocks,
                 "wall_s_timed_region": wall}
@@ -538,7 +576,13 @@ def main():
     ap.add_argument("--rollouts", type=int, default=None, help="override the global rollout count")
     ap.add_argument("--mlp-engine", default="tcgen05", choices=["simt", "tcgen05", "tcgen05_bf16", "tcgen05_fast"], help="MLP predictor engine (mppi_mlp_c4 workload)")
     ap.add_argument("--cpu-sample", type=int, default=250_000, help="rollouts per CPU-baseline tick (bounded sample; C1-C4 run at their full size)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed tick computed to DIR/<name>.npy (own arm, rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

@@ -1,11 +1,11 @@
 """oracle.gen_golden -- TEST INFRASTRUCTURE ONLY.  Generates tests/golden/*.npz.
 
 Runs the reference's UNMODIFIED ``controller_mpc`` + ``optimizer_mppi`` / ``optimizer_rpgd`` /
-``optimizer_cem_tf`` / ``optimizer_random_action_tf`` files (imported from /root/reference through the shims in oracle/refharness) on
+``optimizer_cem_tf`` / ``optimizer_random_action_tf`` files (imported from the checkout CTK_REFERENCE names, through the shims in oracle/refharness) on
 torch-CPU fp32 with the build's pinned predictor / cost spec and INJECTED noise, and stores inputs +
-outputs as small fixtures.  Must be run in the build container (needs /root/reference):
+outputs as small fixtures.  Needs a checkout of the original Control_Toolkit:
 
-    python -m oracle.gen_golden            # writes tests/golden/*.npz
+    CTK_REFERENCE=<checkout> python -m oracle.gen_golden            # writes tests/golden/*.npz
     python -m oracle.gen_golden --out DIR mppi_c1_n64 rpgd_c3   # some cases, into another directory
 
 Each fixture holds: the case config (json), the per-tick states, the noise seed (noise is regenerated from

@@ -1,6 +1,6 @@
-"""TEST-ONLY driver (run as a subprocess by tests/test_dropin_reference.py; needs /root/reference, i.e. the build container).
+"""TEST-ONLY driver (run as a subprocess by tests/test_dropin_reference.py; needs the Control_Toolkit checkout named by CTK_REFERENCE).
 
-Enters the refharness workspace (``Control_Toolkit -> /root/reference`` + a working ``Control_Toolkit_ASF``), copies the shim files of
+Enters the refharness workspace (``Control_Toolkit -> $CTK_REFERENCE`` + a working ``Control_Toolkit_ASF``), copies the shim files of
 ``integration/Control_Toolkit_ASF/Optimizers/`` next to the application's optimizers exactly as INTEGRATION.md section 2 tells a
 maintainer to, and drives the reference's UNMODIFIED ``controller_mpc`` (reference Controllers/controller_mpc.py:24-109) with
 ``optimizer_name="<name>-b200"``: discovery by file / class name (others/globals_and_utils.py:103-133), construction with the

@@ -20,6 +20,18 @@ def golden_names(prefix=""):
     return sorted(f[:-4] for f in os.listdir(GOLDEN) if f.endswith(".npz") and f.startswith(prefix))
 
 
+def load_interpolation_weights():
+    """{(horizon, period): W [n_ind, horizon] float32}: the reference Interpolator's weights over the sweep of
+    tests/dropin/drive_reference_interpolator.py, stored in tests/golden/interpolator/weights_sweep.npz."""
+    z = np.load(os.path.join(GOLDEN, "interpolator", "weights_sweep.npz"))
+    out, off = {}, 0
+    for H, period, n_ind in z["geometry"].tolist():
+        out[(H, period)] = z["weights"][off:off + n_ind * H].reshape(n_ind, H)
+        off += n_ind * H
+    assert off == z["weights"].size
+    return out
+
+
 def load_golden(name):
     z = np.load(os.path.join(GOLDEN, name + ".npz"))
     meta = json.loads(str(z["config"]))

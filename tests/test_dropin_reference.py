@@ -1,8 +1,8 @@
 """CPU test of the drop-in claim ("nothing in the reference has to be modified", INTEGRATION.md section 2): the reference's own
 UNMODIFIED controller_mpc discovers, constructs and configures the B200 plugins through the shim files of integration/ and gets all
 the way to ``ctk_create`` -- which, on a box without a GPU, is the first thing that can fail (BackendUnavailable: no CPU fallback).
-Needs /root/reference (the build container); skipped on the GPU box, where tests/test_gpu_parity.py drives the same plugins through
-the repo's controller_mpc mirror.  Reference: Controllers/controller_mpc.py:56-89, others/globals_and_utils.py:103-133."""
+Needs a checkout of the original Control_Toolkit named by CTK_REFERENCE and skips without one; tests/test_gpu_parity.py drives the
+same plugins through the repo's controller_mpc mirror.  Reference: Controllers/controller_mpc.py:56-89, others/globals_and_utils.py:103-133."""
 import json
 import os
 import subprocess
@@ -10,11 +10,12 @@ import sys
 
 import pytest
 
+from oracle.refharness.workspace import reference_available
+
 HERE = os.path.dirname(os.path.abspath(__file__))
-REFERENCE = os.environ.get("CTK_REFERENCE", "/root/reference")
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REFERENCE, "Optimizers")), reason="needs the reference checkout (build container only)")
+@pytest.mark.skipif(not reference_available(), reason="needs a Control_Toolkit checkout: set CTK_REFERENCE to its path")
 def test_reference_controller_mpc_reaches_ctk_create_through_the_shims():
     r = subprocess.run([sys.executable, os.path.join(HERE, "dropin", "drive_reference_controller.py")], capture_output=True, text=True,
                        timeout=600)

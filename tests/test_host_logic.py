@@ -1,11 +1,15 @@
 """CPU tests of the host-side logic of the plugin layer: registry / naming / config plumbing, parameter derivation
 (independently written in control_toolkit_b200/specs.py and oracle/spec.py), shard geometry."""
 import math
+import os
 
 import numpy as np
 import pytest
 
 from oracle import spec as ospec
+from oracle.refharness.workspace import REFERENCE, reference_has
+
+TEMPLATE_YAML = os.path.join("Control_Toolkit_ASF_Template", "config_optimizers.yml")
 
 
 def test_ode_and_cost_constants_agree_with_oracle_spec():
@@ -157,8 +161,7 @@ def test_environment_registry_second_environment_and_recurrent_predictor():
         specs.GRUSpec(**{**{k: getattr(a, k) for k in a._KEYS}, "W3": np.zeros((32, 4), np.float32)})
 
 
-@pytest.mark.skipif(not __import__("os").path.isfile("/root/reference/Control_Toolkit_ASF_Template/config_optimizers.yml"),
-                    reason="needs the reference checkout (build container only)")
+@pytest.mark.skipif(not reference_has(TEMPLATE_YAML), reason="needs a Control_Toolkit checkout: set CTK_REFERENCE to its path")
 @pytest.mark.parametrize("key", ["mppi", "cem-tf", "random-action-tf", "gradient-tf", "cem-naive-grad-tf", "cem-grad-bharadhwaj-tf"])
 def test_reference_template_yaml_blocks_feed_the_plugins_unchanged(key):
     """The reference's OWN template blocks (Control_Toolkit_ASF_Template/config_optimizers.yml) go into the plugin constructors exactly as
@@ -170,7 +173,7 @@ def test_reference_template_yaml_blocks_feed_the_plugins_unchanged(key):
     import control_toolkit_b200 as ctk
     from control_toolkit_b200._lib import BackendUnavailable
     from control_toolkit_b200.Controllers.controller_mpc import controller_mpc
-    with open("/root/reference/Control_Toolkit_ASF_Template/config_optimizers.yml") as f:
+    with open(os.path.join(REFERENCE, TEMPLATE_YAML)) as f:
         block = dict(yaml.safe_load(f)[key])
     block["mpc_timestep"] = 0.02
     predictor = "ODE"

@@ -9,6 +9,7 @@ import numpy as np
 import pytest
 
 from helpers import golden_names, load_golden, make_oracle, maybe_reset_oracle, rel_err, replay
+from oracle.refharness.workspace import reference_available, reference_has
 
 TOL = 2e-6
 
@@ -217,7 +218,7 @@ REGEN_CASES = ["mppi_c1_n64", "mppi_h43_p10_n64", "mppi_gru_n256", "mppi_dubins_
                "gradient_warmup_n33", "gradcem_bharadhwaj_n32", "random_action_n512"]
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/Optimizers"), reason="needs the reference checkout (build container only)")
+@pytest.mark.skipif(not reference_available(), reason="needs a Control_Toolkit checkout: set CTK_REFERENCE to its path")
 def test_committed_fixtures_are_what_the_unmodified_reference_produces(tmp_path):
     """Pinning of the fixtures themselves: re-run the reference's UNMODIFIED optimizer files (oracle/gen_golden.py, in a process of
     its own because the harness changes the working directory and the module table) and compare every array of a committed fixture
@@ -256,11 +257,22 @@ def test_committed_fixtures_are_what_the_unmodified_reference_produces(tmp_path)
         warnings.warn(f"regenerated fixtures equal the committed ones to tolerance, not bit for bit (other host CPU?): {not_bitwise[:5]}")
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/others"), reason="needs the reference checkout (build container only)")
 def test_interpolation_matrix_equals_the_unmodified_reference_interpolator():
-    """a2 (others/Interpolator.py:53-84,97-106) pinned directly: oracle.mppi.interpolation_matrix against the reference class over 1152
-    geometries (H = 1 .. 101, period = 1 .. 12, one and two control inputs; includes H < period, period 1, and H - 1 a multiple of the
-    period, where the last-point quirk shows): weights bit for bit, applied interpolation to one ulp."""
+    """a2 (others/Interpolator.py:53-84,97-106) pinned directly: oracle.mppi.interpolation_matrix against the reference class's weights
+    over 1152 geometries (H = 1 .. 101, period = 1 .. 12, one and two control inputs; includes H < period, period 1, and H - 1 a multiple
+    of the period, where the last-point quirk shows), bit for bit.  The weights do not depend on the number of control inputs, so
+    tests/golden/interpolator/weights_sweep.npz stores them once per (H, period).  They were written from oracle.mppi.interpolation_matrix
+    as it stands since the live check below found it equal to the reference Interpolator bit for bit over this sweep;
+    ``drive_reference_interpolator.py --write`` rewrites them from the reference itself.  With CTK_REFERENCE naming a checkout, the
+    reference class is also run live: its weights against the stored ones and the oracle's, its applied interpolation to one ulp."""
+    from helpers import load_interpolation_weights
+    from oracle.mppi import interpolation_matrix
+    stored = load_interpolation_weights()
+    assert len(stored) == 576  # 48 horizons x 12 periods
+    for (H, period), W in stored.items():
+        np.testing.assert_array_equal(interpolation_matrix(H, period), W, err_msg=f"H={H} period={period}")
+    if not reference_has("others"):
+        return
     import json
     import subprocess
     repo = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))

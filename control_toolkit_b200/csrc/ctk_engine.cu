@@ -10,6 +10,7 @@
 #include <algorithm>
 #include <atomic>
 #include <chrono>
+#include <memory>
 #include <string>
 #include <vector>
 
@@ -37,14 +38,55 @@ static int fail(int code, const std::string& msg) {
     if (!(cond)) return fail(CTK_EINVAL, std::string("invalid argument: ") + (msg)); \
   } while (0)
 
+// Owning device (or, Pinned, page-locked host) allocation of n elements of T: move-only, freed in the destructor, converts to
+// T* so that kernel argument structs and copies take it as they took the raw pointer.  zero: cudaMemset / memset after the
+// allocation (the mailbox, partials and record buffers rely on starting at zero).
+template <typename T, bool Pinned = false>
+class Owned {
+ public:
+  Owned() = default;
+  Owned(const Owned&) = delete;
+  Owned& operator=(const Owned&) = delete;
+  Owned(Owned&& o) noexcept : p_(o.p_) { o.p_ = nullptr; }
+  Owned& operator=(Owned&& o) noexcept {
+    if (this != &o) { reset(); p_ = o.p_; o.p_ = nullptr; }
+    return *this;
+  }
+  ~Owned() { reset(); }
+  operator T*() const { return p_; }
+  T* get() const { return p_; }
+  void reset() {
+    if (p_ && Pinned) cudaFreeHost(p_);
+    else if (p_) cudaFree(p_);
+    p_ = nullptr;
+  }
+  // frees what was held first; on failure the pointer stays null
+  cudaError_t alloc(size_t n, bool zero = true, unsigned int host_flags = cudaHostAllocDefault) {
+    reset();
+    const size_t bytes = (n ? n : 1) * sizeof(T);
+    void* q = nullptr;
+    cudaError_t e = Pinned ? cudaHostAlloc(&q, bytes, host_flags) : cudaMalloc(&q, bytes);
+    if (e != cudaSuccess) return e;
+    p_ = static_cast<T*>(q);
+    if (zero && Pinned) memset(q, 0, bytes);
+    else if (zero) e = cudaMemset(q, 0, bytes);
+    return e;
+  }
+
+ private:
+  T* p_ = nullptr;
+};
+template <typename T>
+using Pinned = Owned<T, true>;
+
 struct ctk_handle {
   ctk_config cfg;
   OdeC ode;
   FwdK fwd;
   CostC cost;
   MlpDev mlp;
-  DevConsts* d_kc = nullptr;  // device copy of {fwd, cost}
-  float* d_kx = nullptr;      // device: {lo, hi, k_du2, k_udu}
+  Owned<DevConsts> d_kc;  // device copy of {fwd, cost}
+  Owned<float> d_kx;      // device: {lo, hi, k_du2, k_udu}
   cudaStream_t stream = nullptr;
   int N = 0, NG = 0, off = 0, H = 0, period = 1, n_ind = 0, nblocks = 0;
   int mppi_grid = 0, mppi_block = 0, mppi_rpb = 0, mppi_iters = 0, mppi_stash = 0, num_sms = 0;  // rpb: rollouts per block
@@ -54,10 +96,10 @@ struct ctk_handle {
   OdeHot ode_hot{};
   bool ode_kernel = false;     // MPPI + ODE predictor + intermediate_steps == 1 + few inducing points
   int ode_ilp = 2, ode_period_t = 0, ode_grid = 0, ode_block = 0, ode_fshare16 = 16;
-  unsigned long long* d_trace = nullptr;  // optional per-block phase timeline of the last ODE-kernel launch
+  Owned<unsigned long long> d_trace;  // optional per-block phase timeline of the last ODE-kernel launch
   size_t ode_smem = 0;
   // fused tick finish / cross-GPU exchange (MppiFuse)
-  unsigned long long* d_mbox = nullptr;           // local mailbox (layout: MppiFuse)
+  Owned<unsigned long long> d_mbox;               // local mailbox (layout: MppiFuse)
   unsigned int bseq = 0;                          // sequence number of the exchange barrier (ctk_exchange_barrier)
   bool chain_hint = false;                        // set by ctk_step_device_n for ticks 1.. of a chain: the tick may poll the hand-over
   bool chain_next = false;                        // set by ctk_step_device_n for ticks that a chained tick follows: publish the hand-over
@@ -66,47 +108,47 @@ struct ctk_handle {
   int xworld = 1, xrank = 0;
   unsigned int xseq = 0;
   // common
-  float *d_s0 = nullptr, *d_u_prev = nullptr, *d_u_out = nullptr, *d_J = nullptr;
-  float *h_pin = nullptr;  // MAPPED pinned memory: s[8] | u, status, sequence flag .. [16) | one [H] state array (HostMirror layout)
-  float *d_pin = nullptr;  // the device's view of h_pin
-  void* h_log[8] = {nullptr};      // pinned host buffers of ctk_get_log_view, by log id
+  Owned<float> d_u_prev, d_u_out, d_J;
+  Pinned<float> h_pin;     // MAPPED pinned memory: s[8] | u, status, sequence flag .. [16) | one [H] state array (HostMirror layout)
+  float* d_pin = nullptr;  // the device's view of h_pin
+  Pinned<char> h_log[8];   // pinned host buffers of ctk_get_log_view, by log id
   size_t h_log_cap[8] = {0};
   HostMirror mirror{nullptr, 0};  // non-null only while a host-facing tick (ctk_step / ctk_step_state) is being enqueued
   unsigned int hseq = 0;
   // mppi
-  float *d_u_nom = nullptr, *d_partials = nullptr, *d_record = nullptr;
+  Owned<float> d_u_nom, d_partials, d_record;
   // cem
-  float *d_mu = nullptr, *d_sd = nullptr;
-  uint64_t *d_keys[2] = {nullptr, nullptr};
-  int32_t* d_elite_idx = nullptr;
+  Owned<float> d_mu, d_sd;
+  Owned<uint64_t> d_keys[2];
+  Owned<int32_t> d_elite_idx;
   int elite_log_cap = 0, elite_log_rows = 0;
   int cem_it = 0, cem_iters = 0, cem_cand = 0;
   uint64_t* cem_cand_ptr = nullptr;
   NoiseSrc cem_noise{};
-  unsigned long long *d_cem_cand = nullptr, *d_cem_dist = nullptr;  // persistent CEM tick: tagged candidate / distribution slots
+  Owned<unsigned long long> d_cem_cand, d_cem_dist;  // persistent CEM tick: tagged candidate / distribution slots
   unsigned int cem_seq = 0;
   int cem_tick_per_sm = -1;  // resident blocks per SM of the persistent tick kernel (re-queried when the instantiation changes)
   bool cem_coop_refused = false;  // the runtime refused the cooperative launch once: multi-launch path from then on
   // rpgd
-  float *d_Q[2] = {nullptr, nullptr}, *d_m[2] = {nullptr, nullptr}, *d_v[2] = {nullptr, nullptr}, *d_ages[2] = {nullptr, nullptr};
+  Owned<float> d_Q[2], d_m[2], d_v[2], d_ages[2];
   int cur = 0;
   const float* pending_s = nullptr;  // gradient-assisted CEM modes: state pointer of the tick in flight
-  float *d_unom_log = nullptr, *d_ages_log = nullptr, *d_Q_log = nullptr;
-  int32_t* d_best_idx = nullptr;
+  Owned<float> d_unom_log, d_ages_log, d_Q_log;
+  Owned<int32_t> d_best_idx;
   // logs
-  float *d_log_traj_soa = nullptr, *d_log_Q_soa = nullptr, *d_log_tmp = nullptr;
+  Owned<float> d_log_traj_soa, d_log_Q_soa, d_log_tmp;
   // top-M logging (ctk_get_log_top): K4 key buffers, gathered rows, pinned host staging
-  uint64_t* d_top_keys[2] = {nullptr, nullptr};
-  float* d_top_out = nullptr;
-  float* h_top = nullptr;
+  Owned<uint64_t> d_top_keys[2];
+  Owned<float> d_top_out;
+  Pinned<float> h_top;
   size_t top_keys_cap = 0, top_out_cap = 0;
   // injected noise queue
-  float* d_inj = nullptr;
+  Owned<float> d_inj;
   size_t inj_cap = 0, inj_size = 0, inj_pos = 0;
   // mlp
-  float* d_mlp = nullptr;
-  void* d_mlp_tc = nullptr;  // tcgen05 engine blob (ctk_mlp_tc.cuh)
-  float* d_rnn_h = nullptr;  // recurrent predictor: saved hidden state [2][2 hid] (row 0 current, row 1 before the last update)
+  Owned<float> d_mlp;
+  Owned<uint8_t> d_mlp_tc;  // tcgen05 engine blob (ctk_mlp_tc.cuh)
+  Owned<float> d_rnn_h;     // recurrent predictor: saved hidden state [2][2 hid] (row 0 current, row 1 before the last update)
   const float* step_s = nullptr;  // state pointer of the tick in flight (staged MPPI ticks: predictor.update runs in ctk_step_finish)
   // environments beyond the CartPole (ctk_kernels_env.cuh): env id, dimensions, parameter block, per-input limits
   int env = 0, ns = 6, nu = 1;
@@ -116,7 +158,7 @@ struct ctk_handle {
   // multi-client batching (ctk_step_batch): per-client state sits behind the pointers of client 0 at fixed strides
   int nclients = 1;
   uint32_t client_tick[kMaxBatchClients] = {0};
-  float* h_batch = nullptr;  // pinned: [nclients][2] u, status
+  Pinned<float> h_batch;  // [nclients][2] u, status
   size_t mbox_stride = 0, partials_stride = 0;
   // counters
   int64_t count = 0, adam_step = 0, tick = 0, launches = 0;
@@ -126,6 +168,17 @@ struct ctk_handle {
   std::vector<cudaEvent_t> ev;  // pairs
   size_t ev_used = 0;
   std::string last_kernel;  // instantiation of the last rollout-kernel launch (ctk_last_kernel: tests pin the production kernels)
+
+  ~ctk_handle() {
+    close_peers();
+    for (cudaEvent_t e : ev) cudaEventDestroy(e);
+  }
+  void close_peers() {  // the IPC-mapped peer mailboxes of ctk_exchange_connect
+    for (int r = 0; r < CTK_MAX_PEERS; ++r) {
+      if (mbox_ipc[r] && mbox_peer[r]) cudaIpcCloseMemHandle(mbox_peer[r]);
+      mbox_peer[r] = nullptr; mbox_ipc[r] = false;
+    }
+  }
 };
 
 struct KernelTimer {  // records an event pair around the dominant kernel launch when timing is enabled
@@ -150,20 +203,13 @@ struct KernelTimer {  // records an event pair around the dominant kernel launch
 };
 
 // ---------------------------------------------------------------------------------------------------------------
-static cudaError_t upload_consts(ctk_handle* h);
-
-template <typename T>
-static cudaError_t dalloc(T** p, size_t n) {
-  cudaError_t e = cudaMalloc((void**)p, (n ? n : 1) * sizeof(T));
-  if (e == cudaSuccess) e = cudaMemset(*p, 0, (n ? n : 1) * sizeof(T));
-  return e;
-}
-
 static void mppi_ode_geometry(ctk_handle* h);
 static int pred_id(const ctk_handle* h);
 static bool tile_engine(int pred);
-static cudaError_t upload_consts(ctk_handle* h) {
-  if (h->env != 0) return cudaSuccess;  // general environments carry their constants in the kernel parameters (EnvParams)
+
+// Host-side constants of the rollout kernels (and, MPPI, the ODE kernel's geometry) from cfg / ode_p / cost_p: no device access
+static void derive_consts(ctk_handle* h) {
+  if (h->env != 0) return;  // general environments carry their constants in the kernel parameters (EnvParams)
   h->cem_tick_per_sm = -1;  // the cost kind selects the persistent tick's instantiation (register count): re-query its occupancy
   if (h->cfg.optimizer == CTK_OPT_MPPI) {
     const ctk_config& c = h->cfg;
@@ -178,6 +224,11 @@ static cudaError_t upload_consts(ctk_handle* h) {
     derive_ode_hot(h->ode_p, h->cost_p, h->H, mc, h->ode_hot);
     h->ode_kernel = c.predictor == CTK_PRED_ODE && h->ode_p.intermediate_steps <= 1 && getenv("CTK_CEM_GENERIC") == nullptr;
   }
+}
+
+// Copies the constants derive_consts / derive_* produced to d_kc / d_kx
+static cudaError_t upload_consts(ctk_handle* h) {
+  if (h->env != 0) return cudaSuccess;
   DevConsts kc;
   kc.fwd = h->fwd;
   kc.cost = h->cost;
@@ -215,6 +266,34 @@ static int make_noise(ctk_handle* h, uint32_t stream_id, int per_rollout, int un
   return CTK_OK;
 }
 
+// K4: hierarchical bitonic top-k (tf.argsort(...)[:k], ties -> lower index), one launch per level, ping-ponging between b0 and b1
+// from level lvl on.  Input: the costs `cost` of n rollouts, or (cost == nullptr) the n candidate keys `keys`.  Levels run until at
+// most 1024 keys are left -- exact_k: until exactly k are (one block) -- and at least one runs on costs.  On return keys / n hold
+// the result.
+static cudaError_t topk_levels(const float* cost, const uint64_t*& keys, int& n, int lvl, int off, int k, bool exact_k, uint64_t* b0,
+                               uint64_t* b1, cudaStream_t stream, int64_t& launches) {
+  while (cost != nullptr || n > TOPK_THREADS || (exact_k && n != k)) {
+    const int nb = (n + TOPK_THREADS - 1) / TOPK_THREADS;
+    uint64_t* out = (lvl++ & 1) ? b1 : b0;
+    launches++;
+    const cudaError_t e = launch_topk_level(cost, keys, n, off, k, out, stream);
+    if (e != cudaSuccess) return e;
+    cost = nullptr; keys = out; n = nb * k;
+  }
+  return cudaSuccess;
+}
+
+// outer iterations of this CEM tick (optimizer_cem_tf.py:92)
+static int cem_tick_iters(const ctk_handle* h) {
+  return (h->cfg.cem_warmup && h->count == 0) ? h->cfg.cem_warmup_iterations : h->cfg.cem_outer_it;
+}
+
+// next value of a wrapping sequence number that skips 0 (0 marks an empty slot)
+static unsigned int next_seq(unsigned int& seq) {
+  if (++seq == 0) seq = 1;
+  return seq;
+}
+
 // ---------------------------------------------------------------------------------------------------------------
 // lifecycle
 // ---------------------------------------------------------------------------------------------------------------
@@ -224,38 +303,18 @@ extern "C" int ctk_abi_version(void) { return CTK_ABI_VERSION; }
 extern "C" int ctk_destroy(ctk_handle* h) {
   if (!h) return CTK_OK;
   cudaSetDevice(h->cfg.device);
-  float* fp[] = {h->d_s0, h->d_u_prev, h->d_u_out, h->d_J, h->d_u_nom, h->d_partials, h->d_record, h->d_mu, h->d_sd,
-                 h->d_Q[0], h->d_Q[1], h->d_m[0], h->d_m[1], h->d_v[0], h->d_v[1], h->d_ages[0], h->d_ages[1],
-                 h->d_unom_log, h->d_ages_log, h->d_Q_log, h->d_log_traj_soa, h->d_log_Q_soa, h->d_log_tmp, h->d_inj, h->d_mlp};
-  for (float* p : fp) if (p) cudaFree(p);
-  if (h->d_kc) cudaFree(h->d_kc);
-  if (h->d_kx) cudaFree(h->d_kx);
-  if (h->d_keys[0]) cudaFree(h->d_keys[0]);
-  if (h->d_keys[1]) cudaFree(h->d_keys[1]);
-  if (h->d_elite_idx) cudaFree(h->d_elite_idx);
-  if (h->d_top_keys[0]) cudaFree(h->d_top_keys[0]);
-  if (h->d_top_keys[1]) cudaFree(h->d_top_keys[1]);
-  if (h->d_top_out) cudaFree(h->d_top_out);
-  if (h->h_top) cudaFreeHost(h->h_top);
-  if (h->d_cem_cand) cudaFree(h->d_cem_cand);
-  if (h->d_cem_dist) cudaFree(h->d_cem_dist);
-  if (h->d_best_idx) cudaFree(h->d_best_idx);
-  if (h->d_mlp_tc) cudaFree(h->d_mlp_tc);
-  if (h->d_rnn_h) cudaFree(h->d_rnn_h);
-  for (int r = 0; r < CTK_MAX_PEERS; ++r)
-    if (h->mbox_ipc[r] && h->mbox_peer[r]) cudaIpcCloseMemHandle(h->mbox_peer[r]);
-  if (h->d_trace) cudaFree(h->d_trace);
-  if (h->d_mbox) cudaFree(h->d_mbox);
-  for (cudaEvent_t e : h->ev) cudaEventDestroy(e);
-  if (h->h_pin) cudaFreeHost(h->h_pin);
-  if (h->h_batch) cudaFreeHost(h->h_batch);
-  for (void* p : h->h_log) if (p) cudaFreeHost(p);
   delete h;
   return CTK_OK;
 }
 
-extern "C" int ctk_create(const ctk_config* cfg, const ctk_ode_params* ode, const ctk_cost_params* cost, ctk_handle** out) {
-  REQ(cfg && ode && cost && out, "null pointer");
+static int inducing_points(int H, int period) { return (int)std::ceil((double)(H - 1) / (double)period) + 1; }  // Interpolator.py:79-84
+// rows of the CEM elite-index log: the outer iterations of the longest tick (the warm-up tick may run more)
+static int elite_log_rows_max(const ctk_config& c) {
+  return (c.cem_warmup && c.cem_warmup_iterations > c.cem_outer_it) ? c.cem_warmup_iterations : c.cem_outer_it;
+}
+
+// Every rejection that needs nothing but the arguments: a configuration that cannot run is refused before the device is touched
+static int check_config(const ctk_config* cfg, const ctk_ode_params* ode, const ctk_cost_params* cost) {
   REQ(cfg->abi_version == CTK_ABI_VERSION, "abi_version mismatch");
   REQ(cfg->optimizer >= CTK_OPT_MPPI && cfg->optimizer <= CTK_OPT_RPGD, "unknown optimizer");
   REQ(cfg->predictor == CTK_PRED_ODE || cfg->predictor == CTK_PRED_MLP || cfg->predictor == CTK_PRED_GRU, "unknown predictor");
@@ -282,163 +341,165 @@ extern "C" int ctk_create(const ctk_config* cfg, const ctk_ode_params* ode, cons
   REQ(B <= kMaxBatchClients, "num_clients must be <= 16");
   REQ(B == 1 || (cfg->optimizer == CTK_OPT_MPPI && cfg->predictor == CTK_PRED_ODE && !cfg->logging && cfg->num_rollouts == cfg->num_rollouts_global),
       "multi-client handles are implemented for MPPI with the ODE predictor, logging off, unsharded");
+  const int N = cfg->num_rollouts, H = cfg->mpc_horizon, period = cfg->period_interpolation_inducing_points;
+  if (cfg->optimizer != CTK_OPT_CEM && period < 1) return fail(CTK_EINVAL, "period_interpolation_inducing_points must be >= 1");
+  if (cfg->environment != CTK_ENV_CARTPOLE) {
+    if (cfg->optimizer == CTK_OPT_MPPI && (inducing_points(H, period) * env_nu > 32 || H * env_nu > 1024))
+      return fail(CTK_EINVAL, "environment MPPI: n_ind * nu <= 32 and H * nu <= 1024");
+    if (cfg->optimizer == CTK_OPT_CEM &&
+        !(cfg->cem_best_k >= 1 && cfg->cem_best_k <= 512 && cfg->cem_best_k <= N && H * env_nu <= 1024 && cfg->cem_outer_it >= 1))
+      return fail(CTK_EINVAL, "environment CEM needs 1 <= cem_best_k <= min(512, num_rollouts), H * nu <= 1024, cem_outer_it >= 1");
+  } else if (cfg->optimizer == CTK_OPT_CEM) {
+    if (!(cfg->cem_best_k >= 1 && cfg->cem_best_k <= 512 && cfg->cem_best_k <= cfg->num_rollouts_global && H <= 1024 && cfg->cem_outer_it >= 1))
+      return fail(CTK_EINVAL, "CEM needs 1 <= cem_best_k <= min(512, num_rollouts), mpc_horizon <= 1024, cem_outer_it >= 1");
+  } else if (cfg->optimizer == CTK_OPT_RPGD) {
+    if (!(N <= 1024 && cfg->rpgd_keep_k >= 1 && cfg->rpgd_keep_k <= N && N == cfg->num_rollouts_global && cfg->predictor == CTK_PRED_ODE &&
+          ode->intermediate_steps <= 1 && cfg->rpgd_shift_previous >= 0))
+      return fail(CTK_EINVAL, "RPGD needs num_rollouts <= 1024 (replicas only, no sharding), the ODE predictor with "
+                              "intermediate_steps == 1 and 1 <= keep_k <= num_rollouts");
+    if (cfg->rpgd_gradient_mode >= 2 && !(cfg->rpgd_gradient_mode <= 3 && cfg->cem_best_k >= 1 && cfg->cem_best_k <= N && cfg->cem_outer_it >= 1 &&
+                                          period == 1 && elite_log_rows_max(*cfg) >= 1))
+      return fail(CTK_EINVAL, "gradient-assisted CEM needs 1 <= cem_best_k <= num_rollouts, cem_outer_it >= 1 and inducing-point period 1");
+  }
+  return CTK_OK;
+}
+
+// K1 geometry of the CartPole MPPI rollout kernels: one CTA per SM, block sized so that every thread runs the same number of
+// rollouts (no tail wave).  Needs num_sms; allocates nothing.
+static int mppi_geometry(ctk_handle* h) {
+  const int N = h->N;
+  const int maxb = mppi_max_block_threads(pred_id(h));
+  const long long slots = (long long)h->num_sms * maxb;
+  const int r = (int)((N + slots - 1) / slots);                                  // rollouts per thread
+  int T = (int)(((((long long)N + (long long)r * h->num_sms - 1) / ((long long)r * h->num_sms)) + 31) / 32 * 32);
+  if (T > maxb) T = maxb;
+  if (T < 32) T = 32;
+  h->mppi_block = T;
+  h->mppi_grid = (int)std::min<long long>(h->num_sms, ((long long)N + T - 1) / T);  // every SM gets a CTA
+  if (h->mppi_grid < 1) h->mppi_grid = 1;
+  h->mppi_iters = (int)((N + (long long)h->mppi_grid * T - 1) / ((long long)h->mppi_grid * T));
+  h->mppi_stash = ((size_t)h->n_ind * T * sizeof(float) <= 96 * 1024) ? 1 : 0;
+  if ((size_t)h->n_ind * T * sizeof(float) > 100 * 1024) {  // accumulator array must fit: shrink the block
+    T = (int)((100 * 1024 / sizeof(float) / (size_t)h->n_ind) / 32 * 32);
+    if (T < 32) return fail(CTK_EINVAL, "MPPI: too many inducing points for the shared-memory accumulators");
+    h->mppi_block = T;
+    h->mppi_grid = (int)std::min<long long>(h->num_sms, ((long long)N + T - 1) / T);
+    h->mppi_stash = 0;
+  }
+  h->mppi_rpb = h->mppi_block;
+  if (tile_engine(pred_id(h))) {
+    // tcgen05 MLP engines (ctk_mlp_tc.cuh): one CTA per SM, every CTA an equal contiguous share of the population (kBalanced); rollouts per
+    // block = tiles in flight x 128: the single-product engines run four tiles (one per warp group), the exact engine two, its round-1
+    // structure (pred 6) one tile with 16 worker warps + 1 MMA-issuer warp
+    const int pid = pred_id(h);
+    h->mppi_block = mppi_max_block_threads(pid); h->mppi_rpb = pid == 6 ? 128 : (pid == 2 ? 256 : 512);
+    h->mppi_grid = (int)std::min<long long>((long long)h->num_sms, ((long long)N + 127) / 128);
+    if (h->mppi_grid < 1) h->mppi_grid = 1;
+    h->mppi_iters = (int)((N + (long long)h->mppi_grid * h->mppi_rpb - 1) / ((long long)h->mppi_grid * h->mppi_rpb));
+    h->mppi_stash = (pid == 6 && (size_t)h->n_ind * 128 * sizeof(float) <= 8 * 1024) ? 1 : 0;
+    // what the operand tiles leave of the 227 KB for the per-rollout accumulators [n_ind][rollouts per block]
+    const size_t acc_limit = pid == 6 ? 8 * 1024 : (pid == 2 ? 12 * 1024 : 32 * 1024);
+    if ((size_t)h->n_ind * h->mppi_rpb * sizeof(float) > acc_limit) return fail(CTK_EINVAL, "tcgen05 MLP engine: too many inducing points (shared memory is taken by the operand tiles)");
+  }
+  h->partials_stride = (size_t)(h->num_sms > h->mppi_grid ? h->num_sms : h->mppi_grid) * (h->mppi_iters + 1) * (h->n_ind + 2);
+  if (h->mppi_grid > CTK_MBOX_BLOCKS || h->num_sms > CTK_MBOX_BLOCKS) return fail(CTK_EINVAL, "device has more SMs than the mailbox has block slots (CTK_MBOX_BLOCKS)");
+  h->mbox_stride = (mbox_total_slots(h->n_ind, h->H) + 1) & ~(size_t)1;  // even: the records are polled with 16-byte loads
+  return CTK_OK;
+}
+
+extern "C" int ctk_create(const ctk_config* cfg, const ctk_ode_params* ode, const ctk_cost_params* cost, ctk_handle** out) {
+  REQ(cfg && ode && cost && out, "null pointer");
+  int rc = check_config(cfg, ode, cost);
+  if (rc != CTK_OK) return rc;
   int ndev = 0;
   CU(cudaGetDeviceCount(&ndev));
   REQ(cfg->device >= 0 && cfg->device < ndev, "no such CUDA device");
   CU(cudaSetDevice(cfg->device));
 
-  ctk_handle* h = new ctk_handle();
+  std::unique_ptr<ctk_handle> owner(new ctk_handle());  // a failing create frees whatever it allocated
+  ctk_handle* h = owner.get();
+  const int B = cfg->num_clients > 1 ? cfg->num_clients : 1;
   h->cfg = *cfg;
   h->N = cfg->num_rollouts; h->NG = cfg->num_rollouts_global; h->off = cfg->rollout_offset; h->H = cfg->mpc_horizon;
   h->ode_p = *ode; h->cost_p = *cost;
   h->nclients = B;
-  h->env = cfg->environment; h->ns = env_ns; h->nu = env_nu;
+  h->env = cfg->environment;
+  env_dims(cfg->environment, &h->ns, &h->nu);
   for (int c = 0; c < kEnvMaxControls; ++c) { h->lo_v[c] = cfg->action_low; h->hi_v[c] = cfg->action_high; }
   derive_ode(*ode, h->ode);
   derive_fwd(*ode, h->fwd);
   derive_cost(*cost, h->H, h->cost);
   h->mlp = MlpDev{0, nullptr, 0, nullptr, nullptr};
   h->nblocks = (h->N + 127) / 128;
-  const int N = h->N, H = h->H;
-  int rc = CTK_OK;
+  if (cfg->optimizer == CTK_OPT_MPPI || cfg->optimizer == CTK_OPT_RPGD) {
+    h->period = cfg->period_interpolation_inducing_points;
+    h->n_ind = inducing_points(h->H, h->period);
+  }
+  const int N = h->N, H = h->H, nu = h->nu;
   auto A = [&](cudaError_t e, const char* what) {
     if (e != cudaSuccess && rc == CTK_OK) rc = fail(CTK_ECUDA, std::string("cudaMalloc ") + what + ": " + cudaGetErrorString(e));
   };
-  A(dalloc(&h->d_s0, 8), "s0"); A(dalloc(&h->d_u_prev, (size_t)(B > env_nu ? B : env_nu)), "u_prev"); A(dalloc(&h->d_u_out, 4 + 2 * (size_t)B), "u_out");
-  A(dalloc(&h->d_J, (size_t)N * B), "J");
-  if (B > 1) A(cudaHostAlloc((void**)&h->h_batch, 2 * (size_t)B * sizeof(float), cudaHostAllocDefault), "pinned (batch results)");
-  A(cudaMalloc((void**)&h->d_kc, sizeof(DevConsts)), "consts");
-  A(dalloc(&h->d_kx, 4), "kx");
-  A(cudaHostAlloc((void**)&h->h_pin, (32 + 2 * (size_t)H) * sizeof(float), cudaHostAllocMapped), "pinned");
-  if (h->h_pin) { memset(h->h_pin, 0, (32 + 2 * (size_t)H) * sizeof(float)); A(cudaHostGetDevicePointer((void**)&h->d_pin, h->h_pin, 0), "pinned (device view)"); }
-  if (cfg->logging) {
-    A(dalloc(&h->d_log_traj_soa, (size_t)(H + 1) * env_ns * N), "log_traj");
-    A(dalloc(&h->d_log_Q_soa, (size_t)H * env_nu * N), "log_Q");
-    if (h->env == 0) A(dalloc(&h->d_log_tmp, (size_t)(H + 1) * 6 * N), "log_tmp");
-  }
-  if (cfg->optimizer == CTK_OPT_MPPI || cfg->optimizer == CTK_OPT_RPGD) {
-    h->period = cfg->period_interpolation_inducing_points;
-    if (h->period < 1) { ctk_destroy(h); return fail(CTK_EINVAL, "period_interpolation_inducing_points must be >= 1"); }
-    h->n_ind = (int)std::ceil((double)(H - 1) / (double)h->period) + 1;  // Interpolator.py:79-84
-  }
-  if (h->env != 0) {
-    // general-environment kernels: flat [H][nu] state arrays; CEM shares K4 (top-k levels) with the CartPole path
-    if (cfg->optimizer == CTK_OPT_MPPI) {
-      if (h->n_ind * env_nu > 32 || H * env_nu > 1024) { ctk_destroy(h); return fail(CTK_EINVAL, "environment MPPI: n_ind * nu <= 32 and H * nu <= 1024"); }
-      A(dalloc(&h->d_u_nom, (size_t)H * env_nu), "u_nom");
-    } else {
-      if (!(cfg->cem_best_k >= 1 && cfg->cem_best_k <= 512 && cfg->cem_best_k <= N && H * env_nu <= 1024 && cfg->cem_outer_it >= 1)) {
-        ctk_destroy(h);
-        return fail(CTK_EINVAL, "environment CEM needs 1 <= cem_best_k <= min(512, num_rollouts), H * nu <= 1024, cem_outer_it >= 1");
-      }
-      A(dalloc(&h->d_mu, (size_t)H * env_nu), "mu"); A(dalloc(&h->d_sd, (size_t)H * env_nu), "sd");
-      const size_t nk = (size_t)((N + 1023) / 1024) * cfg->cem_best_k + 1024;
-      A(dalloc(&h->d_keys[0], nk), "keys0"); A(dalloc(&h->d_keys[1], nk), "keys1");
-      int iters = cfg->cem_outer_it;
-      if (cfg->cem_warmup && cfg->cem_warmup_iterations > iters) iters = cfg->cem_warmup_iterations;
-      h->elite_log_cap = iters;
-      A(dalloc(&h->d_elite_idx, (size_t)iters * cfg->cem_best_k), "elite_idx");
-    }
-  } else if (cfg->optimizer == CTK_OPT_MPPI) {
-    // K1 geometry: one CTA per SM, block sized so that every thread runs the same number of rollouts (no tail wave)
+  // geometry checks that need the SM count, before any allocation
+  if (h->env == 0 && cfg->optimizer != CTK_OPT_RPGD) {
     cudaDeviceProp prop;
     A(cudaGetDeviceProperties(&prop, cfg->device), "props");
+    if (rc != CTK_OK) return rc;
     h->num_sms = prop.multiProcessorCount > 0 ? prop.multiProcessorCount : 148;
-    const int maxb = mppi_max_block_threads(pred_id(h));
-    const long long slots = (long long)h->num_sms * maxb;
-    const int r = (int)((N + slots - 1) / slots);                                  // rollouts per thread
-    int T = (int)(((((long long)N + (long long)r * h->num_sms - 1) / ((long long)r * h->num_sms)) + 31) / 32 * 32);
-    if (T > maxb) T = maxb;
-    if (T < 32) T = 32;
-    h->mppi_block = T;
-    h->mppi_grid = (int)std::min<long long>(h->num_sms, ((long long)N + T - 1) / T);  // every SM gets a CTA
-    if (h->mppi_grid < 1) h->mppi_grid = 1;
-    h->mppi_iters = (int)((N + (long long)h->mppi_grid * T - 1) / ((long long)h->mppi_grid * T));
-    h->mppi_stash = ((size_t)h->n_ind * T * sizeof(float) <= 96 * 1024) ? 1 : 0;
-    if ((size_t)h->n_ind * T * sizeof(float) > 100 * 1024) {  // accumulator array must fit: shrink the block
-      T = (int)((100 * 1024 / sizeof(float) / (size_t)h->n_ind) / 32 * 32);
-      if (T < 32) { ctk_destroy(h); return fail(CTK_EINVAL, "MPPI: too many inducing points for the shared-memory accumulators"); }
-      h->mppi_block = T;
-      h->mppi_grid = (int)std::min<long long>(h->num_sms, ((long long)N + T - 1) / T);
-      h->mppi_stash = 0;
-    }
-    h->mppi_rpb = h->mppi_block;
-    if (tile_engine(pred_id(h))) {
-      // tcgen05 MLP engines (ctk_mlp_tc.cuh): one CTA per SM, every CTA an equal contiguous share of the population (kBalanced); rollouts per
-      // block = tiles in flight x 128: the single-product engines run four tiles (one per warp group), the exact engine two, its round-1
-      // structure (pred 6) one tile with 16 worker warps + 1 MMA-issuer warp
-      const int pid = pred_id(h);
-      h->mppi_block = mppi_max_block_threads(pid); h->mppi_rpb = pid == 6 ? 128 : (pid == 2 ? 256 : 512);
-      h->mppi_grid = (int)std::min<long long>((long long)h->num_sms, ((long long)N + 127) / 128);
-      if (h->mppi_grid < 1) h->mppi_grid = 1;
-      h->mppi_iters = (int)((N + (long long)h->mppi_grid * h->mppi_rpb - 1) / ((long long)h->mppi_grid * h->mppi_rpb));
-      h->mppi_stash = (pid == 6 && (size_t)h->n_ind * 128 * sizeof(float) <= 8 * 1024) ? 1 : 0;
-      // what the operand tiles leave of the 227 KB for the per-rollout accumulators [n_ind][rollouts per block]
-      const size_t acc_limit = pid == 6 ? 8 * 1024 : (pid == 2 ? 12 * 1024 : 32 * 1024);
-      if ((size_t)h->n_ind * h->mppi_rpb * sizeof(float) > acc_limit) { ctk_destroy(h); return fail(CTK_EINVAL, "tcgen05 MLP engine: too many inducing points (shared memory is taken by the operand tiles)"); }
-    }
-    A(dalloc(&h->d_u_nom, (size_t)H * B), "u_nom");
-    h->partials_stride = (size_t)(h->num_sms > h->mppi_grid ? h->num_sms : h->mppi_grid) * (h->mppi_iters + 1) * (h->n_ind + 2);
-    A(dalloc(&h->d_partials, h->partials_stride * B), "partials");
-    A(dalloc(&h->d_record, (size_t)(h->n_ind + 2) * B), "record");
-    if (h->mppi_grid > CTK_MBOX_BLOCKS || h->num_sms > CTK_MBOX_BLOCKS) { ctk_destroy(h); return fail(CTK_EINVAL, "device has more SMs than the mailbox has block slots (CTK_MBOX_BLOCKS)"); }
-    h->mbox_stride = (mbox_total_slots(h->n_ind, H) + 1) & ~(size_t)1;  // even: the records are polled with 16-byte loads
-    A(dalloc(&h->d_mbox, h->mbox_stride * B), "mailbox");
+    if (cfg->optimizer == CTK_OPT_MPPI && (rc = mppi_geometry(h)) != CTK_OK) return rc;
+  }
+  derive_consts(h);
+  if (B > 1 && !(h->ode_kernel && h->ode_ilp == 1))
+    return fail(CTK_EINVAL, "multi-client handles run the one-rollout-per-thread ODE kernel: intermediate_steps == 1, few inducing points, "
+                            "num_rollouts <= 1024 x SMs per client");
+
+  A(h->d_u_prev.alloc((size_t)(B > nu ? B : nu)), "u_prev"); A(h->d_u_out.alloc(4 + 2 * (size_t)B), "u_out");
+  A(h->d_J.alloc((size_t)N * B), "J");
+  if (B > 1) A(h->h_batch.alloc(2 * (size_t)B, false), "pinned (batch results)");
+  A(h->d_kc.alloc(1, false), "consts");
+  A(h->d_kx.alloc(4), "kx");
+  A(h->h_pin.alloc(32 + 2 * (size_t)H, true, cudaHostAllocMapped), "pinned");
+  if (h->h_pin) A(cudaHostGetDevicePointer((void**)&h->d_pin, h->h_pin, 0), "pinned (device view)");
+  if (cfg->logging) {
+    A(h->d_log_traj_soa.alloc((size_t)(H + 1) * h->ns * N), "log_traj");
+    A(h->d_log_Q_soa.alloc((size_t)H * nu * N), "log_Q");
+    if (h->env == 0) A(h->d_log_tmp.alloc((size_t)(H + 1) * 6 * N), "log_tmp");
+  }
+  // state arrays are flat [H][nu] ([H] x clients for multi-client MPPI)
+  if (cfg->optimizer == CTK_OPT_MPPI) A(h->d_u_nom.alloc((size_t)H * nu * B), "u_nom");
+  if (cfg->optimizer == CTK_OPT_CEM || (cfg->optimizer == CTK_OPT_RPGD && cfg->rpgd_gradient_mode >= 2)) {
+    // CEM distribution and per-iteration elite log (gradient-assisted CEM: on top of the RPGD population)
+    A(h->d_mu.alloc((size_t)H * nu), "mu"); A(h->d_sd.alloc((size_t)H * nu), "sd");
+    h->elite_log_cap = elite_log_rows_max(*cfg);
+    A(h->d_elite_idx.alloc((size_t)h->elite_log_cap * cfg->cem_best_k), "elite_idx");
+  }
+  if (cfg->optimizer == CTK_OPT_CEM) {  // K4 keys: level-0 candidates of 256-rollout blocks (CartPole: fused top-k) or 1024-key blocks
+    const int blk = h->env == 0 ? 256 : 1024;
+    const size_t nk = (size_t)((N + blk - 1) / blk) * cfg->cem_best_k + 1024;
+    A(h->d_keys[0].alloc(nk), "keys0"); A(h->d_keys[1].alloc(nk), "keys1");
+  }
+  if (h->env == 0 && cfg->optimizer == CTK_OPT_MPPI) {
+    A(h->d_partials.alloc(h->partials_stride * B), "partials");
+    A(h->d_record.alloc((size_t)(h->n_ind + 2) * B), "record");
+    A(h->d_mbox.alloc(h->mbox_stride * B), "mailbox");
     h->mbox_peer[0] = h->d_mbox;
-  } else if (cfg->optimizer == CTK_OPT_CEM) {
-    if (!(cfg->cem_best_k >= 1 && cfg->cem_best_k <= 512 && cfg->cem_best_k <= cfg->num_rollouts_global && H <= 1024 && cfg->cem_outer_it >= 1)) {
-      ctk_destroy(h);
-      return fail(CTK_EINVAL, "CEM needs 1 <= cem_best_k <= min(512, num_rollouts), mpc_horizon <= 1024, cem_outer_it >= 1");
-    }
-    A(dalloc(&h->d_mu, (size_t)H), "mu"); A(dalloc(&h->d_sd, (size_t)H), "sd");
-    const size_t nk = (size_t)((N + 255) / 256) * cfg->cem_best_k + 1024;  // level-0 candidates of 256-rollout blocks (fused top-k) or 1024-key blocks
-    A(dalloc(&h->d_keys[0], nk), "keys0"); A(dalloc(&h->d_keys[1], nk), "keys1");
-    int iters = cfg->cem_outer_it;
-    if (cfg->cem_warmup && cfg->cem_warmup_iterations > iters) iters = cfg->cem_warmup_iterations;
-    h->elite_log_cap = iters;
-    A(dalloc(&h->d_elite_idx, (size_t)iters * cfg->cem_best_k), "elite_idx");
-    {  // persistent single-launch tick (cem_tick_kernel): tagged slots for one resident grid
-      cudaDeviceProp prop;
-      A(cudaGetDeviceProperties(&prop, cfg->device), "props");
-      h->num_sms = prop.multiProcessorCount > 0 ? prop.multiProcessorCount : 148;
-      A(dalloc(&h->d_cem_cand, (size_t)2 * h->num_sms * 128), "cem_cand");  // [blocks <= 2 x SMs][k <= 128]
-      A(dalloc(&h->d_mbox, cem_mbox_slots()), "mailbox");  // fused cross-GPU candidate exchange (CemRefitArgs)
-      h->mbox_peer[0] = h->d_mbox;
-      A(dalloc(&h->d_cem_dist, (size_t)2 * 512), "cem_dist");
-    }
-  } else {
-    if (!(N <= 1024 && cfg->rpgd_keep_k >= 1 && cfg->rpgd_keep_k <= N && N == h->NG && cfg->predictor == CTK_PRED_ODE &&
-          ode->intermediate_steps <= 1 && cfg->rpgd_shift_previous >= 0)) {
-      ctk_destroy(h);
-      return fail(CTK_EINVAL, "RPGD needs num_rollouts <= 1024 (replicas only, no sharding), the ODE predictor with "
-                              "intermediate_steps == 1 and 1 <= keep_k <= num_rollouts");
-    }
+  } else if (h->env == 0 && cfg->optimizer == CTK_OPT_CEM) {
+    // persistent single-launch tick (cem_tick_kernel): tagged slots for one resident grid
+    A(h->d_cem_cand.alloc((size_t)2 * h->num_sms * 128), "cem_cand");  // [blocks <= 2 x SMs][k <= 128]
+    A(h->d_mbox.alloc(cem_mbox_slots()), "mailbox");  // fused cross-GPU candidate exchange (CemRefitArgs)
+    h->mbox_peer[0] = h->d_mbox;
+    A(h->d_cem_dist.alloc((size_t)2 * 512), "cem_dist");
+  } else if (cfg->optimizer == CTK_OPT_RPGD) {
     for (int i = 0; i < 2; ++i) {
-      A(dalloc(&h->d_Q[i], (size_t)N * H), "Q"); A(dalloc(&h->d_m[i], (size_t)N * H), "m");
-      A(dalloc(&h->d_v[i], (size_t)N * H), "v"); A(dalloc(&h->d_ages[i], (size_t)N), "ages");
+      A(h->d_Q[i].alloc((size_t)N * H), "Q"); A(h->d_m[i].alloc((size_t)N * H), "m");
+      A(h->d_v[i].alloc((size_t)N * H), "v"); A(h->d_ages[i].alloc((size_t)N), "ages");
     }
-    A(dalloc(&h->d_unom_log, (size_t)H), "unom_log"); A(dalloc(&h->d_ages_log, (size_t)N), "ages_log");
-    A(dalloc(&h->d_Q_log, (size_t)N * H), "Q_log");
-    A(dalloc(&h->d_best_idx, (size_t)N), "best_idx");
-    if (cfg->rpgd_gradient_mode >= 2) {  // gradient-assisted CEM: distribution + per-iteration elite log on top of the population
-      int iters = cfg->cem_outer_it;
-      if (cfg->cem_warmup && cfg->cem_warmup_iterations > iters) iters = cfg->cem_warmup_iterations;
-      if (!(cfg->rpgd_gradient_mode <= 3 && cfg->cem_best_k >= 1 && cfg->cem_best_k <= N && cfg->cem_outer_it >= 1 && h->period == 1 &&
-            iters >= 1)) {
-        ctk_destroy(h);
-        return fail(CTK_EINVAL, "gradient-assisted CEM needs 1 <= cem_best_k <= num_rollouts, cem_outer_it >= 1 and inducing-point period 1");
-      }
-      A(dalloc(&h->d_mu, (size_t)H), "mu"); A(dalloc(&h->d_sd, (size_t)H), "sd");
-      h->elite_log_cap = iters;
-      A(dalloc(&h->d_elite_idx, (size_t)iters * cfg->cem_best_k), "elite_idx");
-    }
+    A(h->d_unom_log.alloc((size_t)H), "unom_log"); A(h->d_ages_log.alloc((size_t)N), "ages_log");
+    A(h->d_Q_log.alloc((size_t)N * H), "Q_log");
+    A(h->d_best_idx.alloc((size_t)N), "best_idx");
   }
   if (rc == CTK_OK) A(upload_consts(h), "upload_consts");
-  if (rc == CTK_OK && B > 1 && !(h->ode_kernel && h->ode_ilp == 1))
-    rc = fail(CTK_EINVAL, "multi-client handles run the one-rollout-per-thread ODE kernel: intermediate_steps == 1, few inducing points, "
-                          "num_rollouts <= 1024 x SMs per client");
-  if (rc != CTK_OK) { std::string keep = g_err; ctk_destroy(h); g_err = keep; return rc; }
-  *out = h;
+  if (rc != CTK_OK) return rc;
+  *out = owner.release();
   return CTK_OK;
 }
 
@@ -449,6 +510,7 @@ extern "C" int ctk_set_cost_params(ctk_handle* h, const ctk_cost_params* c) {
   h->cost_p = *c;
   derive_cost(*c, h->H, h->cost);
   CU(cudaSetDevice(h->cfg.device));
+  derive_consts(h);
   CU(upload_consts(h));
   return CTK_OK;
 }
@@ -459,6 +521,7 @@ extern "C" int ctk_set_ode_params(ctk_handle* h, const ctk_ode_params* o) {
   derive_ode(*o, h->ode);
   derive_fwd(*o, h->fwd);
   CU(cudaSetDevice(h->cfg.device));
+  derive_consts(h);
   CU(upload_consts(h));
   return CTK_OK;
 }
@@ -466,6 +529,7 @@ extern "C" int ctk_set_ode_params(ctk_handle* h, const ctk_ode_params* o) {
 extern "C" int ctk_set_mlp_weights(ctk_handle* h, const ctk_mlp_weights* w) {
   REQ(h && w && w->W1 && w->b1 && w->W2 && w->b2 && w->W3 && w->b3, "null pointer");
   REQ(w->hidden >= 16 && w->hidden <= 128 && w->hidden % 16 == 0, "hidden must be a multiple of 16 in [16,128]");
+  REQ(h->cfg.predictor == CTK_PRED_MLP, "ctk_set_mlp_weights on a handle whose predictor is not CTK_PRED_MLP");
   CU(cudaSetDevice(h->cfg.device));
   const int hid = w->hidden, nf = mlp_blob_floats(hid);
   std::vector<float> blob((size_t)nf, 0.0f);
@@ -477,10 +541,8 @@ extern "C" int ctk_set_mlp_weights(ctk_handle* h, const ctk_mlp_weights* w) {
   for (int k = 0; k < 5; ++k) for (int j = 0; j < hid; ++j) p[k * hid + j] = w->W3[j * 5 + k];  // W3T[5][hid]
   p += 5 * hid;
   memcpy(p, w->b3, sizeof(float) * 5);
-  if (h->d_mlp) { cudaFree(h->d_mlp); h->d_mlp = nullptr; }
-  CU(dalloc(&h->d_mlp, (size_t)nf));
+  CU(h->d_mlp.alloc((size_t)nf));
   CU(cudaMemcpy(h->d_mlp, blob.data(), sizeof(float) * nf, cudaMemcpyHostToDevice));
-  REQ(h->cfg.predictor == CTK_PRED_MLP, "ctk_set_mlp_weights on a handle whose predictor is not CTK_PRED_MLP");
   h->mlp = MlpDev{hid, h->d_mlp, nf, nullptr, nullptr};
   if (h->cfg.mlp_engine != CTK_MLP_SIMT) {
     REQ(h->cfg.mlp_engine >= CTK_MLP_TCGEN05 && h->cfg.mlp_engine <= CTK_MLP_TCGEN05_FAST, "unknown mlp_engine");
@@ -534,8 +596,7 @@ extern "C" int ctk_set_mlp_weights(ctk_handle* h, const ctk_mlp_weights* w) {
         put(n, 36, c1); put(n, 37, c2); put(n, 38, bf16_rn(q2));
       }
     }
-    if (h->d_mlp_tc) { cudaFree(h->d_mlp_tc); h->d_mlp_tc = nullptr; }
-    CU(cudaMalloc(&h->d_mlp_tc, kTcBlobBytes));
+    CU(h->d_mlp_tc.alloc(kTcBlobBytes, false));
     CU(cudaMemcpy(h->d_mlp_tc, tc.data(), kTcBlobBytes, cudaMemcpyHostToDevice));
     h->mlp.tc_blob = h->d_mlp_tc;
   }
@@ -556,12 +617,11 @@ extern "C" int ctk_set_gru_weights(ctk_handle* h, const ctk_gru_weights* w) {
   for (int k = 0; k < 5; ++k) for (int j = 0; j < hid; ++j) p[k * hid + j] = w->W3[j * 5 + k];  // W3T[5][hid]
   p += 5 * hid;
   memcpy(p, w->b3, sizeof(float) * 5);
-  CU(cudaStreamSynchronize(h->stream));
-  if (h->d_mlp) { cudaFree(h->d_mlp); h->d_mlp = nullptr; }
-  if (h->d_rnn_h) { cudaFree(h->d_rnn_h); h->d_rnn_h = nullptr; }
-  CU(dalloc(&h->d_mlp, (size_t)nf));
+  CU(cudaStreamSynchronize(h->stream));  // kernels in flight may still read the old blob
+  h->d_rnn_h.reset();
+  CU(h->d_mlp.alloc((size_t)nf));
   CU(cudaMemcpy(h->d_mlp, blob.data(), sizeof(float) * nf, cudaMemcpyHostToDevice));
-  CU(dalloc(&h->d_rnn_h, (size_t)4 * hid));  // zero state (SI_Toolkit resets the RNN when the predictor is configured)
+  CU(h->d_rnn_h.alloc((size_t)4 * hid));  // zero state (SI_Toolkit resets the RNN when the predictor is configured)
   h->mlp = MlpDev{hid, h->d_mlp, nf, nullptr, h->d_rnn_h};
   return CTK_OK;
 }
@@ -577,11 +637,10 @@ extern "C" int ctk_push_injected_noise(ctk_handle* h, const float* z, size_t n) 
     // grow; pending kernels may still read the old buffer -> sync first
     CU(cudaStreamSynchronize(h->stream));
     const size_t cap = (h->inj_size + n) * 2;
-    float* nb = nullptr;
-    CU(cudaMalloc((void**)&nb, cap * sizeof(float)));
+    Owned<float> nb;
+    CU(nb.alloc(cap, false));
     if (h->inj_size) CU(cudaMemcpy(nb, h->d_inj, h->inj_size * sizeof(float), cudaMemcpyDeviceToDevice));
-    if (h->d_inj) cudaFree(h->d_inj);
-    h->d_inj = nb;
+    h->d_inj = std::move(nb);
     h->inj_cap = cap;
   }
   CU(cudaMemcpyAsync(h->d_inj + h->inj_size, z, n * sizeof(float), cudaMemcpyHostToDevice, h->stream));
@@ -609,43 +668,32 @@ static RpgdSelectArgs rpgd_sample_args(ctk_handle* h, NoiseSrc ns) {
   return a;
 }
 
+// Mid-range warm start of `rows` control rows, per input (optimizer_mppi.py:227-231, optimizer_cem_tf.py:113-117), flat [rows][nu].
+// The CartPole's limits are the config's (ctk_set_control_limits).
+static std::vector<float> mid_range(const ctk_handle* h, size_t rows) {
+  std::vector<float> v(rows * h->nu);
+  for (size_t t = 0; t < rows; ++t) for (int c = 0; c < h->nu; ++c) v[t * h->nu + c] = 0.5f * (h->lo_v[c] + h->hi_v[c]);
+  return v;
+}
+
 extern "C" int ctk_reset(ctk_handle* h) {
   REQ(h, "null handle");
   CU(cudaSetDevice(h->cfg.device));
-  if (h->env != 0) {  // per-input mid-range warm start (optimizer_mppi.py:227-231, optimizer_cem_tf.py:113-117), flat [H][nu]
-    std::vector<float> mid_v((size_t)h->H * h->nu), sd_v((size_t)h->H * h->nu, h->cfg.cem_initial_action_stdev);
-    for (int t = 0; t < h->H; ++t) for (int c = 0; c < h->nu; ++c) mid_v[(size_t)t * h->nu + c] = 0.5f * (h->lo_v[c] + h->hi_v[c]);
-    if (h->cfg.optimizer == CTK_OPT_MPPI) {
-      CU(cudaMemcpyAsync(h->d_u_nom, mid_v.data(), sizeof(float) * mid_v.size(), cudaMemcpyHostToDevice, h->stream));
-    } else {
-      CU(cudaMemcpyAsync(h->d_mu, mid_v.data(), sizeof(float) * mid_v.size(), cudaMemcpyHostToDevice, h->stream));
-      CU(cudaMemcpyAsync(h->d_sd, sd_v.data(), sizeof(float) * sd_v.size(), cudaMemcpyHostToDevice, h->stream));
-      CU(cudaMemsetAsync(h->d_u_prev, 0, sizeof(float) * h->nu, h->stream));  // only optimizer_cem_tf.optimizer_reset zeroes self.u (:117)
-      h->cem_it = 0;
-    }
-    CU(cudaStreamSynchronize(h->stream));
-    h->count = 0;
-    h->was_reset = true;
-    return CTK_OK;
-  }
-  const float mid = 0.5f * (h->cfg.action_low + h->cfg.action_high);
-  std::vector<float> tmp((size_t)h->H * h->nclients, mid);
+  const std::vector<float> mid = mid_range(h, (size_t)h->H * h->nclients), sd((size_t)h->H * h->nu, h->cfg.cem_initial_action_stdev);
   // self.u, the previous_input of the cost, is reset ONLY by optimizer_cem_tf.optimizer_reset (optimizer_cem_tf.py:117); MPPI (:227-231),
   // RPGD (:527-548), random-action, gradient-tf and the gradient-assisted CEM variants keep the last applied control
-  if (h->cfg.optimizer == CTK_OPT_CEM && !h->cfg.cem_uniform_actions) CU(cudaMemsetAsync(h->d_u_prev, 0, sizeof(float), h->stream));
+  if (h->cfg.optimizer == CTK_OPT_CEM && !h->cfg.cem_uniform_actions) CU(cudaMemsetAsync(h->d_u_prev, 0, sizeof(float) * h->nu, h->stream));
   if (h->cfg.optimizer == CTK_OPT_MPPI) {
-    CU(cudaMemcpyAsync(h->d_u_nom, tmp.data(), sizeof(float) * h->H * h->nclients, cudaMemcpyHostToDevice, h->stream));
+    CU(cudaMemcpyAsync(h->d_u_nom, mid.data(), sizeof(float) * mid.size(), cudaMemcpyHostToDevice, h->stream));
   } else if (h->cfg.optimizer == CTK_OPT_CEM) {
-    CU(cudaMemcpyAsync(h->d_mu, tmp.data(), sizeof(float) * h->H, cudaMemcpyHostToDevice, h->stream));
-    std::vector<float> sd((size_t)h->H, h->cfg.cem_initial_action_stdev);
-    CU(cudaMemcpyAsync(h->d_sd, sd.data(), sizeof(float) * h->H, cudaMemcpyHostToDevice, h->stream));
-    CU(cudaStreamSynchronize(h->stream));
+    CU(cudaMemcpyAsync(h->d_mu, mid.data(), sizeof(float) * mid.size(), cudaMemcpyHostToDevice, h->stream));
+    CU(cudaMemcpyAsync(h->d_sd, sd.data(), sizeof(float) * sd.size(), cudaMemcpyHostToDevice, h->stream));
+    if (h->env == 0) CU(cudaStreamSynchronize(h->stream));
     h->cem_it = 0;
   } else if (h->cfg.rpgd_gradient_mode >= 2) {
     // optimizer_cem_naive_grad_tf.py:116-119 / optimizer_cem_grad_bharadhwaj_tf.py:180-184: only the distribution (and count) is
     // reset; the Keras Adam slots of the bharadhwaj variant survive optimizer_reset()
-    CU(cudaMemcpyAsync(h->d_mu, tmp.data(), sizeof(float) * h->H, cudaMemcpyHostToDevice, h->stream));
-    std::vector<float> sd((size_t)h->H, h->cfg.cem_initial_action_stdev);
+    CU(cudaMemcpyAsync(h->d_mu, mid.data(), sizeof(float) * h->H, cudaMemcpyHostToDevice, h->stream));
     CU(cudaMemcpyAsync(h->d_sd, sd.data(), sizeof(float) * h->H, cudaMemcpyHostToDevice, h->stream));
     CU(cudaStreamSynchronize(h->stream));
   } else {
@@ -718,7 +766,7 @@ static int env_tick(ctk_handle* h, const S0e& s0, float* u_out_dev) {
     return CTK_OK;
   }
   // CEM: optimizer_cem_tf.py:83-111
-  const int iters = (c.cem_warmup && h->count == 0) ? c.cem_warmup_iterations : c.cem_outer_it;
+  const int iters = cem_tick_iters(h);
   if (iters < 1) return fail(CTK_EINVAL, "CEM iteration count < 1");
   h->elite_log_rows = 0;
   h->cem_iters = iters;
@@ -735,19 +783,10 @@ static int env_tick(ctk_handle* h, const S0e& s0, float* u_out_dev) {
       CU(launch_env_cem_rollout(h->env, c.logging != 0, a, h->stream));
     }
     h->last_kernel = std::string("env_cem_rollout_kernel<DubinsEnv,") + (c.logging ? "1" : "0") + ">" + (a.noise.inj ? " [injected noise]" : " [philox]");
-    // K4: hierarchical bitonic top-k (tf.argsort(...)[:k], ties -> lower index)
     const int k = c.cem_best_k;
-    int n = h->N, lvl = 0;
-    const float* cost = h->d_J;
+    int n = h->N;
     const uint64_t* kin = nullptr;
-    while (true) {
-      const int nb = (n + TOPK_THREADS - 1) / TOPK_THREADS;
-      uint64_t* outk = h->d_keys[lvl & 1];
-      h->launches++;
-      CU(launch_topk_level(cost, kin, n, h->off, k, outk, h->stream));
-      n = nb * k; cost = nullptr; kin = outk; ++lvl;
-      if (n <= TOPK_THREADS) break;
-    }
+    CU(topk_levels(h->d_J, kin, n, 0, h->off, k, false, h->d_keys[0], h->d_keys[1], h->stream, h->launches));
     EnvCemRefitArgs r{};
     r.H = h->H; r.nu = nu; r.k = k; r.cnt = n; r.cand = kin; r.noise = a.noise;
     for (int i = 0; i < kEnvMaxControls; ++i) { r.lo[i] = h->lo_v[i]; r.hi[i] = h->hi_v[i]; }
@@ -760,16 +799,6 @@ static int env_tick(ctk_handle* h, const S0e& s0, float* u_out_dev) {
     if (r.elite_idx_out) h->elite_log_rows++;
   }
   h->count++;
-  return CTK_OK;
-}
-
-// host-facing tick of a general environment: launch sequence, then ONE device->host copy of u (and the requested state array)
-static int env_step_host(ctk_handle* h, const float* s_host, float* u_out_host, const float* state_dev, float* state_out_host, size_t n_state) {
-  int rc = env_tick(h, make_s0e(h, nullptr, s_host), h->d_u_out);
-  if (rc != CTK_OK) return rc;
-  CU(cudaMemcpyAsync(u_out_host, h->d_u_out, sizeof(float) * h->nu, cudaMemcpyDeviceToHost, h->stream));
-  if (state_dev) CU(cudaMemcpyAsync(state_out_host, state_dev, n_state * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
-  CU(cudaStreamSynchronize(h->stream));
   return CTK_OK;
 }
 
@@ -789,6 +818,10 @@ static int pred_id(const ctk_handle* h) {
     case CTK_MLP_TCGEN05_FAST: return 4;
     default: return 1;
   }
+}
+static const char* pred_name(int pred) {  // the predictor functor of a rollout-kernel instantiation (last_kernel)
+  static const char* const names[] = {"OdePred", "MlpSimtPred", "MlpTcPred", "MlpTcBf16Pred", "MlpTcFastPred", "GruSimtPred", "MlpTcPredV1"};
+  return names[pred];
 }
 static size_t pred_smem_floats(ctk_handle* h) { return mppi_pred_smem_floats(pred_id(h), h->mlp); }
 
@@ -858,7 +891,7 @@ static int make_fuse(ctk_handle* h, int mode, float* u_out_dev, MppiFuse* out) {
   MppiFuse f{};
   f.mode = mode;
   f.world = 1; f.rank = 0; f.seq = 0;
-  if (mode != 0) { h->xseq++; if (h->xseq == 0) h->xseq = 1; }  // every shard ticks in lock step: the same sequence everywhere
+  if (mode != 0) next_seq(h->xseq);  // every shard ticks in lock step: the same sequence everywhere
   f.seq = h->xseq;
   f.record_out = h->d_record;
   f.mbox_local = h->d_mbox;
@@ -888,6 +921,18 @@ static int rnn_update(ctk_handle* h, const float* s_dev) {
   return CTK_OK;
 }
 
+static MppiOdeArgs mppi_ode_args(const ctk_handle* h, const S0& s0, const NoiseSrc& ns, const MppiFuse& fuse) {
+  MppiOdeArgs a{};
+  a.N = h->N; a.off = h->off; a.H = h->H; a.period = h->period; a.n_ind = h->n_ind;
+  a.fshare16 = h->ode_fshare16;
+  a.per16 = (double)h->N / (double)(h->ode_fshare16 + 16 * (h->ode_grid - 1));
+  a.trace = h->d_trace;
+  a.s0 = s0; a.u_nom = h->d_u_nom; a.u_prev = h->d_u_prev; a.noise = ns; a.k = h->ode_hot;
+  a.J = h->d_J; a.partials = h->d_partials; a.log_traj_soa = h->d_log_traj_soa; a.log_Q_soa = h->d_log_Q_soa;
+  a.fuse = fuse;
+  return a;
+}
+
 // mode 1: rollouts + shard record (staged exchange follows)   mode 2: whole tick incl. cross-GPU exchange and u_nom update
 static int mppi_local(ctk_handle* h, const float* s_dev, int mode, float* u_out_dev) {
   NoiseSrc ns{};
@@ -898,14 +943,7 @@ static int mppi_local(ctk_handle* h, const float* s_dev, int mode, float* u_out_
   MppiFuse fuse{};
   make_fuse(h, mode, u_out_dev, &fuse);
   if (h->ode_kernel) {
-    MppiOdeArgs a{};
-    a.N = h->N; a.off = h->off; a.H = h->H; a.period = h->period; a.n_ind = h->n_ind;
-    a.fshare16 = h->ode_fshare16;
-    a.per16 = (double)h->N / (double)(h->ode_fshare16 + 16 * (h->ode_grid - 1));
-    a.trace = h->d_trace;
-    a.s0 = make_s0(h, s_dev); a.u_nom = h->d_u_nom; a.u_prev = h->d_u_prev; a.noise = ns; a.k = h->ode_hot;
-    a.J = h->d_J; a.partials = h->d_partials; a.log_traj_soa = h->d_log_traj_soa; a.log_Q_soa = h->d_log_Q_soa;
-    a.fuse = fuse;
+    const MppiOdeArgs a = mppi_ode_args(h, make_s0(h, s_dev), ns, fuse);
     h->launches++;
     KernelTimer kt(h);
     const char* tail = "";
@@ -941,7 +979,7 @@ static int mppi_local(ctk_handle* h, const float* s_dev, int mode, float* u_out_
   if (tile_engine(pred_id(h)) && h->mlp.tc_blob == nullptr) return fail(CTK_ESTATE, "tcgen05 MLP engine without weights");
   cudaError_t e = launch_mppi_rollout(pred_id(h), h->cost.kind, log, h->mppi_grid, h->mppi_block, smem,
                                       h->stream, a);
-  h->last_kernel = std::string("mppi_rollout_kernel<") + (pred_id(h) == 5 ? "GruSimtPred" : pred_id(h) == 4 ? "MlpTcFastPred" : pred_id(h) == 3 ? "MlpTcBf16Pred" : pred_id(h) == 2 ? "MlpTcPred" : pred_id(h) == 6 ? "MlpTcPredV1" : pred_id(h) == 1 ? "MlpSimtPred" : "OdePred") + "," +
+  h->last_kernel = std::string("mppi_rollout_kernel<") + pred_name(pred_id(h)) + "," +
                    std::to_string(h->cost.kind) + "," + (log ? "1" : "0") + ">" + (ns.inj ? " [injected noise]" : " [philox]");
   if (e != cudaSuccess) return fail(CTK_ECUDA, std::string("mppi_rollout_kernel: ") + cudaGetErrorString(e));
   h->step_s = s_dev;
@@ -988,20 +1026,28 @@ static bool cem_persistent_ok(ctk_handle* h) {
   if (h->cem_tick_per_sm < 0) h->cem_tick_per_sm = cem_tick_blocks_per_sm(h->cost.kind, c.logging != 0, g.smem);
   return h->cem_tick_per_sm >= 1 && g.G <= h->cem_tick_per_sm * h->num_sms;  // every block must be resident: blocks wait for each other
 }
+// random shooting (cem_uniform_actions): Q = z (high - low) + low with z ~ U[0,1)  ==  the CEM sample clip(mu + z sd) with
+// mu = low, sd = high - low
+static int upload_uniform_dist(ctk_handle* h) {
+  const ctk_config& c = h->cfg;
+  std::vector<float> mu((size_t)h->H, c.action_low), sd((size_t)h->H, c.action_high - c.action_low);
+  CU(cudaMemcpyAsync(h->d_mu, mu.data(), sizeof(float) * h->H, cudaMemcpyHostToDevice, h->stream));
+  CU(cudaMemcpyAsync(h->d_sd, sd.data(), sizeof(float) * h->H, cudaMemcpyHostToDevice, h->stream));
+  CU(cudaStreamSynchronize(h->stream));  // mu / sd are stack-lifetime host vectors
+  return CTK_OK;
+}
 // returns 1 if the runtime refused the cooperative launch (grid not co-resident right now): nothing was consumed, the caller runs
 // the multi-launch path
 static int cem_tick_persistent(ctk_handle* h, const float* s_dev, float* u_out_dev) {
   const ctk_config& c = h->cfg;
   const size_t inj_pos0 = h->inj_pos;
   const unsigned int cem_seq0 = h->cem_seq;
-  const int iters = (c.cem_warmup && h->count == 0) ? c.cem_warmup_iterations : c.cem_outer_it;  // optimizer_cem_tf.py:92
+  const int iters = cem_tick_iters(h);
   if (iters < 1) return fail(CTK_EINVAL, "CEM iteration count < 1");
   const int uni = c.cem_uniform_actions ? 1 : 0;
-  if (uni) {  // random shooting: Q = z (high - low) + low  ==  the CEM sample clip(mu + z sd) with mu = low, sd = high - low
-    std::vector<float> mu((size_t)h->H, c.action_low), sd((size_t)h->H, c.action_high - c.action_low);
-    CU(cudaMemcpyAsync(h->d_mu, mu.data(), sizeof(float) * h->H, cudaMemcpyHostToDevice, h->stream));
-    CU(cudaMemcpyAsync(h->d_sd, sd.data(), sizeof(float) * h->H, cudaMemcpyHostToDevice, h->stream));
-    CU(cudaStreamSynchronize(h->stream));
+  if (uni) {
+    const int rc = upload_uniform_dist(h);
+    if (rc != CTK_OK) return rc;
   }
   CemTickArgs a{};
   for (int it = 0; it < iters; ++it) {  // one noise block per outer iteration: consecutive in the injected queue
@@ -1055,17 +1101,14 @@ static int cem_tick_persistent(ctk_handle* h, const float* s_dev, float* u_out_d
 static int cem_local(ctk_handle* h, const float* s_dev, bool to_k) {
   const ctk_config& c = h->cfg;
   if (h->cem_it == 0) {
-    h->cem_iters = (c.cem_warmup && h->count == 0) ? c.cem_warmup_iterations : c.cem_outer_it;  // optimizer_cem_tf.py:92
+    h->cem_iters = cem_tick_iters(h);
     if (h->cem_iters < 1) return fail(CTK_EINVAL, "CEM iteration count < 1");
     h->elite_log_rows = 0;
   }
   const int uni = c.cem_uniform_actions ? 1 : 0;
   if (uni && h->cem_it == 0) {
-    // random shooting: Q = z (high - low) + low with z ~ U[0,1)  ==  the CEM sample clip(mu + z sd) with mu = low, sd = high - low
-    std::vector<float> mu((size_t)h->H, c.action_low), sd((size_t)h->H, c.action_high - c.action_low);
-    CU(cudaMemcpyAsync(h->d_mu, mu.data(), sizeof(float) * h->H, cudaMemcpyHostToDevice, h->stream));
-    CU(cudaMemcpyAsync(h->d_sd, sd.data(), sizeof(float) * h->H, cudaMemcpyHostToDevice, h->stream));
-    CU(cudaStreamSynchronize(h->stream));  // mu / sd are stack-lifetime host vectors
+    const int rc = upload_uniform_dist(h);
+    if (rc != CTK_OK) return rc;
   }
   NoiseSrc ns{};
   int rcn = make_noise(h, STREAM_CEM | ((uint32_t)h->cem_it << 8), h->H, uni, (size_t)h->NG, &ns);
@@ -1096,28 +1139,14 @@ static int cem_local(ctk_handle* h, const float* s_dev, bool to_k) {
     KernelTimer kt(h);
     if (tile_engine(pred_id(h)) && h->mlp.tc_blob == nullptr) return fail(CTK_ESTATE, "tcgen05 MLP engine without weights");
     e = launch_cem_rollout(pred_id(h), h->cost.kind, c.logging != 0, cem_rollout_grid(pred_id(h), h->N, h->num_sms), smem, h->stream, a);
-    h->last_kernel = std::string("cem_rollout_kernel<") + (pred_id(h) == 5 ? "GruSimtPred" : pred_id(h) == 4 ? "MlpTcFastPred" : pred_id(h) == 3 ? "MlpTcBf16Pred" : pred_id(h) == 2 ? "MlpTcPred" : pred_id(h) == 6 ? "MlpTcPredV1" : pred_id(h) == 1 ? "MlpSimtPred" : "OdePred") + "," +
+    h->last_kernel = std::string("cem_rollout_kernel<") + pred_name(pred_id(h)) + "," +
                      std::to_string(h->cost.kind) + "," + (c.logging ? "1" : "0") + ">" + (ns.inj ? " [injected noise]" : " [philox]");
   }
   if (e != cudaSuccess) return fail(CTK_ECUDA, std::string("cem_rollout_kernel: ") + cudaGetErrorString(e));
-  // K4: hierarchical bitonic top-k
-  const int k = c.cem_best_k;
-  int n = h->N, lvl = 0;
-  const float* cost = h->d_J;
-  const uint64_t* kin = nullptr;
-  bool done = false;
-  if (fused_cand > 0) {
-    n = fused_cand; cost = nullptr; kin = h->d_keys[0]; lvl = 1;
-    done = n <= TOPK_THREADS && (!to_k || n == k);
-  }
-  while (!done) {
-    const int nb = (n + TOPK_THREADS - 1) / TOPK_THREADS;
-    uint64_t* outk = h->d_keys[lvl & 1];
-    h->launches++;
-    CU(launch_topk_level(cost, kin, n, h->off, k, outk, h->stream));
-    n = nb * k; cost = nullptr; kin = outk; ++lvl;
-    if (n <= TOPK_THREADS && (!to_k || nb == 1)) break;
-  }
+  int n = fused_cand > 0 ? fused_cand : h->N;
+  const uint64_t* kin = fused_cand > 0 ? h->d_keys[0].get() : nullptr;
+  CU(topk_levels(fused_cand > 0 ? nullptr : h->d_J.get(), kin, n, fused_cand > 0 ? 1 : 0, h->off, c.cem_best_k, to_k, h->d_keys[0], h->d_keys[1],
+                 h->stream, h->launches));
   h->cem_cand = n;
   h->cem_cand_ptr = const_cast<uint64_t*>(kin);
   return CTK_OK;
@@ -1132,9 +1161,7 @@ static int cem_finish(ctk_handle* h, const uint64_t* cand, int cnt, float* u_out
   if (fused && h->xworld > 1) {
     REQ(cnt == c.cem_best_k, "fused CEM exchange needs exactly k local candidates");
     a.world = h->xworld; a.rank = h->xrank;
-    h->xseq++;
-    if (h->xseq == 0) h->xseq = 1;
-    a.seq = h->xseq;
+    a.seq = next_seq(h->xseq);
     a.mbox_local = h->d_mbox;
     for (int r = 0; r < CTK_MAX_PEERS; ++r) a.mbox_peer[r] = h->mbox_peer[r];
   }
@@ -1168,7 +1195,7 @@ static int gradcem_tick(ctk_handle* h, const float* s_dev, float* u_out_dev) {
   const ctk_config& c = h->cfg;
   const bool carry = c.rpgd_gradient_mode == 3;
   const int N = h->N, H = h->H, k = c.cem_best_k;
-  const int iters = (carry && c.cem_warmup && h->count == 0) ? c.cem_warmup_iterations : c.cem_outer_it;
+  const int iters = carry ? cem_tick_iters(h) : c.cem_outer_it;
   const int kc = carry ? k : 0;
   auto sample = [&](int col0, int cnt, uint32_t sub) -> int {
     if (cnt <= 0) return CTK_OK;
@@ -1208,7 +1235,7 @@ static int gradcem_tick(ctk_handle* h, const float* s_dev, float* u_out_dev) {
     const bool last = it == iters - 1;
     if (last && c.logging) CU(cudaMemcpyAsync(h->d_Q_log, h->d_Q[h->cur], sizeof(float) * N * H, cudaMemcpyDeviceToDevice, h->stream));
     GradCemRefitArgs r{};
-    r.N = N; r.H = H; r.k = k; r.J = h->d_J; r.Q = h->d_Q[h->cur]; r.Q_carry = carry ? h->d_Q[h->cur ^ 1] : nullptr;
+    r.N = N; r.H = H; r.k = k; r.J = h->d_J; r.Q = h->d_Q[h->cur]; r.Q_carry = carry ? h->d_Q[h->cur ^ 1].get() : nullptr;
     r.mu = h->d_mu; r.sd = h->d_sd; r.last = last ? 1 : 0; r.u_from_mean = carry ? 0 : 1;
     r.sd_min = c.cem_stdev_min; r.sd_init = c.cem_initial_action_stdev; r.mid = 0.5f * (c.action_low + c.action_high);
     r.u_prev = h->d_u_prev; r.u_out = u_out_dev; r.freeze_prev = c.freeze_previous_input;
@@ -1315,13 +1342,42 @@ static int rpgd_tick(ctk_handle* h, const float* s_dev, float* u_out_dev) {
   return CTK_OK;
 }
 
-extern "C" int ctk_step_local(ctk_handle* h, const float* s_dev) {
-  REQ(h && s_dev, "null pointer");
-  REQ(h->env == 0, "the staged (sharded) tick is implemented for the CartPole environment");
+// Preconditions of every tick entry point
+static int tick_ready(ctk_handle* h) {
   if (!h->was_reset) return fail(CTK_ESTATE, "ctk_step before ctk_reset");
   CU(cudaSetDevice(h->cfg.device));
   if (h->cfg.predictor != CTK_PRED_ODE && h->mlp.blob == nullptr) return fail(CTK_ESTATE, "network predictor without weights (ctk_set_mlp_weights / ctk_set_gru_weights)");
-  int rc;
+  return CTK_OK;
+}
+
+// One whole tick, enqueued.  The state is s_dev (device) or, s_dev == nullptr, s_host: a general environment takes it from there,
+// the CartPole kernels from h_pin, where the caller has put it.
+static int run_tick(ctk_handle* h, const float* s_dev, const float* s_host, float* u_out_dev) {
+  int rc = tick_ready(h);
+  if (rc != CTK_OK) return rc;
+  if (h->env != 0) return env_tick(h, make_s0e(h, s_dev, s_host), u_out_dev);
+  h->tick++;
+  switch (h->cfg.optimizer) {
+    case CTK_OPT_MPPI:
+      return mppi_local(h, s_dev, 2, u_out_dev);
+    case CTK_OPT_CEM:
+      rc = cem_persistent_ok(h) ? cem_tick_persistent(h, s_dev, u_out_dev) : 1;
+      if (rc == 1) do {
+        rc = cem_local(h, s_dev, h->xworld > 1);
+        if (rc != CTK_OK) break;
+        rc = cem_finish(h, h->cem_cand_ptr, h->cem_cand, u_out_dev, h->xworld > 1);
+      } while (rc == CTK_OK && h->cem_it != 0);
+      return rc;
+    default:
+      return rpgd_tick(h, s_dev, u_out_dev);
+  }
+}
+
+extern "C" int ctk_step_local(ctk_handle* h, const float* s_dev) {
+  REQ(h && s_dev, "null pointer");
+  REQ(h->env == 0, "the staged (sharded) tick is implemented for the CartPole environment");
+  int rc = tick_ready(h);
+  if (rc != CTK_OK) return rc;
   switch (h->cfg.optimizer) {
     case CTK_OPT_MPPI:
       h->tick++;
@@ -1379,7 +1435,7 @@ extern "C" int ctk_step_state(ctk_handle* h, const float* s_host, float* u_out_h
 // mirror (value | sequence number, one 8-byte store each: host_put in ctk_device.cuh).  Polling pinned host memory replaces
 // cudaStreamSynchronize + the device->host copies (measured: ~15 us per step).
 static int wait_host_slots(ctk_handle* h, unsigned int seq, int first, int count, float* out) {
-  volatile unsigned long long* slots = reinterpret_cast<volatile unsigned long long*>(h->h_pin);
+  volatile unsigned long long* slots = reinterpret_cast<volatile unsigned long long*>(h->h_pin.get());
   const auto t0 = std::chrono::steady_clock::now();
   unsigned int spins = 0;
   for (int i = 0; i < count; ++i) {
@@ -1413,34 +1469,21 @@ static int wait_host_slots(ctk_handle* h, unsigned int seq, int first, int count
 // written by the tick's last kernel: no cudaMemcpy and no stream synchronisation on this path.
 static int step_host(ctk_handle* h, const float* s_host, float* u_out_host, const float* state_dev, float* state_out_host, size_t n_state) {
   REQ(h && s_host && u_out_host, "null pointer");
-  if (!h->was_reset) return fail(CTK_ESTATE, "ctk_step before ctk_reset");
-  CU(cudaSetDevice(h->cfg.device));
-  if (h->env != 0) return env_step_host(h, s_host, u_out_host, state_dev, state_out_host, n_state);
-  if (h->cfg.predictor != CTK_PRED_ODE && h->mlp.blob == nullptr) return fail(CTK_ESTATE, "network predictor without weights (ctk_set_mlp_weights / ctk_set_gru_weights)");
+  if (h->env != 0) {  // general environments: the launch sequence, then ONE device->host copy of u (and the requested state array)
+    int rc = run_tick(h, nullptr, s_host, h->d_u_out);
+    if (rc != CTK_OK) return rc;
+    CU(cudaMemcpyAsync(u_out_host, h->d_u_out, sizeof(float) * h->nu, cudaMemcpyDeviceToHost, h->stream));
+    if (state_dev) CU(cudaMemcpyAsync(state_out_host, state_dev, n_state * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    return CTK_OK;
+  }
   memcpy(h->h_pin, s_host, sizeof(float) * 6);
   // the mirror carries one [H] array: MPPI's u_nom / RPGD's best sequence; any other state array takes the copy path below
   const bool state_in_mirror = state_dev != nullptr && h->cfg.rpgd_gradient_mode < 2 &&
                                ((h->cfg.optimizer == CTK_OPT_MPPI && state_dev == h->d_u_nom) ||
                                 (h->cfg.optimizer == CTK_OPT_RPGD && state_dev == h->d_unom_log));
-  h->hseq++;
-  if (h->hseq == 0) h->hseq = 1;
-  h->mirror = HostMirror{h->d_pin, h->hseq};
-  int rc = CTK_OK;
-  if (h->cfg.optimizer == CTK_OPT_MPPI) {
-    h->tick++;
-    rc = mppi_local(h, nullptr, 2, h->d_u_out);
-  } else if (h->cfg.optimizer == CTK_OPT_CEM) {
-    h->tick++;
-    rc = cem_persistent_ok(h) ? cem_tick_persistent(h, nullptr, h->d_u_out) : 1;
-    if (rc == 1) do {
-      rc = cem_local(h, nullptr, h->xworld > 1);
-      if (rc != CTK_OK) break;
-      rc = cem_finish(h, h->cem_cand_ptr, h->cem_cand, h->d_u_out, h->xworld > 1);
-    } while (rc == CTK_OK && h->cem_it != 0);
-  } else {
-    h->tick++;
-    rc = rpgd_tick(h, nullptr, h->d_u_out);
-  }
+  h->mirror = HostMirror{h->d_pin, next_seq(h->hseq)};
+  int rc = run_tick(h, nullptr, s_host, h->d_u_out);
   h->mirror = HostMirror{nullptr, 0};
   if (rc != CTK_OK) return rc;
   float us[2];  // u, status
@@ -1470,27 +1513,8 @@ static int step_host(ctk_handle* h, const float* s_host, float* u_out_host, cons
 // calls this once per tick and ends up with the same u_nom / u.
 extern "C" int ctk_step_device(ctk_handle* h, const float* s_dev, float* u_out_dev) {
   REQ(h && s_dev, "null pointer");
-  if (!h->was_reset) return fail(CTK_ESTATE, "ctk_step before ctk_reset");
   REQ(h->cfg.optimizer != CTK_OPT_RPGD || h->xworld == 1, "RPGD is replicas-only (no cross-GPU exchange)");
-  CU(cudaSetDevice(h->cfg.device));
-  if (h->cfg.predictor != CTK_PRED_ODE && h->mlp.blob == nullptr) return fail(CTK_ESTATE, "network predictor without weights (ctk_set_mlp_weights / ctk_set_gru_weights)");
-  float* uo = u_out_dev ? u_out_dev : h->d_u_out;
-  if (h->env != 0) return env_tick(h, make_s0e(h, s_dev, nullptr), uo);  // u_out_dev [nu]
-  int rc = CTK_OK;
-  h->tick++;
-  if (h->cfg.optimizer == CTK_OPT_MPPI) {
-    rc = mppi_local(h, s_dev, 2, uo);
-  } else if (h->cfg.optimizer == CTK_OPT_CEM) {
-    rc = cem_persistent_ok(h) ? cem_tick_persistent(h, s_dev, uo) : 1;
-    if (rc == 1) do {
-      rc = cem_local(h, s_dev, h->xworld > 1);
-      if (rc != CTK_OK) break;
-      rc = cem_finish(h, h->cem_cand_ptr, h->cem_cand, uo, h->xworld > 1);
-    } while (rc == CTK_OK && h->cem_it != 0);
-  } else {
-    rc = rpgd_tick(h, s_dev, uo);
-  }
-  return rc;
+  return run_tick(h, s_dev, nullptr, u_out_dev ? u_out_dev : h->d_u_out.get());  // general environments: u_out_dev [nu]
 }
 
 // n ticks back to back on the handle's stream: tick i reads its state from s_dev + i * s_stride (device memory) and writes
@@ -1541,14 +1565,8 @@ extern "C" int ctk_step_batch(ctk_handle* h, const float* s_host, const int32_t*
   make_fuse(h, 2, h->d_u_out, &fuse);
   fuse.host = HostMirror{nullptr, 0};
   fuse.handover = nullptr;  // (no chained tick follows a batch launch)
-  MppiOdeArgs a{};
-  a.N = h->N; a.off = h->off; a.H = h->H; a.period = h->period; a.n_ind = h->n_ind;
-  a.fshare16 = h->ode_fshare16;
-  a.per16 = (double)h->N / (double)(h->ode_fshare16 + 16 * (h->ode_grid - 1));
+  MppiOdeArgs a = mppi_ode_args(h, S0{}, nsrc, fuse);  // logging is off: no log buffers
   a.trace = nullptr;
-  a.s0 = S0{}; a.u_nom = h->d_u_nom; a.u_prev = h->d_u_prev; a.noise = nsrc; a.k = h->ode_hot;
-  a.J = h->d_J; a.partials = h->d_partials; a.log_traj_soa = nullptr; a.log_Q_soa = nullptr;
-  a.fuse = fuse;
   b.stride_unom = (size_t)h->H; b.stride_J = (size_t)h->N; b.stride_partials = h->partials_stride;
   b.stride_record = (size_t)h->n_ind + 2; b.stride_mbox = h->mbox_stride;
   h->launches++;
@@ -1574,8 +1592,7 @@ extern "C" int ctk_reset_client(ctk_handle* h, int client) {
   REQ(h && client >= 0 && client < h->nclients, "no such client slot");
   REQ(h->cfg.optimizer == CTK_OPT_MPPI, "multi-client handles are MPPI handles");
   CU(cudaSetDevice(h->cfg.device));
-  const float mid = 0.5f * (h->cfg.action_low + h->cfg.action_high);
-  std::vector<float> tmp((size_t)h->H, mid);
+  const std::vector<float> tmp = mid_range(h, (size_t)h->H);
   CU(cudaMemcpyAsync(h->d_u_nom + (size_t)client * h->H, tmp.data(), sizeof(float) * h->H, cudaMemcpyHostToDevice, h->stream));
   CU(cudaMemsetAsync(h->d_u_prev + client, 0, sizeof(float), h->stream));
   CU(cudaStreamSynchronize(h->stream));
@@ -1601,10 +1618,7 @@ static int exchange_reset(ctk_handle* h, int rank, int world) {
   REQ(world >= 1 && world <= CTK_MAX_PEERS && rank >= 0 && rank < world, "need 0 <= rank < world <= 8");
   REQ(h->cfg.optimizer != CTK_OPT_CEM || (long long)world * h->cfg.cem_best_k <= TOPK_THREADS, "sharded CEM: world x cem_best_k must be <= 1024");
   CU(cudaStreamSynchronize(h->stream));
-  for (int r = 0; r < CTK_MAX_PEERS; ++r) {
-    if (h->mbox_ipc[r] && h->mbox_peer[r]) cudaIpcCloseMemHandle(h->mbox_peer[r]);
-    h->mbox_peer[r] = nullptr; h->mbox_ipc[r] = false;
-  }
+  h->close_peers();
   h->xworld = world; h->xrank = rank; h->xseq = 0;
   h->bseq = 0;
   CU(cudaMemset(h->d_mbox, 0, sizeof(unsigned long long) * (h->cfg.optimizer == CTK_OPT_CEM ? cem_mbox_slots() : mbox_total_slots(h->n_ind, h->H))));
@@ -1638,9 +1652,7 @@ extern "C" int ctk_exchange_barrier(ctk_handle* h) {
   CU(cudaSetDevice(h->cfg.device));
   MppiFuse f{};
   f.world = h->xworld; f.rank = h->xrank;
-  h->bseq++;
-  if (h->bseq == 0) h->bseq = 1;
-  f.seq = h->bseq;
+  f.seq = next_seq(h->bseq);
   f.mbox_local = h->d_mbox;
   for (int r = 0; r < CTK_MAX_PEERS; ++r) f.mbox_peer[r] = h->mbox_peer[r];
   h->launches++;
@@ -1706,16 +1718,13 @@ extern "C" int ctk_get_state(ctk_handle* h, int which, float* dst, size_t n) {
   if (rc != CTK_OK) return rc;
   REQ(n == cnt, "size mismatch");
   if (tm) {
-    float* tmp = nullptr;
-    CU(cudaMalloc((void**)&tmp, cnt * sizeof(float)));
+    Owned<float> tmp;
+    CU(tmp.alloc(cnt, false));
     rc = transpose_dev(h, p, tmp, h->H, h->N);  // [H][N] -> [N][H]
-    if (rc == CTK_OK) {
-      cudaError_t e = cudaMemcpyAsync(dst, tmp, cnt * sizeof(float), cudaMemcpyDeviceToHost, h->stream);
-      if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-      cudaFree(tmp);
-      CU(e);
-    } else cudaFree(tmp);
-    return rc;
+    if (rc != CTK_OK) return rc;
+    CU(cudaMemcpyAsync(dst, tmp, cnt * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    return CTK_OK;
   }
   CU(cudaMemcpyAsync(dst, p, cnt * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
   CU(cudaStreamSynchronize(h->stream));
@@ -1730,12 +1739,11 @@ extern "C" int ctk_set_state(ctk_handle* h, int which, const float* src, size_t 
   if (rc != CTK_OK) return rc;
   REQ(n == cnt, "size mismatch");
   if (tm) {
-    float* tmp = nullptr;
-    CU(cudaMalloc((void**)&tmp, cnt * sizeof(float)));
-    cudaError_t e = cudaMemcpyAsync(tmp, src, cnt * sizeof(float), cudaMemcpyHostToDevice, h->stream);
-    if (e == cudaSuccess) { rc = transpose_dev(h, tmp, p, h->N, h->H); e = cudaStreamSynchronize(h->stream); }
-    cudaFree(tmp);
-    CU(e);
+    Owned<float> tmp;
+    CU(tmp.alloc(cnt, false));
+    CU(cudaMemcpyAsync(tmp, src, cnt * sizeof(float), cudaMemcpyHostToDevice, h->stream));
+    rc = transpose_dev(h, tmp, p, h->N, h->H);
+    CU(cudaStreamSynchronize(h->stream));
     return rc;
   }
   CU(cudaMemcpyAsync(p, src, cnt * sizeof(float), cudaMemcpyHostToDevice, h->stream));
@@ -1810,8 +1818,8 @@ extern "C" int ctk_debug_trace(ctk_handle* h, int enable, uint64_t* out_host, si
     }
   }
   if (grid_out) *grid_out = h->ode_grid;
-  if (enable && !h->d_trace) { CU(cudaMalloc((void**)&h->d_trace, n * sizeof(uint64_t))); CU(cudaMemset(h->d_trace, 0, n * sizeof(uint64_t))); }
-  if (!enable && h->d_trace) { cudaFree(h->d_trace); h->d_trace = nullptr; }
+  if (enable && !h->d_trace) CU(h->d_trace.alloc(n));
+  if (!enable) h->d_trace.reset();
   return CTK_OK;
 }
 // instantiation of the last rollout-kernel launch of this handle, e.g. "mppi_ode_kernel<0,0,10,2,896,0>" (verification: the parity
@@ -1884,8 +1892,9 @@ extern "C" int ctk_get_log_view(ctk_handle* h, int which, const void** host_ptr,
   int rc = log_source(h, which, &src, &need);
   if (rc != CTK_OK) return rc;
   if (h->h_log_cap[which] < need) {
-    if (h->h_log[which]) { CU(cudaStreamSynchronize(h->stream)); cudaFreeHost(h->h_log[which]); h->h_log[which] = nullptr; h->h_log_cap[which] = 0; }
-    CU(cudaHostAlloc(&h->h_log[which], need ? need : 4, cudaHostAllocDefault));
+    if (h->h_log[which]) CU(cudaStreamSynchronize(h->stream));
+    h->h_log_cap[which] = 0;
+    CU(h->h_log[which].alloc(need ? need : 4, false));
     h->h_log_cap[which] = need;
   }
   CU(cudaMemcpyAsync(h->h_log[which], src, need, cudaMemcpyDeviceToHost, h->stream));
@@ -1908,32 +1917,22 @@ extern "C" int ctk_get_log_top(ctk_handle* h, int m, int32_t* idx_out, float* J_
   const size_t RQ = H * h->nu, RT = (H + 1) * h->ns;
   const size_t nk = (size_t)((N + TOPK_THREADS - 1) / TOPK_THREADS) * m + TOPK_THREADS;
   if (h->top_keys_cap < nk) {
-    for (int i = 0; i < 2; ++i) { if (h->d_top_keys[i]) cudaFree(h->d_top_keys[i]); h->d_top_keys[i] = nullptr; }
     h->top_keys_cap = 0;
-    CU(dalloc(&h->d_top_keys[0], nk));
-    CU(dalloc(&h->d_top_keys[1], nk));
+    CU(h->d_top_keys[0].alloc(nk));
+    CU(h->d_top_keys[1].alloc(nk));
     h->top_keys_cap = nk;
   }
   const size_t no = (size_t)m * (RQ + RT + 2);
   if (h->top_out_cap < no) {
-    if (h->d_top_out) cudaFree(h->d_top_out);
-    if (h->h_top) cudaFreeHost(h->h_top);
-    h->d_top_out = nullptr; h->h_top = nullptr; h->top_out_cap = 0;
-    CU(dalloc(&h->d_top_out, no));
-    CU(cudaHostAlloc((void**)&h->h_top, no * sizeof(float), cudaHostAllocDefault));
+    h->top_out_cap = 0;
+    CU(h->d_top_out.alloc(no));
+    CU(h->h_top.alloc(no, false));
     h->top_out_cap = no;
   }
   // K4 levels over the costs of the last tick (global ids: shard offset + local index)
-  int cnt = (int)N, lvl = 0;
-  const float* cost = h->d_J;
+  int cnt = (int)N;
   const uint64_t* kin = nullptr;
-  for (;;) {
-    const int nb = (cnt + TOPK_THREADS - 1) / TOPK_THREADS;
-    h->launches++;
-    CU(launch_topk_level(cost, kin, cnt, h->off, m, h->d_top_keys[lvl & 1], h->stream));
-    kin = h->d_top_keys[lvl & 1]; cost = nullptr; cnt = nb * m; ++lvl;
-    if (nb == 1) break;
-  }
+  CU(topk_levels(h->d_J, kin, cnt, 0, h->off, m, true, h->d_top_keys[0], h->d_top_keys[1], h->stream, h->launches));
   float* d_Q = h->d_top_out;                       // [m][H nu]
   float* d_T = d_Q + (size_t)m * RQ;               // [m][(H+1) ns]
   float* d_Jm = d_T + (size_t)m * RT;              // [m]
@@ -1967,22 +1966,17 @@ extern "C" int ctk_rollout_single(ctk_handle* h, const float* s_host, const floa
   REQ(h->env == 0, "the standalone nominal rollout is implemented for the CartPole environment");
   CU(cudaSetDevice(h->cfg.device));
   const int H = h->H;
-  float* d = nullptr;
-  const size_t n = 8 + H + (size_t)(H + 1) * 6 + 1;
-  CU(cudaMalloc((void**)&d, n * sizeof(float)));
-  float *d_s = d, *d_Q = d + 8, *d_traj = d_Q + H, *d_sum = d_traj + (size_t)(H + 1) * 6;
-  cudaError_t e = cudaMemcpyAsync(d_s, s_host, 6 * sizeof(float), cudaMemcpyHostToDevice, h->stream);
-  if (e == cudaSuccess) e = cudaMemcpyAsync(d_Q, Q_host, H * sizeof(float), cudaMemcpyHostToDevice, h->stream);
-  if (e == cudaSuccess) {
-    h->launches++;
-    e = launch_single_rollout(h->cfg.predictor == CTK_PRED_ODE ? 0 : (h->cfg.predictor == CTK_PRED_GRU ? 5 : 1), d_s, d_Q, H, h->d_kc, h->mlp, h->d_u_prev, d_traj,
-                              d_sum, h->stream);
-  }
+  Owned<float> d;
+  CU(d.alloc(8 + H + (size_t)(H + 1) * 6 + 1, false));
+  float *d_s = d, *d_Q = d_s + 8, *d_traj = d_Q + H, *d_sum = d_traj + (size_t)(H + 1) * 6;
+  CU(cudaMemcpyAsync(d_s, s_host, 6 * sizeof(float), cudaMemcpyHostToDevice, h->stream));
+  CU(cudaMemcpyAsync(d_Q, Q_host, H * sizeof(float), cudaMemcpyHostToDevice, h->stream));
+  h->launches++;
+  CU(launch_single_rollout(h->cfg.predictor == CTK_PRED_ODE ? 0 : (h->cfg.predictor == CTK_PRED_GRU ? 5 : 1), d_s, d_Q, H, h->d_kc, h->mlp, h->d_u_prev, d_traj,
+                           d_sum, h->stream));
   std::vector<float> tmp((size_t)(H + 1) * 6 + 1);
-  if (e == cudaSuccess) e = cudaMemcpyAsync(tmp.data(), d_traj, tmp.size() * sizeof(float), cudaMemcpyDeviceToHost, h->stream);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-  cudaFree(d);
-  CU(e);
+  CU(cudaMemcpyAsync(tmp.data(), d_traj, tmp.size() * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaStreamSynchronize(h->stream));
   memcpy(traj_host, tmp.data(), sizeof(float) * (size_t)(H + 1) * 6);
   if (summed) *summed = tmp.back();
   return CTK_OK;
@@ -1997,8 +1991,8 @@ extern "C" int ctk_fp32_peak(int device, double* tflops, double* clk_mhz) {
   cudaDeviceProp prop;
   CU(cudaGetDeviceProperties(&prop, device));
   const int blocks = prop.multiProcessorCount * 8, threads = 256, iters = 4096;
-  float* d = nullptr;
-  CU(cudaMalloc((void**)&d, sizeof(float) * blocks * threads));
+  Owned<float> d;
+  CU(d.alloc((size_t)blocks * threads, false));
   cudaEvent_t e0, e1;
   CU(cudaEventCreate(&e0)); CU(cudaEventCreate(&e1));
   double best = 0.0;
@@ -2013,7 +2007,6 @@ extern "C" int ctk_fp32_peak(int device, double* tflops, double* clk_mhz) {
     if (rep > 0) best = std::max(best, fl / (ms * 1e-3) / 1e12);
   }
   cudaEventDestroy(e0); cudaEventDestroy(e1);
-  cudaFree(d);
   *tflops = best;
   if (clk_mhz) *clk_mhz = best * 1e12 / (2.0 * 128.0 * prop.multiProcessorCount) / 1e6;  // implied FFMA issue clock
   return CTK_OK;
@@ -2026,9 +2019,9 @@ extern "C" int ctk_fp32_microbench(int device, int variant, double* ginstr_per_s
   cudaDeviceProp prop;
   CU(cudaGetDeviceProperties(&prop, device));
   const int blocks = prop.multiProcessorCount * 8, threads = 256, iters = 2048;
-  float *d = nullptr, *seed = nullptr;
-  CU(cudaMalloc((void**)&d, sizeof(float) * blocks * threads));
-  CU(cudaMalloc((void**)&seed, sizeof(float) * 64));
+  Owned<float> d, seed;
+  CU(d.alloc((size_t)blocks * threads, false));
+  CU(seed.alloc(64, false));
   float hs[64];
   for (int i = 0; i < 64; ++i) hs[i] = 0.5f + 0.001f * i;
   CU(cudaMemcpy(seed, hs, sizeof(hs), cudaMemcpyHostToDevice));
@@ -2046,7 +2039,6 @@ extern "C" int ctk_fp32_microbench(int device, int variant, double* ginstr_per_s
     if (rep > 0) best = std::max(best, ninstr / (ms * 1e-3) / 1e9);
   }
   cudaEventDestroy(e0); cudaEventDestroy(e1);
-  cudaFree(d); cudaFree(seed);
   *ginstr_per_s = best;
   return CTK_OK;
 }
@@ -2054,15 +2046,13 @@ extern "C" int ctk_fp32_microbench(int device, int variant, double* ginstr_per_s
 extern "C" int ctk_philox_fill(int device, uint64_t seed, int kind, float* dst, size_t n) {
   REQ(dst, "null pointer");
   CU(cudaSetDevice(device));
-  float* d = nullptr;
-  CU(cudaMalloc((void**)&d, sizeof(float) * (n ? n : 1)));
+  Owned<float> d;
+  CU(d.alloc(n, false));
   NoiseSrc ns{};
   ns.inj = nullptr; ns.key0 = (uint32_t)seed; ns.key1 = (uint32_t)(seed >> 32); ns.tick = 1; ns.stream = STREAM_MPPI;
   ns.per_rollout = 16; ns.uniform = kind;
-  cudaError_t e = launch_philox_fill(ns, d, n, nullptr);
-  if (e == cudaSuccess) e = cudaMemcpy(dst, d, sizeof(float) * n, cudaMemcpyDeviceToHost);
-  cudaFree(d);
-  CU(e);
+  CU(launch_philox_fill(ns, d, n, nullptr));
+  CU(cudaMemcpy(dst, d, sizeof(float) * n, cudaMemcpyDeviceToHost));
   return CTK_OK;
 }
 
@@ -2081,37 +2071,30 @@ extern "C" int ctk_philox_export(ctk_handle* h, uint32_t stream, int64_t tick, i
   NoiseSrc ns{};
   ns.inj = nullptr; ns.key0 = (uint32_t)(h->cfg.seed & 0xffffffffull); ns.key1 = (uint32_t)(h->cfg.seed >> 32);
   ns.tick = (uint32_t)tick; ns.stream = stream; ns.per_rollout = per_rollout; ns.uniform = uniform ? 1 : 0;
-  float* d = nullptr;
-  CU(cudaMalloc((void**)&d, sizeof(float) * n));
-  cudaError_t e = launch_philox_export(ns, row0, d, n, h->stream);
-  if (e == cudaSuccess) e = cudaMemcpyAsync(dst_host, d, sizeof(float) * n, cudaMemcpyDeviceToHost, h->stream);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-  cudaFree(d);
-  CU(e);
+  Owned<float> d;
+  CU(d.alloc(n, false));
+  CU(launch_philox_export(ns, row0, d, n, h->stream));
+  CU(cudaMemcpyAsync(dst_host, d, sizeof(float) * n, cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaStreamSynchronize(h->stream));
   return CTK_OK;
 }
 
 extern "C" int ctk_topk(int device, const float* cost_host, int n, int k, int32_t* idx_out) {
   REQ(cost_host && idx_out && n >= 1 && k >= 1 && k <= n && k <= 512, "need 1 <= k <= min(n, 512)");
   CU(cudaSetDevice(device));
-  float* d_c = nullptr; uint64_t *d_k0 = nullptr, *d_k1 = nullptr;
+  Owned<float> d_c;
+  Owned<uint64_t> d_k0, d_k1;
   const size_t nk = (size_t)((n + 1023) / 1024) * k + 1024;
-  CU(cudaMalloc((void**)&d_c, sizeof(float) * n));
-  CU(cudaMalloc((void**)&d_k0, sizeof(uint64_t) * nk));
-  CU(cudaMalloc((void**)&d_k1, sizeof(uint64_t) * nk));
-  cudaError_t e = cudaMemcpy(d_c, cost_host, sizeof(float) * n, cudaMemcpyHostToDevice);
-  uint64_t* bufs[2] = {d_k0, d_k1};
-  int cnt = n, lvl = 0; const float* cost = d_c; const uint64_t* kin = nullptr;
-  while (e == cudaSuccess) {
-    const int nb = (cnt + TOPK_THREADS - 1) / TOPK_THREADS;
-    e = launch_topk_level(cost, kin, cnt, 0, k, bufs[lvl & 1], nullptr);
-    kin = bufs[lvl & 1]; cost = nullptr; cnt = nb * k; ++lvl;
-    if (nb == 1) break;
-  }
+  CU(d_c.alloc(n, false));
+  CU(d_k0.alloc(nk, false));
+  CU(d_k1.alloc(nk, false));
+  CU(cudaMemcpy(d_c, cost_host, sizeof(float) * n, cudaMemcpyHostToDevice));
+  int cnt = n;
+  const uint64_t* kin = nullptr;
+  int64_t launches = 0;  // no handle to count them on
+  CU(topk_levels(d_c, kin, cnt, 0, 0, k, true, d_k0, d_k1, nullptr, launches));
   std::vector<uint64_t> keys((size_t)k);
-  if (e == cudaSuccess) e = cudaMemcpy(keys.data(), kin, sizeof(uint64_t) * k, cudaMemcpyDeviceToHost);
-  cudaFree(d_c); cudaFree(d_k0); cudaFree(d_k1);
-  CU(e);
+  CU(cudaMemcpy(keys.data(), kin, sizeof(uint64_t) * k, cudaMemcpyDeviceToHost));
   for (int i = 0; i < k; ++i) idx_out[i] = (int32_t)(keys[i] & 0xffffffffu);
   return CTK_OK;
 }

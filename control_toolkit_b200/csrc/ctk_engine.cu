@@ -530,6 +530,13 @@ extern "C" int ctk_set_mlp_weights(ctk_handle* h, const ctk_mlp_weights* w) {
   REQ(h && w && w->W1 && w->b1 && w->W2 && w->b2 && w->W3 && w->b3, "null pointer");
   REQ(w->hidden >= 16 && w->hidden <= 128 && w->hidden % 16 == 0, "hidden must be a multiple of 16 in [16,128]");
   REQ(h->cfg.predictor == CTK_PRED_MLP, "ctk_set_mlp_weights on a handle whose predictor is not CTK_PRED_MLP");
+  // every rejection before the current weights are touched: a rejected call leaves the handle as it was
+  const bool tc_engine = h->cfg.mlp_engine != CTK_MLP_SIMT;
+  if (tc_engine) {
+    REQ(h->cfg.mlp_engine >= CTK_MLP_TCGEN05 && h->cfg.mlp_engine <= CTK_MLP_TCGEN05_FAST, "unknown mlp_engine");
+    REQ(w->hidden == kTcHidden, "the tcgen05 MLP engines are built for hidden == 128 (use mlp_engine=simt otherwise)");
+    REQ(h->cfg.optimizer == CTK_OPT_MPPI || h->cfg.optimizer == CTK_OPT_CEM, "the tcgen05 MLP engines are implemented for MPPI and CEM");
+  }
   CU(cudaSetDevice(h->cfg.device));
   const int hid = w->hidden, nf = mlp_blob_floats(hid);
   std::vector<float> blob((size_t)nf, 0.0f);
@@ -544,10 +551,7 @@ extern "C" int ctk_set_mlp_weights(ctk_handle* h, const ctk_mlp_weights* w) {
   CU(h->d_mlp.alloc((size_t)nf));
   CU(cudaMemcpy(h->d_mlp, blob.data(), sizeof(float) * nf, cudaMemcpyHostToDevice));
   h->mlp = MlpDev{hid, h->d_mlp, nf, nullptr, nullptr};
-  if (h->cfg.mlp_engine != CTK_MLP_SIMT) {
-    REQ(h->cfg.mlp_engine >= CTK_MLP_TCGEN05 && h->cfg.mlp_engine <= CTK_MLP_TCGEN05_FAST, "unknown mlp_engine");
-    REQ(hid == kTcHidden, "the tcgen05 MLP engines are built for hidden == 128 (use mlp_engine=simt otherwise)");
-    REQ(h->cfg.optimizer == CTK_OPT_MPPI || h->cfg.optimizer == CTK_OPT_CEM, "the tcgen05 MLP engines are implemented for MPPI and CEM");
+  if (tc_engine) {
     // W2 as three bf16 terms (w = w1 + w2 + w3, round-to-nearest-even each), B operand tiles: row n = output unit, k = input unit
     std::vector<uint8_t> tc(kTcBlobBytes, 0);
     auto bf16_rn = [](float f) -> uint16_t {

@@ -13,13 +13,18 @@ def has_cuda():
         return False
 
 
-def make_controller(meta, logging=True, rng="replay", shard=None, **optimizer_over):
+def make_controller(meta, logging=True, rng="replay", shard=None, weights=None, optimal_trajectory=False, **optimizer_over):
+    """weights: an MLPSpec / GRUSpec registered under meta["predictor"] (default: the fixture's random_init network)."""
     import control_toolkit_b200 as ctk
     from control_toolkit_b200.Controllers.controller_mpc import controller_mpc
 
-    if meta["predictor"].startswith("Dense"):
+    if isinstance(weights, ctk.MLPSpec):
+        ctk.register_mlp(meta["predictor"], weights)
+    elif isinstance(weights, ctk.GRUSpec):
+        ctk.register_gru(meta["predictor"], weights)
+    elif meta["predictor"].startswith("Dense"):
         ctk.register_mlp(meta["predictor"], ctk.MLPSpec.random_init(meta["mlp_seed"]))
-    if meta["predictor"].startswith("GRU"):
+    elif meta["predictor"].startswith("GRU"):
         ctk.register_gru(meta["predictor"], ctk.GRUSpec.random_init(meta["gru_seed"]))
     cfg = dict(meta["cfg"])
     cfg.update(optimizer_over)
@@ -33,7 +38,7 @@ def make_controller(meta, logging=True, rng="replay", shard=None, **optimizer_ov
         initial_environment_attributes={"target_position": 0.0, "target_equilibrium": 1.0},
         config_controller=dict(optimizer=meta["optimizer"], predictor_specification=meta["predictor"],
                                cost_function_specification=meta["cost"], controller_logging=logging,
-                               calculate_optimal_trajectory=False),
+                               calculate_optimal_trajectory=optimal_trajectory),
         config_optimizers={meta["optimizer"]: cfg},
         config_cost_function={"cost_function_name_default": "default"},
     )

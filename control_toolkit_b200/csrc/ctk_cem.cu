@@ -19,13 +19,16 @@ static cudaError_t launch_cem_p(int kind, bool log, int nblocks, size_t smem, cu
   if (kind == 0) return log ? launch_cem_t<Pred, 0, true>(nblocks, smem, st, a) : launch_cem_t<Pred, 0, false>(nblocks, smem, st, a);
   return log ? launch_cem_t<Pred, 1, true>(nblocks, smem, st, a) : launch_cem_t<Pred, 1, false>(nblocks, smem, st, a);
 }
-cudaError_t launch_cem_rollout(int pred, int kind, bool log, int nblocks, size_t smem, cudaStream_t st, const CemArgs& a) {
-  if (pred == 5) return launch_cem_rollout_gru(kind, log, nblocks, smem, st, a);  // ctk_gru.cu
-  if (pred == 2) return launch_cem_p<MlpTcPred>(kind, log, nblocks, smem, st, a);      // the MLP predictor on the tcgen05 engines
-  if (pred == 6) return launch_cem_p<MlpTcPredV1>(kind, log, nblocks, smem, st, a);
-  if (pred == 3) return launch_cem_p<MlpTcBf16Pred>(kind, log, nblocks, smem, st, a);
-  if (pred == 4) return launch_cem_p<MlpTcFastPred>(kind, log, nblocks, smem, st, a);
-  return pred == 0 ? launch_cem_p<OdePred>(kind, log, nblocks, smem, st, a) : launch_cem_p<MlpSimtPred>(kind, log, nblocks, smem, st, a);
+cudaError_t launch_cem_rollout(PredKind pred, int kind, bool log, int nblocks, size_t smem, cudaStream_t st, const CemArgs& a) {
+  switch (pred) {
+    case PredKind::Ode: return launch_cem_p<OdePred>(kind, log, nblocks, smem, st, a);
+    case PredKind::MlpSimt: return launch_cem_p<MlpSimtPred>(kind, log, nblocks, smem, st, a);
+    case PredKind::MlpTc: return launch_cem_p<MlpTcPred>(kind, log, nblocks, smem, st, a);
+    case PredKind::MlpTcBf16: return launch_cem_p<MlpTcBf16Pred>(kind, log, nblocks, smem, st, a);
+    case PredKind::MlpTcFast: return launch_cem_p<MlpTcFastPred>(kind, log, nblocks, smem, st, a);
+    case PredKind::Gru: return launch_cem_rollout_gru(kind, log, nblocks, smem, st, a);  // ctk_gru.cu
+  }
+  return cudaErrorInvalidValue;
 }
 cudaError_t launch_cem_ode(int kind, bool log, int nblocks, size_t smem, cudaStream_t st, const CemOdeArgs& a) {
   void (*k)(const CemOdeArgs) = nullptr;
@@ -67,10 +70,10 @@ cudaError_t launch_cem_tick(int kind, bool log, int nblocks, size_t smem, cudaSt
   cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, k, a);
 }
-// grid of the generic CEM rollout kernel: one block per 128 rollouts; the single-product tile engines run one CTA per SM with equal shares
-int cem_rollout_grid(int pred, int N, int num_sms) {
+// grid of the generic CEM rollout kernel: one block per 128 rollouts; the tile engines run one CTA per SM with equal shares (kBalanced)
+int cem_rollout_grid(PredKind pred, int N, int num_sms) {
   const int nb = (N + 127) / 128;
-  return ((pred >= 2 && pred <= 4) || pred == 6) ? (nb < num_sms ? nb : num_sms) : nb;  // tile engines: one CTA per SM, equal shares (kBalanced)
+  return pred_info(pred).balanced ? (nb < num_sms ? nb : num_sms) : nb;
 }
 int cem_tick_rollouts_per_block() { return kCemTickRollouts; }
 // resident blocks per SM of the persistent tick kernel (its blocks wait for each other: the whole grid must be resident)

@@ -204,8 +204,8 @@ struct KernelTimer {  // records an event pair around the dominant kernel launch
 
 // ---------------------------------------------------------------------------------------------------------------
 static void mppi_ode_geometry(ctk_handle* h);
-static int pred_id(const ctk_handle* h);
-static bool tile_engine(int pred);
+static PredKind pred_kind(const ctk_handle* h);
+static bool tile_engine(PredKind pred);
 
 // Host-side constants of the rollout kernels (and, MPPI, the ODE kernel's geometry) from cfg / ode_p / cost_p: no device access
 static void derive_consts(ctk_handle* h) {
@@ -368,7 +368,8 @@ static int check_config(const ctk_config* cfg, const ctk_ode_params* ode, const 
 // rollouts (no tail wave).  Needs num_sms; allocates nothing.
 static int mppi_geometry(ctk_handle* h) {
   const int N = h->N;
-  const int maxb = mppi_max_block_threads(pred_id(h));
+  const PredInfo pred = pred_info(pred_kind(h));
+  const int maxb = pred.max_threads;
   const long long slots = (long long)h->num_sms * maxb;
   const int r = (int)((N + slots - 1) / slots);                                  // rollouts per thread
   int T = (int)(((((long long)N + (long long)r * h->num_sms - 1) / ((long long)r * h->num_sms)) + 31) / 32 * 32);
@@ -387,19 +388,16 @@ static int mppi_geometry(ctk_handle* h) {
     h->mppi_stash = 0;
   }
   h->mppi_rpb = h->mppi_block;
-  if (tile_engine(pred_id(h))) {
+  if (tile_engine(pred_kind(h))) {
     // tcgen05 MLP engines (ctk_mlp_tc.cuh): one CTA per SM, every CTA an equal contiguous share of the population (kBalanced); rollouts per
-    // block = tiles in flight x 128: the single-product engines run four tiles (one per warp group), the exact engine two, its round-1
-    // structure (pred 6) one tile with 16 worker warps + 1 MMA-issuer warp
-    const int pid = pred_id(h);
-    h->mppi_block = mppi_max_block_threads(pid); h->mppi_rpb = pid == 6 ? 128 : (pid == 2 ? 256 : 512);
+    // block = tiles in flight x 128 (kRolloutsPerBlock)
+    h->mppi_block = pred.max_threads; h->mppi_rpb = pred.rollouts_per_pass;
     h->mppi_grid = (int)std::min<long long>((long long)h->num_sms, ((long long)N + 127) / 128);
     if (h->mppi_grid < 1) h->mppi_grid = 1;
     h->mppi_iters = (int)((N + (long long)h->mppi_grid * h->mppi_rpb - 1) / ((long long)h->mppi_grid * h->mppi_rpb));
-    h->mppi_stash = (pid == 6 && (size_t)h->n_ind * 128 * sizeof(float) <= 8 * 1024) ? 1 : 0;
+    h->mppi_stash = 0;
     // what the operand tiles leave of the 227 KB for the per-rollout accumulators [n_ind][rollouts per block]
-    const size_t acc_limit = pid == 6 ? 8 * 1024 : (pid == 2 ? 12 * 1024 : 32 * 1024);
-    if ((size_t)h->n_ind * h->mppi_rpb * sizeof(float) > acc_limit) return fail(CTK_EINVAL, "tcgen05 MLP engine: too many inducing points (shared memory is taken by the operand tiles)");
+    if ((size_t)h->n_ind * h->mppi_rpb * sizeof(float) > pred.acc_smem_bytes) return fail(CTK_EINVAL, "tcgen05 MLP engine: too many inducing points (shared memory is taken by the operand tiles)");
   }
   h->partials_stride = (size_t)(h->num_sms > h->mppi_grid ? h->num_sms : h->mppi_grid) * (h->mppi_iters + 1) * (h->n_ind + 2);
   if (h->mppi_grid > CTK_MBOX_BLOCKS || h->num_sms > CTK_MBOX_BLOCKS) return fail(CTK_EINVAL, "device has more SMs than the mailbox has block slots (CTK_MBOX_BLOCKS)");
@@ -810,24 +808,21 @@ static int env_tick(ctk_handle* h, const S0e& s0, float* u_out_dev) {
 // the tick
 // ---------------------------------------------------------------------------------------------------------------
 
-// 0 ODE, 1 MLP on the FP32 pipe, 2 MLP with the dense layer on tcgen05 (bf16 x 3 split, fp32-level), 3 one bf16 product, 4 + MUFU.TANH
-static bool tile_engine(int pred) { return (pred >= 2 && pred <= 4) || pred == 6; }  // the tcgen05 engines of ctk_mlp_tc.cuh
-static int pred_id(const ctk_handle* h) {
-  if (h->cfg.predictor == CTK_PRED_GRU) return 5;  // recurrent predictor on the FP32 pipe (GruSimtPred)
-  if (h->cfg.predictor != CTK_PRED_MLP) return 0;
-  if (h->cfg.optimizer == CTK_OPT_RPGD) return 1;
+// the tcgen05 engines of ctk_mlp_tc.cuh: a pass of a block covers a fixed number of rollouts (tiles in flight x 128)
+static bool tile_engine(PredKind pred) { return pred_info(pred).rollouts_per_pass > 0; }
+static PredKind pred_kind(const ctk_handle* h) {
+  if (h->cfg.predictor == CTK_PRED_GRU) return PredKind::Gru;
+  if (h->cfg.predictor != CTK_PRED_MLP) return PredKind::Ode;
+  if (h->cfg.optimizer == CTK_OPT_RPGD) return PredKind::MlpSimt;
   switch (h->cfg.mlp_engine) {
-    case CTK_MLP_TCGEN05: return getenv("CTK_TC_EXACT_V1") != nullptr ? 6 : 2;  // 6: the round-1 structure of the exact engine (A/B runs)
-    case CTK_MLP_TCGEN05_BF16: return 3;
-    case CTK_MLP_TCGEN05_FAST: return 4;
-    default: return 1;
+    case CTK_MLP_TCGEN05: return PredKind::MlpTc;
+    case CTK_MLP_TCGEN05_BF16: return PredKind::MlpTcBf16;
+    case CTK_MLP_TCGEN05_FAST: return PredKind::MlpTcFast;
+    default: return PredKind::MlpSimt;
   }
 }
-static const char* pred_name(int pred) {  // the predictor functor of a rollout-kernel instantiation (last_kernel)
-  static const char* const names[] = {"OdePred", "MlpSimtPred", "MlpTcPred", "MlpTcBf16Pred", "MlpTcFastPred", "GruSimtPred", "MlpTcPredV1"};
-  return names[pred];
-}
-static size_t pred_smem_floats(ctk_handle* h) { return mppi_pred_smem_floats(pred_id(h), h->mlp); }
+static const char* pred_name(const ctk_handle* h) { return pred_info(pred_kind(h)).name; }  // the rollout kernel's functor (last_kernel)
+static size_t pred_smem_floats(const ctk_handle* h) { return pred_info(pred_kind(h)).smem_floats(h->mlp); }
 
 // Launch geometry of the ODE kernel: one CTA per SM, block sized so that every thread runs the same number of
 // rollout groups (no partially filled last wave); the iteration count with the least padding wins.
@@ -980,10 +975,10 @@ static int mppi_local(ctk_handle* h, const float* s_dev, int mode, float* u_out_
                                        pred_smem_floats(h));
   h->launches++;
   KernelTimer kt(h);
-  if (tile_engine(pred_id(h)) && h->mlp.tc_blob == nullptr) return fail(CTK_ESTATE, "tcgen05 MLP engine without weights");
-  cudaError_t e = launch_mppi_rollout(pred_id(h), h->cost.kind, log, h->mppi_grid, h->mppi_block, smem,
+  if (tile_engine(pred_kind(h)) && h->mlp.tc_blob == nullptr) return fail(CTK_ESTATE, "tcgen05 MLP engine without weights");
+  cudaError_t e = launch_mppi_rollout(pred_kind(h), h->cost.kind, log, h->mppi_grid, h->mppi_block, smem,
                                       h->stream, a);
-  h->last_kernel = std::string("mppi_rollout_kernel<") + pred_name(pred_id(h)) + "," +
+  h->last_kernel = std::string("mppi_rollout_kernel<") + pred_name(h) + "," +
                    std::to_string(h->cost.kind) + "," + (log ? "1" : "0") + ">" + (ns.inj ? " [injected noise]" : " [philox]");
   if (e != cudaSuccess) return fail(CTK_ECUDA, std::string("mppi_rollout_kernel: ") + cudaGetErrorString(e));
   h->step_s = s_dev;
@@ -1141,9 +1136,9 @@ static int cem_local(ctk_handle* h, const float* s_dev, bool to_k) {
     a.log_traj_soa = h->d_log_traj_soa; a.log_Q_soa = h->d_log_Q_soa;
     const size_t smem = sizeof(float) * (2 * (size_t)h->H + pred_smem_floats(h));
     KernelTimer kt(h);
-    if (tile_engine(pred_id(h)) && h->mlp.tc_blob == nullptr) return fail(CTK_ESTATE, "tcgen05 MLP engine without weights");
-    e = launch_cem_rollout(pred_id(h), h->cost.kind, c.logging != 0, cem_rollout_grid(pred_id(h), h->N, h->num_sms), smem, h->stream, a);
-    h->last_kernel = std::string("cem_rollout_kernel<") + pred_name(pred_id(h)) + "," +
+    if (tile_engine(pred_kind(h)) && h->mlp.tc_blob == nullptr) return fail(CTK_ESTATE, "tcgen05 MLP engine without weights");
+    e = launch_cem_rollout(pred_kind(h), h->cost.kind, c.logging != 0, cem_rollout_grid(pred_kind(h), h->N, h->num_sms), smem, h->stream, a);
+    h->last_kernel = std::string("cem_rollout_kernel<") + pred_name(h) + "," +
                      std::to_string(h->cost.kind) + "," + (c.logging ? "1" : "0") + ">" + (ns.inj ? " [injected noise]" : " [philox]");
   }
   if (e != cudaSuccess) return fail(CTK_ECUDA, std::string("cem_rollout_kernel: ") + cudaGetErrorString(e));
@@ -1976,8 +1971,7 @@ extern "C" int ctk_rollout_single(ctk_handle* h, const float* s_host, const floa
   CU(cudaMemcpyAsync(d_s, s_host, 6 * sizeof(float), cudaMemcpyHostToDevice, h->stream));
   CU(cudaMemcpyAsync(d_Q, Q_host, H * sizeof(float), cudaMemcpyHostToDevice, h->stream));
   h->launches++;
-  CU(launch_single_rollout(h->cfg.predictor == CTK_PRED_ODE ? 0 : (h->cfg.predictor == CTK_PRED_GRU ? 5 : 1), d_s, d_Q, H, h->d_kc, h->mlp, h->d_u_prev, d_traj,
-                           d_sum, h->stream));
+  CU(launch_single_rollout(pred_kind(h), d_s, d_Q, H, h->d_kc, h->mlp, h->d_u_prev, d_traj, d_sum, h->stream));
   std::vector<float> tmp((size_t)(H + 1) * 6 + 1);
   CU(cudaMemcpyAsync(tmp.data(), d_traj, tmp.size() * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
   CU(cudaStreamSynchronize(h->stream));

@@ -27,9 +27,27 @@ inline cudaError_t launch_pdl(void (*kern)(P...), dim3 grid, dim3 block, size_t 
   return cudaLaunchKernelEx(&cfg, kern, std::forward<A>(args)...);
 }
 
-// pred: 0 ODE, 1 MLP (SIMT engine); kind: cost class; log: write SoA trajectory logs
-cudaError_t launch_mppi_rollout(int pred, int kind, bool log, int nblocks, int block, size_t smem, cudaStream_t st, const MppiArgs& a);
-int mppi_max_block_threads(int pred);
+// The predictor functor a rollout kernel is instantiated with (ctk_predictor.cuh, ctk_mlp_tc.cuh)
+enum class PredKind {
+  Ode,        // OdePred: CartPole ODE
+  MlpSimt,    // MlpSimtPred: MLP on the FP32 pipe
+  MlpTc,      // MlpTcPred: MLP with layers 1 and 2 on tcgen05, bf16 x 3 split (fp32-level)
+  MlpTcBf16,  // MlpTcBf16Pred: one bf16 product
+  MlpTcFast,  // MlpTcFastPred: one bf16 product + MUFU.TANH
+  Gru         // GruSimtPred: recurrent predictor on the FP32 pipe
+};
+// What the host needs to know about a predictor functor, read from its type (ctk_mppi.cu)
+struct PredInfo {
+  const char* name;           // the functor's name, as in the rollout kernel's instantiation
+  int max_threads;            // kMaxThreads: block size of the MPPI rollout kernel
+  int rollouts_per_pass;      // kRolloutsPerBlock: > 0 for the tile engines (a pass of a block covers that many rollouts), else 0
+  bool balanced;              // kBalanced: one CTA per SM, each an equal contiguous share of the population
+  size_t acc_smem_bytes;      // tile engines: shared memory left for the MPPI accumulators [n_ind][rollouts_per_pass]
+  size_t (*smem_floats)(const MlpDev&);  // dynamic shared memory of the functor
+};
+PredInfo pred_info(PredKind pred);
+// kind: cost class; log: write SoA trajectory logs
+cudaError_t launch_mppi_rollout(PredKind pred, int kind, bool log, int nblocks, int block, size_t smem, cudaStream_t st, const MppiArgs& a);
 // K1 for the ODE predictor with intermediate_steps == 1 (scaled variables, ILP rollouts per thread)
 cudaError_t launch_mppi_ode(int kind, bool log, int period_t, int ilp, int grid, int block, size_t smem, cudaStream_t st, const MppiOdeArgs& a,
                             const char** name = nullptr);
@@ -45,7 +63,6 @@ cudaError_t launch_transpose(const float* in, float* out, int R, int C, cudaStre
 // top-M logging: gather the rows of the rollouts named by m sorted K4 keys out of an SoA [R][N] or reference-layout [N][R] log
 cudaError_t launch_log_gather(const uint64_t* keys, int m, int off, const float* J, size_t N, const float* src, int R, int soa, float* out,
                               float* J_out, int32_t* idx_out, cudaStream_t st);
-size_t mppi_pred_smem_floats(int pred, const MlpDev& m);
 // environments beyond the CartPole (ctk_env.cu): MPPI = rollout + update launches, CEM = rollout, K4 levels, refit
 cudaError_t launch_env_mppi(int env, bool log, const EnvMppiArgs& a, cudaStream_t st);
 cudaError_t launch_env_cem_rollout(int env, bool log, const EnvCemArgs& a, cudaStream_t st);
@@ -58,8 +75,8 @@ cudaError_t launch_single_rollout_gru(const float* s0, const float* Q, int H, co
                                       float* traj, float* summed, cudaStream_t st);
 cudaError_t launch_gru_update(const S0& s0, const float* u_nom, const MlpDev& mlp, float* rnn_h, cudaStream_t st);
 
-cudaError_t launch_cem_rollout(int pred, int kind, bool log, int nblocks, size_t smem, cudaStream_t st, const CemArgs& a);
-int cem_rollout_grid(int pred, int N, int num_sms);
+cudaError_t launch_cem_rollout(PredKind pred, int kind, bool log, int nblocks, size_t smem, cudaStream_t st, const CemArgs& a);
+int cem_rollout_grid(PredKind pred, int N, int num_sms);
 cudaError_t launch_cem_ode(int kind, bool log, int nblocks, size_t smem, cudaStream_t st, const CemOdeArgs& a);
 cudaError_t launch_cem_tick(int kind, bool log, int nblocks, size_t smem, cudaStream_t st, const CemTickArgs& a);
 int cem_tick_rollouts_per_block();
@@ -76,7 +93,8 @@ cudaError_t launch_rpgd_init(const RpgdSelectArgs& a, cudaStream_t st);
 cudaError_t launch_gradcem_sample(const GradCemSampleArgs& a, cudaStream_t st);
 cudaError_t launch_gradcem_refit(const GradCemRefitArgs& a, cudaStream_t st);
 
-cudaError_t launch_single_rollout(int pred, const float* s0, const float* Q, int H, const DevConsts* kc, const MlpDev& mlp, const float* u_prev, float* traj, float* summed, cudaStream_t st);
+// ODE -> OdePred, GRU -> the GRU kernel, every MLP engine -> MlpSimtPred (one rollout: no tile to fill)
+cudaError_t launch_single_rollout(PredKind pred, const float* s0, const float* Q, int H, const DevConsts* kc, const MlpDev& mlp, const float* u_prev, float* traj, float* summed, cudaStream_t st);
 cudaError_t launch_fma_peak(float* out, int blocks, int threads, int iters, cudaStream_t st);
 cudaError_t launch_fp32_micro(int variant, float* out, int blocks, int threads, int iters, const float* seed, cudaStream_t st);
 cudaError_t launch_philox_fill(const NoiseSrc& ns, float* out, size_t n, cudaStream_t st);

@@ -1,25 +1,15 @@
-// ctk_mlp_tc.cuh -- tcgen05 (UMMA + TMEM) engine of the MLP predictor (6 -> 128 tanh -> 128 tanh -> 5, config C4).
+// ctk_mlp_tc.cuh -- tcgen05 (UMMA + TMEM) engines of the MLP predictor (6 -> 128 tanh -> 128 tanh -> 5, config C4).
 // Replaces PredictorWrapper.predict_core for the neural predictor (reference call sites optimizer_mppi.py:188,
-// optimizer_cem_tf.py:57).  Drop-in `Pred` of the generic rollout kernels (ctk_kernels_mppi.cuh): one CTA = 128
-// rollouts = the M dimension of the MMA, 16 worker warps: thread (row r, quarter q) works on a quarter of row r's columns in the
-// FP32 stages (4 warps per scheduler hide the MUFU / shared-memory latency), threads with q = 0 own the rollouts; a 17th warp
-// only issues the MMAs, one K-quarter at a time, as soon as the workers have produced it (named barriers 1..4), so the
-// tensor core runs underneath the FP32 layer-1 stage.
-//
-//   layer 1 (6 -> 128, 4 % of the FLOPs)  : FP32 FMAs per thread, weights broadcast from shared memory; tanh; the row of h1
-//                                            is split into THREE bf16 terms (h = a1 + a2 + a3, 24 mantissa bits) and stored
-//                                            as three K-major operand tiles in the canonical no-swizzle core-matrix layout;
-//   layer 2 (128 -> 128, 92 % of the FLOPs): D[128x128] (fp32, TMEM) = sum of the six significant products of the bf16
-//                                            splits of h1 and W2 (a3 w1, a2 w2, a1 w3, a2 w1, a1 w2, a1 w1; smallest first):
-//                                            48 tcgen05.mma.kind::f16 (M128 N128 K16) issued by one thread, completion by
-//                                            tcgen05.commit -> mbarrier;  error vs an exact product ~2e-7 (tools/lab/umma_lab.cu);
-//   layer 3 (128 -> 5)                     : each thread reads its accumulator row back with tcgen05.ld (32 columns at a
-//                                            time), applies bias + tanh and folds the 5 outputs with FP32 FMAs.
-// bf16 x 3 instead of TF32 x 3: same tensor time (6 products at twice the rate), but the operand tiles are half the size,
-// which is what lets A (96 KB) and W2 (96 KB) both live in shared memory.
+// optimizer_cem_tf.py:57).  Drop-in `Pred`s of the generic rollout kernels (ctk_kernels_mppi.cuh).  Both structures run ONE CTA per
+// SM with several 128-rollout tiles in flight (a tile = the M dimension of an MMA), give every CTA an equal contiguous share of the
+// population, and run layer 1 on the tensor core (one K = 48 operand row of split inputs per rollout against the resident B1):
+//   MlpTcFastPredT (tcgen05_bf16, tcgen05_fast): four tiles, one per warp group, one thread per rollout; layer 2 as ONE bf16
+//                                                 product (8 UMMAs per tile-step);
+//   MlpTcPred      (tcgen05, fp32-level):        two tiles, an owner and a helper thread per rollout; layer 2 as the six significant
+//                                                 products of three-term bf16 splits of h1 and W2, issued by K-quarters (48 UMMAs).
+// Layer 3 (128 -> 5) runs on the FP32 pipe from the accumulator rows (tcgen05.ld).  Measurements and the earlier structures: DESIGN §5.2.
 #pragma once
 #include <cuda_bf16.h>
-#include <cstdio>
 
 #include "ctk_args.cuh"
 #include "ctk_device.cuh"
@@ -35,10 +25,12 @@ constexpr uint32_t kTcMnStride = 128;             // bytes between 8-row groups 
 __host__ __device__ inline uint32_t tc_tile_offset(int row, int k) { return (uint32_t)(k >> 3) * kTcKStride + (uint32_t)row * 16u + (uint32_t)(k & 7) * 2u; }
 // device blob: W2 split tiles [3][32768 B] | W1 [6][128] | b1 [128] | b2 [128] | W3T [5][128] | b3 [8]   (floats after the tiles)
 constexpr uint32_t kTcBlobFloats = 6 * 128 + 128 + 128 + 5 * 128 + 8;
-// ... | B1 [6 k-groups][128 n][8] bf16 (single-product engines: layer 1 on the tensor core, see MlpTcFastPredT): rows of
-// K = 48: W1 term 1 three times (x1, x2, x3), W1 term 2 twice (x1, x2), W1 term 3 (x1), the three terms of b1 (against 1.0), zeros
+// ... | B1 [6 k-groups][128 n][8] bf16 (layer 1 on the tensor core): rows of K = 48: W1 term 1 three times (x1, x2, x3), W1 term 2
+// twice (x1, x2), W1 term 3 (x1), the three terms of b1 (against 1.0), zeros
 constexpr uint32_t kTcB1Bytes = 6 * kTcKStride;
 constexpr uint32_t kTcBlobBytes = 3 * kTcTileBytes + kTcBlobFloats * 4 + kTcB1Bytes;
+// instruction descriptor of every MMA here: D fp32, A/B bf16, both K-major, N = 128, M = 128
+constexpr uint32_t kTcIdescM128N128 = (1u << 4) | (1u << 7) | (1u << 10) | ((128u >> 3) << 17) | ((128u >> 4) << 24);
 
 #ifdef __CUDACC__
 __device__ __forceinline__ uint64_t umma_smem_desc(uint32_t saddr) {
@@ -51,271 +43,108 @@ __device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t adesc, uint6
       "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}\n" ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
-
-struct MlpTcPredV1 {
-  static constexpr bool kCooperative = true;  // every thread of the CTA must call step() the same number of times
-  static constexpr bool kBalanced = true;     // CTA b rolls out the contiguous share [b N / grid, (b + 1) N / grid): with one CTA per SM every
-                                              // SM gets 442.8 of C4's 65536 rollouts (3 tiles + a 59-row tile whose idle warps skip the
-                                              // arithmetic) instead of 3 or 4 whole tiles (512 tiles on 148 SMs = 3.46 waves)
-  static constexpr int kMaxThreads = 544;  // 16 worker warps + 1 MMA-issuer warp
-  static constexpr int kCemThreads = 544;
-  static constexpr int kMinBlocks = 1;
-  static constexpr int kRolloutsPerBlock = 128;  // threads 128..543 are helpers: they own no rollout
-  uint8_t* sA;        // [3][32768] activation split tiles (written per step); reused for the layer-3 partial sums
-  float* sx;          // [128][8] network inputs of the rows (owners -> helpers)
-  uint8_t* sB;        // [3][32768] W2 split tiles (resident)
-  const float *W1, *b1, *b2, *W3T, *b3;
-  uint64_t* mbar;
-  uint32_t* tmem_slot;
-  uint32_t phase;
-  int rows_on;        // real rollouts of the tile in flight (rows >= rows_on are padding: their warps skip the FP32 / MUFU stages)
-#ifdef CTK_TC_TRACE
-  long long tr[8];  // accumulated clock64 deltas of the step phases (diagnostics build)
-  long long tl;
-#endif
-
-  static size_t smem_floats(const MlpDev&) { return (6 * (size_t)kTcTileBytes + kTcBlobFloats * 4 + 64 + 128 * 8 * 4 + 1024) / 4; }
-
-  __device__ __forceinline__ MlpTcPredV1(const DevConsts*, const MlpDev& m, float* sm) {
-    uint8_t* base = reinterpret_cast<uint8_t*>(((uintptr_t)sm + 1023) & ~(uintptr_t)1023);
-    sA = base;
-    sB = base + 3 * kTcTileBytes;
-    float* f = reinterpret_cast<float*>(sB + 3 * kTcTileBytes);
-    W1 = f; b1 = W1 + 6 * 128; b2 = b1 + 128; W3T = b2 + 128; b3 = W3T + 5 * 128;
-    mbar = reinterpret_cast<uint64_t*>(f + kTcBlobFloats);  // [2]: one per half of the accumulator columns
-    tmem_slot = reinterpret_cast<uint32_t*>(mbar + 2);
-    sx = f + kTcBlobFloats + 16;
-    phase = 0;
-    rows_on = 128;
-#ifdef CTK_TC_TRACE
-    for (int i = 0; i < 8; ++i) tr[i] = 0;
-    tl = 0;
-#endif
-    const uint4* src = reinterpret_cast<const uint4*>(m.tc_blob);
-    uint4* dst = reinterpret_cast<uint4*>(sB);
-    for (int i = threadIdx.x; i < (int)((3 * kTcTileBytes + kTcBlobFloats * 4) / 16); i += blockDim.x) dst[i] = src[i];  // (not the B1 tile behind them)
-    if (threadIdx.x == 0) {
-      asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(mbar)) : "memory");
-      asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(mbar + 1)) : "memory");
-      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if ((threadIdx.x >> 5) == 0) {  // one warp allocates 128 TMEM columns (the fp32 accumulator) for the CTA's lifetime
-      asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 128;" ::"r"(smem_u32(tmem_slot)) : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // W2 tiles were written through the generic proxy
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    // caller issues __syncthreads() after construction
+// the MMAs this thread has issued so far -> one arrival on the mbarrier at shared address `bar` when they complete
+__device__ __forceinline__ void umma_commit(uint32_t bar) {
+  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
+}
+// one lane spins until the mbarrier at shared address `bar` has completed the phase of the given parity
+__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
+  uint32_t done = 0;
+  while (!done) {
+    asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.b32 %0, 1, 0, p;\n\t}\n"
+                 : "=r"(done) : "r"(bar), "r"(parity) : "memory");
   }
-  __device__ __forceinline__ ~MlpTcPredV1() {
-#ifdef CTK_TC_TRACE
-    if (blockIdx.x == 0 && (threadIdx.x == 0 || threadIdx.x == 200))
-      printf("tc trace tid %d: B1 %lld  L1 %lld  B2 %lld  issue %lld  mma-wait %lld  epilogue %lld  B3+update %lld  outside %lld (cycles, summed)\n", (int)threadIdx.x, tr[0], tr[1], tr[2], tr[3], tr[4], tr[5], tr[6], tr[7]);
-#endif
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    if ((threadIdx.x >> 5) == 0) {
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-      asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 128;" ::"r"(*tmem_slot) : "memory");
-    }
+}
+// 16 consecutive fp32 columns of this thread's TMEM lane (accumulator row), starting at `taddr`; waits for the load
+__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&v)[16]) {
+  asm volatile(
+      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
+      : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
+        "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
+      : "r"(taddr));
+  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+}
+// the CTA's TMEM for its lifetime: warp 0 allocates NCOLS columns (base address -> *slot) and gives up the allocation permit
+template <int NCOLS>
+__device__ __forceinline__ void tmem_alloc_cta(uint32_t* slot) {
+  if ((threadIdx.x >> 5) == 0) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(slot)), "n"(NCOLS) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
   }
-  __device__ __forceinline__ void substep(State& z, float u, float& omc) { step(z, u, omc); }
-  __device__ __forceinline__ bool single_substep() const { return false; }
-  __device__ __forceinline__ void use_uniform(const HotUK&) {}
-  __device__ __forceinline__ void begin_rollout(bool = true) {}
-  // called by every thread at the top of a pass of the rollout loop: the whole CTA works on the tile [base, base + 128)
-  __device__ __forceinline__ bool group_active(int base, int end) { rows_on = end - base; return true; }
-
-  // tanh(x) = 1 - 2 / (exp(2x) + 1) for either sign (x -> -inf: e -> 0, t -> -1; x -> +inf: e -> inf, r -> 0, t -> 1):
-  // FMUL, MUFU.EX2, FADD, MUFU.RCP, FFMA.  Absolute error <= ~3e-7 (the two MUFU approximations), the same bound the
-  // FP32-pipe engine's tanh_acc has outside its small-|x| series branch.
-  static __device__ __forceinline__ float tanh5(float x) {
-    float e, r;
-    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e) : "f"(x * 2.8853900817779268f));  // exp(2x) = 2^(2x log2 e)
-    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(e + 1.0f));
-    return fmaf(-2.0f, r, 1.0f);
-  }
-  static __device__ __forceinline__ float4 lds4(uint32_t addr) {
-    float4 v;
-    asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(addr));
-    return v;
-  }
-  // three bf16 terms of two floats by TRUNCATION (x = t1 + t2 + t3 + O(2^-24 x), every residual exact): the high halves are
-  // picked by PRMT, the residuals by LOP3 + FADD -- ALU / FMA pipes only, the conversion unit stays free for the MUFU tanh
-  static __device__ __forceinline__ void split3(float a0, float a1, uint32_t& p1, uint32_t& p2, uint32_t& p3) {
-    const uint32_t u0 = __float_as_uint(a0), u1 = __float_as_uint(a1);
-    p1 = __byte_perm(u0, u1, 0x7632);
-    const float r0 = a0 - __uint_as_float(u0 & 0xffff0000u), r1 = a1 - __uint_as_float(u1 & 0xffff0000u);
-    const uint32_t v0 = __float_as_uint(r0), v1 = __float_as_uint(r1);
-    p2 = __byte_perm(v0, v1, 0x7632);
-    const float s0 = r0 - __uint_as_float(v0 & 0xffff0000u), s1 = r1 - __uint_as_float(v1 & 0xffff0000u);
-    p3 = __byte_perm(__float_as_uint(s0), __float_as_uint(s1), 0x7632);
-  }
-
-  // net input [Q, angleD, cos, sin, position, positionD] -> next [angleD, cos, sin, position, positionD];
-  // angle = atan2(sin, cos)  (oracle/spec.py MLPPredictor.step).  Called by all 512 threads; only q = 0 threads carry state.
-  __device__ __forceinline__ void step(State& z, float u, float& omc) {
-    const int tid = threadIdx.x, row = tid & 127, q = tid >> 7;
-#ifdef CTK_TC_TRACE
-    long long tc0 = clock64();
-    if (tl) tr[7] += tc0 - tl;
-#define TCT(i) { long long tc1 = clock64(); tr[i] += tc1 - tc0; tc0 = tc1; }
-#else
-#define TCT(i)
-#endif
-    const uint32_t aW1 = smem_u32(W1), ab1 = smem_u32(b1), ab2 = smem_u32(b2), aW3 = smem_u32(W3T);
-    if (tid >= 512) {
-      // ===== MMA issuer warp: layer 2 on the tensor core, pipelined against the workers' layer-1 stage by quarters of K =====
-      __syncthreads();  // (S1)
-      const uint32_t tmem_i = *tmem_slot;
-      // instruction descriptor: D fp32, A/B bf16, both K-major, N = 128, M = 128
-      constexpr uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((128u >> 3) << 17) | ((128u >> 4) << 24);
-      const uint32_t a0 = smem_u32(sA), b0 = smem_u32(sB);
-      uint32_t acc = 0;
-#pragma unroll 1
-      for (int p = 0; p < 4; ++p) {
-        asm volatile("bar.sync %0, 544;" ::"r"(1 + p) : "memory");  // quarter p of the operand tiles is complete (workers arrive)
-        if (tid == 512) {
-          asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-#pragma unroll
-          for (int term = 0; term < 6; ++term) {  // per quarter, smallest products first: (a3 w1) (a2 w2) (a1 w3) (a2 w1) (a1 w2) (a1 w1)
-            constexpr int ta[6] = {2, 1, 0, 1, 0, 0}, tb[6] = {0, 1, 2, 0, 1, 0};
-            const uint32_t ab = a0 + ta[term] * kTcTileBytes, bb = b0 + tb[term] * kTcTileBytes;
-#pragma unroll
-            for (int kq = 0; kq < 2; ++kq) {
-              const uint32_t ks = (uint32_t)(2 * p + kq);
-              umma_bf16(tmem_i, umma_smem_desc(ab + ks * 2 * kTcKStride), umma_smem_desc(bb + ks * 2 * kTcKStride), idesc, acc);
-              acc = 1;
-            }
-          }
-          if (p == 3)
-            asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(mbar)) : "memory");
-        }
-        __syncwarp();
-      }
-      {  // this warp alone waits for the MMAs; the workers sleep in the hardware barrier (S2) instead of polling shared memory
-        uint32_t done = 0;
-        const uint32_t bar = smem_u32(mbar);
-        while (!done) {
-          asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.b32 %0, 1, 0, p;\n\t}\n"
-                       : "=r"(done) : "r"(bar), "r"(phase) : "memory");
-        }
-        phase ^= 1u;
-      }
-      asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-      __syncthreads();  // (S2) accumulator complete
-      __syncthreads();  // (S3) partial sums exchanged
-      return;
-    }
-    if (q == 0) {
-      float4* d = reinterpret_cast<float4*>(sx + row * 8);
-      d[0] = make_float4(u, z.om, z.c, z.s);
-      d[1] = make_float4(z.x, z.v, 0.f, 0.f);
-    }
-    __syncthreads();  // (S1) inputs visible; also: every thread is done with the previous step's partial sums (they alias sA)
-    TCT(0)
-    float x[6];
-    {
-      const float4 v0 = lds4(smem_u32(sx + row * 8)), v1 = lds4(smem_u32(sx + row * 8 + 4));
-      x[0] = v0.x; x[1] = v0.y; x[2] = v0.z; x[3] = v0.w; x[4] = v1.x; x[5] = v1.y;
-    }
-    // ---- layer 1 + tanh + 3-term bf16 split -> operand tiles.  In phase p this thread produces k-group 4 p + q of its row, so
-    //      that after phase p the K-quarter [32 p, 32 p + 32) is complete for all rows and its MMAs can start ----
-    const uint32_t arow = smem_u32(sA) + (uint32_t)row * 16u;
-    const bool warp_on = (row & ~31) < rows_on;  // warp-uniform: this warp's 32 rows hold at least one real rollout
-#pragma unroll
-    for (int p = 0; p < 4; ++p) {
-      const int kg = 4 * p + q;
-      if (!warp_on) {  // padding rows: keep the barrier protocol, skip the arithmetic (their accumulator rows are never read)
-        asm volatile("bar.arrive %0, 544;" ::"r"(1 + p) : "memory");
-        continue;
-      }
-      uint32_t p1[4], p2[4], p3[4];
-#pragma unroll
-      for (int half = 0; half < 2; ++half) {
-        const uint32_t jo = (uint32_t)(kg * 8 + half * 4) * 4u;
-        float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);  // torch: (x @ W1) + b1 -> accumulate the dot product first, then add the bias
-#pragma unroll
-        for (int i = 0; i < 6; ++i) {
-          const float4 w = lds4(aW1 + (uint32_t)i * 512u + jo);
-          acc.x = fmaf(x[i], w.x, acc.x); acc.y = fmaf(x[i], w.y, acc.y); acc.z = fmaf(x[i], w.z, acc.z); acc.w = fmaf(x[i], w.w, acc.w);
-        }
-        const float4 bb = lds4(ab1 + jo);
-        split3(tanh5(acc.x + bb.x), tanh5(acc.y + bb.y), p1[2 * half], p2[2 * half], p3[2 * half]);
-        split3(tanh5(acc.z + bb.z), tanh5(acc.w + bb.w), p1[2 * half + 1], p2[2 * half + 1], p3[2 * half + 1]);
-      }
-      const uint32_t dst = arow + (uint32_t)kg * kTcKStride;
-      asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(dst), "r"(p1[0]), "r"(p1[1]), "r"(p1[2]), "r"(p1[3]) : "memory");
-      asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(dst + kTcTileBytes), "r"(p2[0]), "r"(p2[1]), "r"(p2[2]), "r"(p2[3]) : "memory");
-      asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(dst + 2 * kTcTileBytes), "r"(p3[0]), "r"(p3[1]), "r"(p3[2]), "r"(p3[3]) : "memory");
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // operand tiles -> visible to the tensor core (async proxy)
-      asm volatile("bar.arrive %0, 544;" ::"r"(1 + p) : "memory");  // non-blocking: tell the issuer warp that quarter p is written
-    }
-    TCT(1)
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();  // (S2) released when the issuer warp has seen the MMAs complete
-    TCT(2)
-    const uint32_t tmem = *tmem_slot;
-    TCT(3)
-    // ---- accumulator -> bias + tanh -> layer 3 partial sums: columns [32 q, 32 q + 32) ----
-    float y[5] = {0.f, 0.f, 0.f, 0.f, 0.f};
-    const uint32_t trow = tmem + ((uint32_t)(((tid >> 5) & 3) * 32) << 16);
+}
+// called by every thread of the CTA: after the CTA's last tcgen05 operation, warp 0 frees the columns of tmem_alloc_cta
+template <int NCOLS>
+__device__ __forceinline__ void tmem_dealloc_cta(const uint32_t* slot) {
+  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  __syncthreads();
+  if ((threadIdx.x >> 5) == 0) {
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    TCT(4)
-#pragma unroll 1
-    for (int hh = 0; hh < (warp_on ? 2 : 0); ++hh) {
-      const int c0 = q * 32 + hh * 16;
-      uint32_t v[16];
-      asm volatile(
-          "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-          : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
-            "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-          : "r"(trow + c0));
-      asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-      for (int g = 0; g < 4; ++g) {
-        const uint32_t jo = (uint32_t)(c0 + g * 4) * 4u;
-        const float4 bb = lds4(ab2 + jo);
-        const float h0 = tanh5(__uint_as_float(v[4 * g]) + bb.x), h1 = tanh5(__uint_as_float(v[4 * g + 1]) + bb.y);
-        const float h2 = tanh5(__uint_as_float(v[4 * g + 2]) + bb.z), h3 = tanh5(__uint_as_float(v[4 * g + 3]) + bb.w);
-#pragma unroll
-        for (int k = 0; k < 5; ++k) {
-          const float4 w = lds4(aW3 + (uint32_t)k * 512u + jo);
-          y[k] = fmaf(h3, w.w, fmaf(h2, w.z, fmaf(h1, w.y, fmaf(h0, w.x, y[k]))));
-        }
-      }
-    }
-    TCT(5)
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    // all MMAs of this step have completed (both barriers observed): the operand tiles are free and carry the partial sums
-    float* sy = reinterpret_cast<float*>(sA);  // [3][128][8]
-    if (q > 0) {
-      float4* d = reinterpret_cast<float4*>(sy + ((q - 1) * 128 + row) * 8);
-      d[0] = make_float4(y[0], y[1], y[2], y[3]);
-      d[1] = make_float4(y[4], 0.f, 0.f, 0.f);
-    }
-    __syncthreads();  // (S3)
-    if (q == 0) {
-#pragma unroll
-      for (int p = 0; p < 3; ++p) {
-        const float4 v0 = lds4(smem_u32(sy + (p * 128 + row) * 8)), v1 = lds4(smem_u32(sy + (p * 128 + row) * 8 + 4));
-        y[0] += v0.x; y[1] += v0.y; y[2] += v0.z; y[3] += v0.w; y[4] += v1.x;
-      }
-      z.om = y[0] + b3[0];
-      z.c = y[1] + b3[1];
-      z.s = y[2] + b3[2];
-      z.x = y[3] + b3[3];
-      z.v = y[4] + b3[4];
-      z.th = atan2f(z.s, z.c);
-      // the network's (cos, sin) outputs are not normalised: cos(atan2(s, c)) = c / hypot(s, c)
-      omc = 1.0f - z.c * rsqrtf(fmaf(z.c, z.c, z.s * z.s));
-    }
-    TCT(6)
-#ifdef CTK_TC_TRACE
-    tl = clock64();
-#endif
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(*slot), "n"(NCOLS) : "memory");
   }
-};
+}
+
+// tanh(x) = 1 - 2 / (exp(2x) + 1) for either sign (x -> -inf: e -> 0, t -> -1; x -> +inf: e -> inf, r -> 0, t -> 1):
+// FMUL, MUFU.EX2, FADD, MUFU.RCP, FFMA.  Absolute error <= ~3e-7 (the two MUFU approximations), the same bound the
+// FP32-pipe engine's tanh_acc has outside its small-|x| series branch.
+__device__ __forceinline__ float tanh5(float x) {
+  float e, r;
+  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e) : "f"(x * 2.8853900817779268f));  // exp(2x) = 2^(2x log2 e)
+  asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(e + 1.0f));
+  return fmaf(-2.0f, r, 1.0f);
+}
+__device__ __forceinline__ float4 lds4(uint32_t addr) {
+  float4 v;
+  asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(addr));
+  return v;
+}
+__device__ __forceinline__ void sts4(uint32_t addr, uint32_t w0, uint32_t w1, uint32_t w2, uint32_t w3) {
+  asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(w0), "r"(w1), "r"(w2), "r"(w3) : "memory");
+}
+// three bf16 terms of two floats by TRUNCATION (x = t1 + t2 + t3 + O(2^-24 x), every residual exact): the high halves are
+// picked by PRMT, the residuals by LOP3 + FADD -- ALU / FMA pipes only, the conversion unit stays free for the MUFU tanh
+__device__ __forceinline__ void split3(float a0, float a1, uint32_t& p1, uint32_t& p2, uint32_t& p3) {
+  const uint32_t u0 = __float_as_uint(a0), u1 = __float_as_uint(a1);
+  p1 = __byte_perm(u0, u1, 0x7632);
+  const float r0 = a0 - __uint_as_float(u0 & 0xffff0000u), r1 = a1 - __uint_as_float(u1 & 0xffff0000u);
+  const uint32_t v0 = __float_as_uint(r0), v1 = __float_as_uint(r1);
+  p2 = __byte_perm(v0, v1, 0x7632);
+  const float s0 = r0 - __uint_as_float(v0 & 0xffff0000u), s1 = r1 - __uint_as_float(v1 & 0xffff0000u);
+  p3 = __byte_perm(__float_as_uint(s0), __float_as_uint(s1), 0x7632);
+}
+// layer-1 operand row of one rollout at shared address `arow`: [x1 x2 x3 x1 x2 x1 | 1 1 1 | 0 ...], the three-term bf16 split of the
+// six inputs [Q, angleD, cos, sin, position, positionD]; K = 48 = six 16-byte k-groups of the K-major core-matrix layout
+__device__ __forceinline__ void store_l1_operand_row(uint32_t arow, float u, const State& z) {
+  uint32_t p1[3], p2[3], p3[3];
+  split3(u, z.om, p1[0], p2[0], p3[0]);
+  split3(z.c, z.s, p1[1], p2[1], p3[1]);
+  split3(z.x, z.v, p1[2], p2[2], p3[2]);
+  sts4(arow + 0u * kTcKStride, p1[0], p1[1], p1[2], p2[0]);          // k  0.. 7: x1[0..5] x2[0..1]
+  sts4(arow + 1u * kTcKStride, p2[1], p2[2], p3[0], p3[1]);          // k  8..15: x2[2..5] x3[0..3]
+  sts4(arow + 2u * kTcKStride, p3[2], p1[0], p1[1], p1[2]);          // k 16..23: x3[4..5] x1[0..5]
+  sts4(arow + 3u * kTcKStride, p2[0], p2[1], p2[2], p1[0]);          // k 24..31: x2[0..5] x1[0..1]
+  sts4(arow + 4u * kTcKStride, p1[1], p1[2], 0x3f803f80u, 0x00003f80u);  // k 32..39: x1[2..5] 1 1 1 0
+  sts4(arow + 5u * kTcKStride, 0u, 0u, 0u, 0u);                      // k 40..47
+}
+// layer 3 over one 16-column chunk of this thread's layer-2 accumulator row (TMEM address `taddr`, hidden units [c0, c0 + 16)):
+// bias b2, activation ACT, five FMAs per column into the partial outputs y
+template <float (*ACT)(float)>
+__device__ __forceinline__ void fold_l3_chunk(uint32_t taddr, int c0, uint32_t ab2, uint32_t aW3, float (&y)[5]) {
+  uint32_t v[16];
+  tmem_ld16(taddr, v);
+#pragma unroll
+  for (int q4 = 0; q4 < 4; ++q4) {
+    const uint32_t jo = (uint32_t)(c0 + q4 * 4) * 4u;
+    const float4 bb = lds4(ab2 + jo);
+    const float h0 = ACT(__uint_as_float(v[4 * q4]) + bb.x), h1 = ACT(__uint_as_float(v[4 * q4 + 1]) + bb.y);
+    const float h2 = ACT(__uint_as_float(v[4 * q4 + 2]) + bb.z), h3 = ACT(__uint_as_float(v[4 * q4 + 3]) + bb.w);
+#pragma unroll
+    for (int k = 0; k < 5; ++k) {
+      const float4 w = lds4(aW3 + (uint32_t)k * 512u + jo);
+      y[k] = fmaf(h3, w.w, fmaf(h2, w.z, fmaf(h1, w.y, fmaf(h0, w.x, y[k]))));
+    }
+  }
+}
+
 // ---------------------------------------------------------------------------------------------------------------
 // Opt-in reduced-precision engines of the same predictor (SURVEY section 7 hard part 4: "ship exact and fast variants, report both"):
 // layer 2 as ONE bf16 product (h1 and W2 rounded to bfloat16, round to nearest even; fp32 accumulation in TMEM) -- 8 UMMAs per
@@ -346,6 +175,7 @@ struct MlpTcFastPredT {
   static constexpr int kCemThreads = 512;
   static constexpr int kMinBlocks = 1;
   static constexpr int kRolloutsPerBlock = 512;
+  static constexpr size_t kAccSmemBytes = 32 * 1024;  // what the tiles leave of the 227 KB for the MPPI accumulators [n_ind][512]
   uint8_t* sA;        // this group's bf16 tile of h1 [32768]
   uint8_t* sB;        // [32768] W2 rounded to bf16 (resident, shared by the groups)
   const float *W1, *b1, *b2, *W3T, *b3;
@@ -385,22 +215,12 @@ struct MlpTcFastPredT {
     for (int i = threadIdx.x; i < (int)(kTcBlobFloats * 4 / 16); i += blockDim.x) dstf[i] = srcf[i];
     if (threadIdx.x < 4) asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(mb0 + threadIdx.x)) : "memory");
     if (threadIdx.x == 0) asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    if ((threadIdx.x >> 5) == 0) {  // the CTA owns the SM: all 512 TMEM columns, 128 per group
-      asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(smem_u32(tmem_slot)) : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    tmem_alloc_cta<512>(tmem_slot);  // the CTA owns the SM: all 512 TMEM columns, 128 per group
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     // caller issues __syncthreads() after construction
   }
-  __device__ __forceinline__ ~MlpTcFastPredT() {
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    if ((threadIdx.x >> 5) == 0) {
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-      asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(*tmem_slot) : "memory");
-    }
-  }
+  __device__ __forceinline__ ~MlpTcFastPredT() { tmem_dealloc_cta<512>(tmem_slot); }
   __device__ __forceinline__ void substep(State& z, float u, float& omc) { step(z, u, omc); }
   __device__ __forceinline__ bool single_substep() const { return false; }
   __device__ __forceinline__ void use_uniform(const HotUK&) {}
@@ -414,7 +234,7 @@ struct MlpTcFastPredT {
       asm("tanh.approx.f32 %0, %1;" : "=f"(t) : "f"(x));
       return t;
     }
-    return MlpTcPredV1::tanh5(x);
+    return tanh5(x);
   }
   static __device__ __forceinline__ uint32_t pack2(float lo, float hi) {  // two floats -> bf16x2 (RN-even), first element in the low half
     uint32_t d;
@@ -429,7 +249,6 @@ struct MlpTcFastPredT {
     const uint32_t arow = smem_u32(sA) + (uint32_t)row * 16u;
     const uint32_t tmem_g = *tmem_slot + (uint32_t)g * 128u;
     const uint32_t trow = tmem_g + ((uint32_t)(wq * 32) << 16);
-    constexpr uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((128u >> 3) << 17) | ((128u >> 4) << 24);
     // the group's first thread issues nk K16 UMMAs (A from the group's tile, B from b_base) and commits them to the group's mbarrier;
     // one lane of the group's first warp waits for them, the other three warps sleep in the hardware barrier that follows
     auto mma_round = [&](uint32_t b_base, int nk) {
@@ -440,18 +259,11 @@ struct MlpTcFastPredT {
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
         const uint32_t a0 = smem_u32(sA);
         for (int ks = 0; ks < nk; ++ks)
-          umma_bf16(tmem_g, umma_smem_desc(a0 + (uint32_t)ks * 2u * kTcKStride), umma_smem_desc(b_base + (uint32_t)ks * 2u * kTcKStride), idesc, ks > 0 ? 1u : 0u);
-        asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(mbar)) : "memory");
+          umma_bf16(tmem_g, umma_smem_desc(a0 + (uint32_t)ks * 2u * kTcKStride), umma_smem_desc(b_base + (uint32_t)ks * 2u * kTcKStride), kTcIdescM128N128, ks > 0 ? 1u : 0u);
+        umma_commit(smem_u32(mbar));
       }
       if (wq == 0) {
-        if ((tid & 31) == 0) {
-          uint32_t done = 0;
-          const uint32_t bar = smem_u32(mbar);
-          while (!done) {
-            asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.b32 %0, 1, 0, p;\n\t}\n"
-                         : "=r"(done) : "r"(bar), "r"(phase) : "memory");
-          }
-        }
+        if ((tid & 31) == 0) mbar_wait(smem_u32(mbar), phase);
         __syncwarp();
       }
       phase ^= 1u;
@@ -459,40 +271,20 @@ struct MlpTcFastPredT {
       asm volatile("bar.sync %0, 128;" ::"r"(5 + g) : "memory");        // the group's accumulator is complete
       asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     };
-    // ---- layer 1 on the tensor core: this thread's operand row [x1 x2 x3 x1 x2 x1 | 1 1 1 | 0 ...] (three-term bf16 split of the
-    //      six inputs, K = 48 = six 16-byte k-groups of the K-major core-matrix layout) ----
-    if (warp_on) {
-      uint32_t p1[3], p2[3], p3[3];
-      MlpTcPredV1::split3(u, z.om, p1[0], p2[0], p3[0]);
-      MlpTcPredV1::split3(z.c, z.s, p1[1], p2[1], p3[1]);
-      MlpTcPredV1::split3(z.x, z.v, p1[2], p2[2], p3[2]);
-      auto sts4 = [&](int kg, uint32_t w0, uint32_t w1, uint32_t w2, uint32_t w3) {
-        asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(arow + (uint32_t)kg * kTcKStride), "r"(w0), "r"(w1), "r"(w2), "r"(w3) : "memory");
-      };
-      sts4(0, p1[0], p1[1], p1[2], p2[0]);          // k  0.. 7: x1[0..5] x2[0..1]
-      sts4(1, p2[1], p2[2], p3[0], p3[1]);          // k  8..15: x2[2..5] x3[0..3]
-      sts4(2, p3[2], p1[0], p1[1], p1[2]);          // k 16..23: x3[4..5] x1[0..5]
-      sts4(3, p2[0], p2[1], p2[2], p1[0]);          // k 24..31: x2[0..5] x1[0..1]
-      sts4(4, p1[1], p1[2], 0x3f803f80u, 0x00003f80u);  // k 32..39: x1[2..5] 1 1 1 0
-      sts4(5, 0u, 0u, 0u, 0u);                      // k 40..47
-    }
+    // ---- layer 1 on the tensor core: this thread's operand row ----
+    if (warp_on) store_l1_operand_row(arow, u, z);
     mma_round(smem_u32(sB1), 3);
     // ---- accumulator row (x W1 + b1) -> activation -> bf16 -> this thread's row of the group's A tile ----
     if (warp_on) {
 #pragma unroll 2
       for (int c0 = 0; c0 < 128; c0 += 16) {
         uint32_t v[16];
-        asm volatile(
-            "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-            : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
-              "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-            : "r"(trow + (uint32_t)c0));
-        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+        tmem_ld16(trow + (uint32_t)c0, v);
         uint32_t pk[8];
 #pragma unroll
         for (int j = 0; j < 8; ++j) pk[j] = pack2(act(__uint_as_float(v[2 * j])), act(__uint_as_float(v[2 * j + 1])));
-        asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(arow + (uint32_t)(c0 >> 3) * kTcKStride), "r"(pk[0]), "r"(pk[1]), "r"(pk[2]), "r"(pk[3]) : "memory");
-        asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(arow + (uint32_t)((c0 >> 3) + 1) * kTcKStride), "r"(pk[4]), "r"(pk[5]), "r"(pk[6]), "r"(pk[7]) : "memory");
+        sts4(arow + (uint32_t)(c0 >> 3) * kTcKStride, pk[0], pk[1], pk[2], pk[3]);
+        sts4(arow + (uint32_t)((c0 >> 3) + 1) * kTcKStride, pk[4], pk[5], pk[6], pk[7]);
       }
     }
     // ---- layer 2 on the tensor core: 8 UMMAs (M128 N128 K16) ----
@@ -501,34 +293,8 @@ struct MlpTcFastPredT {
     // ---- this thread's accumulator row -> bias + activation -> layer 3 -> next state ----
     float y[5] = {0.f, 0.f, 0.f, 0.f, 0.f};
 #pragma unroll 2
-    for (int c0 = 0; c0 < 128; c0 += 16) {
-      uint32_t v[16];
-      asm volatile(
-          "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-          : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
-            "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-          : "r"(trow + (uint32_t)c0));
-      asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-      for (int q4 = 0; q4 < 4; ++q4) {
-        const uint32_t jo = (uint32_t)(c0 + q4 * 4) * 4u;
-        const float4 bb = MlpTcPredV1::lds4(ab2 + jo);
-        const float h0 = act(__uint_as_float(v[4 * q4]) + bb.x), h1 = act(__uint_as_float(v[4 * q4 + 1]) + bb.y);
-        const float h2 = act(__uint_as_float(v[4 * q4 + 2]) + bb.z), h3 = act(__uint_as_float(v[4 * q4 + 3]) + bb.w);
-#pragma unroll
-        for (int k = 0; k < 5; ++k) {
-          const float4 w = MlpTcPredV1::lds4(aW3 + (uint32_t)k * 512u + jo);
-          y[k] = fmaf(h3, w.w, fmaf(h2, w.z, fmaf(h1, w.y, fmaf(h0, w.x, y[k]))));
-        }
-      }
-    }
-    z.om = y[0] + b3[0];
-    z.c = y[1] + b3[1];
-    z.s = y[2] + b3[2];
-    z.x = y[3] + b3[3];
-    z.v = y[4] + b3[4];
-    z.th = atan2f(z.s, z.c);
-    omc = 1.0f - z.c * rsqrtf(fmaf(z.c, z.c, z.s * z.s));
+    for (int c0 = 0; c0 < 128; c0 += 16) fold_l3_chunk<act>(trow + (uint32_t)c0, c0, ab2, aW3, y);
+    mlp_outputs_to_state(z, y, b3, omc);
   }
 };
 using MlpTcBf16Pred = MlpTcFastPredT<false>;
@@ -536,7 +302,7 @@ using MlpTcFastPred = MlpTcFastPredT<true>;
 
 // ---------------------------------------------------------------------------------------------------------------
 // The exact (fp32-level) engine, round-2 structure: the tile-per-warp-group organisation of the single-product engines above with
-// the six-product bf16 x 3 arithmetic of MlpTcPredV1.  TWO 128-rollout tiles in flight per SM (groups), each worked on by 256 threads:
+// six-product bf16 x 3 arithmetic.  TWO 128-rollout tiles in flight per SM (groups), each worked on by 256 threads:
 // the 128 OWNER threads (one per rollout: operand row of layer 1, state, cost) and 128 HELPER threads; owner and helper of a row split
 // the row's columns in the FP32 / MUFU stages (the row's 512 MUFU operations per step at 8 cycles per warp instruction are the longest
 // link of a tile's serial chain: with one thread per row the two tiles ran the tensor core, the MUFU and the FP32 pipe one after
@@ -545,7 +311,7 @@ using MlpTcFastPred = MlpTcFastPredT<true>;
 //             [0, 128) of the group;
 //   layer 2 : K is processed in QUARTERS: owner and helper read 16 columns each of the row's L1 accumulator, apply tanh, split the
 //             values into three bf16 terms and write them into one of the group's two quarter buffers (3 terms x 4 k-groups = 24 KB;
-//             the three full A tiles of the V1 engine, 96 KB per tile in flight, are what kept it at one tile per SM); the group's first
+//             three full A tiles, 96 KB per tile in flight, would allow only one tile per SM); the group's first
 //             thread then issues that quarter's 12 UMMAs (six products x two K16 slices, smallest products first) into the L2
 //             accumulator, TMEM columns [128, 256), and commits them to the buffer's mbarrier -- the tensor core works on quarter p
 //             while the group's threads produce quarter p + 1 (TMEM load, MUFU, split) and while the OTHER group is in any phase;
@@ -563,6 +329,7 @@ struct MlpTcPred {
   static constexpr int kCemThreads = 256 * kGroups;
   static constexpr int kMinBlocks = 1;
   static constexpr int kRolloutsPerBlock = 128 * kGroups;
+  static constexpr size_t kAccSmemBytes = 12 * 1024;  // what the buffers leave of the 227 KB for the MPPI accumulators [n_ind][256]
   static constexpr uint32_t kQBuf = 3u * 4u * kTcKStride;  // one K-quarter (four k-groups) of the three split terms: 24 KB
   uint8_t* sA;        // this group's two quarter buffers [2][kQBuf]; buffer 0 also takes the layer-1 operand rows (six k-groups)
   uint8_t* sB;        // [3][32768] W2 split tiles (resident, shared by the groups)
@@ -599,22 +366,12 @@ struct MlpTcPred {
     for (int i = threadIdx.x; i < (int)(kTcBlobBytes / 16); i += blockDim.x) dst[i] = src[i];
     if (threadIdx.x < 4 * kGroups) asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(mb0 + threadIdx.x)) : "memory");
     if (threadIdx.x == 0) asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    if ((threadIdx.x >> 5) == 0) {  // the CTA owns the SM: all 512 TMEM columns, 256 per group (layer-1 and layer-2 accumulators)
-      asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(smem_u32(tmem_slot)) : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    tmem_alloc_cta<512>(tmem_slot);  // the CTA owns the SM: all 512 TMEM columns, 256 per group (layer-1 and layer-2 accumulators)
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     // caller issues __syncthreads() after construction
   }
-  __device__ __forceinline__ ~MlpTcPred() {
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    if ((threadIdx.x >> 5) == 0) {
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-      asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(*tmem_slot) : "memory");
-    }
-  }
+  __device__ __forceinline__ ~MlpTcPred() { tmem_dealloc_cta<512>(tmem_slot); }
   __device__ __forceinline__ void substep(State& z, float u, float& omc) { step(z, u, omc); }
   __device__ __forceinline__ bool single_substep() const { return false; }
   __device__ __forceinline__ void use_uniform(const HotUK&) {}
@@ -622,8 +379,6 @@ struct MlpTcPred {
   __device__ __forceinline__ void begin_rollout(bool = true) { row_on = grp * 128 + (int)(threadIdx.x & 127u) < tile_rows; }
   // a group runs a pass of the rollout loop iff its first row is a real rollout (group-uniform: the group's barriers stay matched)
   __device__ __forceinline__ bool group_active(int base, int end) { tile_rows = end - base; return grp * 128 < tile_rows; }
-
-  static __device__ __forceinline__ float tanh5(float x) { return MlpTcPredV1::tanh5(x); }
 
   __device__ __forceinline__ void step(State& z, float u, float& omc) {
     const int tid = threadIdx.x, g = grp, row = tid & 127, wq = (tid >> 5) & 3;
@@ -635,7 +390,6 @@ struct MlpTcPred {
     const uint32_t trow = tmem_g + ((uint32_t)(wq * 32) << 16);
     const uint32_t bar0 = smem_u32(mbar);
     const bool issuer = (row == 0) && (half == 0);
-    constexpr uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((128u >> 3) << 17) | ((128u >> 4) << 24);
     // operand rows written by this group -> visible to the tensor core; then the group's named barrier
     auto publish = [&]() {
       asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
@@ -644,41 +398,21 @@ struct MlpTcPred {
     };
     // one lane per warp polls the mbarrier, the warp's other lanes wait at the warp barrier
     auto wait_mbar = [&](uint32_t bar, uint32_t parity) {
-      if ((tid & 31) == 0) {
-        uint32_t done = 0;
-        while (!done) {
-          asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.b32 %0, 1, 0, p;\n\t}\n"
-                       : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-        }
-      }
+      if ((tid & 31) == 0) mbar_wait(bar, parity);
       __syncwarp();
       asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     };
-    // ---- layer 1 on the tensor core: the owner's operand row [x1 x2 x3 x1 x2 x1 | 1 1 1 | 0 ...] (three-term bf16 split of the six
-    //      inputs, K = 48 = six k-groups at the start of quarter buffer 0, which the previous step's MMAs have released) ----
-    if (warp_on && half == 0) {
-      uint32_t p1[3], p2[3], p3[3];
-      MlpTcPredV1::split3(u, z.om, p1[0], p2[0], p3[0]);
-      MlpTcPredV1::split3(z.c, z.s, p1[1], p2[1], p3[1]);
-      MlpTcPredV1::split3(z.x, z.v, p1[2], p2[2], p3[2]);
-      auto sts4 = [&](int kg, uint32_t w0, uint32_t w1, uint32_t w2, uint32_t w3) {
-        asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(arow + (uint32_t)kg * kTcKStride), "r"(w0), "r"(w1), "r"(w2), "r"(w3) : "memory");
-      };
-      sts4(0, p1[0], p1[1], p1[2], p2[0]);          // k  0.. 7: x1[0..5] x2[0..1]
-      sts4(1, p2[1], p2[2], p3[0], p3[1]);          // k  8..15: x2[2..5] x3[0..3]
-      sts4(2, p3[2], p1[0], p1[1], p1[2]);          // k 16..23: x3[4..5] x1[0..5]
-      sts4(3, p2[0], p2[1], p2[2], p1[0]);          // k 24..31: x2[0..5] x1[0..1]
-      sts4(4, p1[1], p1[2], 0x3f803f80u, 0x00003f80u);  // k 32..39: x1[2..5] 1 1 1 0
-      sts4(5, 0u, 0u, 0u, 0u);                      // k 40..47
-    }
+    // ---- layer 1 on the tensor core: the owner's operand row, at the start of quarter buffer 0, which the previous step's MMAs have
+    //      released ----
+    if (warp_on && half == 0) store_l1_operand_row(arow, u, z);
     publish();
     if (issuer) {
       asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
       const uint32_t b1a = smem_u32(sB1);
 #pragma unroll
       for (int ks = 0; ks < 3; ++ks)
-        umma_bf16(tmem_g, umma_smem_desc(a_grp + (uint32_t)ks * 2u * kTcKStride), umma_smem_desc(b1a + (uint32_t)ks * 2u * kTcKStride), idesc, ks > 0 ? 1u : 0u);
-      asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar0) : "memory");
+        umma_bf16(tmem_g, umma_smem_desc(a_grp + (uint32_t)ks * 2u * kTcKStride), umma_smem_desc(b1a + (uint32_t)ks * 2u * kTcKStride), kTcIdescM128N128, ks > 0 ? 1u : 0u);
+      umma_commit(bar0);
     }
     wait_mbar(bar0, phase);
     phase ^= 1u;
@@ -692,22 +426,17 @@ struct MlpTcPred {
       const uint32_t brow = arow + bsel * kQBuf;
       if (warp_on) {
         uint32_t v[16];
-        asm volatile(
-            "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-            : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
-              "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-            : "r"(trow + (uint32_t)(32 * p + 16 * half)));
-        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+        tmem_ld16(trow + (uint32_t)(32 * p + 16 * half), v);
         uint32_t q1[8], q2[8], q3[8];
 #pragma unroll
         for (int j = 0; j < 8; ++j)
-          MlpTcPredV1::split3(tanh5(__uint_as_float(v[2 * j])), tanh5(__uint_as_float(v[2 * j + 1])), q1[j], q2[j], q3[j]);
+          split3(tanh5(__uint_as_float(v[2 * j])), tanh5(__uint_as_float(v[2 * j + 1])), q1[j], q2[j], q3[j]);
 #pragma unroll
         for (int kk = 0; kk < 2; ++kk) {
           const uint32_t dst = brow + (uint32_t)(2 * half + kk) * kTcKStride;
-          asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(dst), "r"(q1[4 * kk]), "r"(q1[4 * kk + 1]), "r"(q1[4 * kk + 2]), "r"(q1[4 * kk + 3]) : "memory");
-          asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(dst + 4u * kTcKStride), "r"(q2[4 * kk]), "r"(q2[4 * kk + 1]), "r"(q2[4 * kk + 2]), "r"(q2[4 * kk + 3]) : "memory");
-          asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(dst + 8u * kTcKStride), "r"(q3[4 * kk]), "r"(q3[4 * kk + 1]), "r"(q3[4 * kk + 2]), "r"(q3[4 * kk + 3]) : "memory");
+          sts4(dst, q1[4 * kk], q1[4 * kk + 1], q1[4 * kk + 2], q1[4 * kk + 3]);
+          sts4(dst + 4u * kTcKStride, q2[4 * kk], q2[4 * kk + 1], q2[4 * kk + 2], q2[4 * kk + 3]);
+          sts4(dst + 8u * kTcKStride, q3[4 * kk], q3[4 * kk + 1], q3[4 * kk + 2], q3[4 * kk + 3]);
         }
       }
       publish();
@@ -720,10 +449,10 @@ struct MlpTcPred {
 #pragma unroll
           for (int ks = 0; ks < 2; ++ks)
             umma_bf16(tmem_g + 128u, umma_smem_desc(abuf + (uint32_t)ta[term] * 4u * kTcKStride + (uint32_t)ks * 2u * kTcKStride),
-                      umma_smem_desc(b2t + (uint32_t)tb[term] * kTcTileBytes + (uint32_t)(2 * p + ks) * 2u * kTcKStride), idesc,
+                      umma_smem_desc(b2t + (uint32_t)tb[term] * kTcTileBytes + (uint32_t)(2 * p + ks) * 2u * kTcKStride), kTcIdescM128N128,
                       (p > 0 || term > 0 || ks > 0) ? 1u : 0u);
         }
-        asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar0 + 8u * (1u + bsel)) : "memory");
+        umma_commit(bar0 + 8u * (1u + bsel));
       }
     }
     wait_mbar(bar0 + 8u, 1u);   // quarter 2 (buffer 0 is free for the next step's layer-1 rows)
@@ -732,27 +461,7 @@ struct MlpTcPred {
     float y[5] = {0.f, 0.f, 0.f, 0.f, 0.f};
     if (warp_on) {
 #pragma unroll 2
-      for (int c0 = 64 * half; c0 < 64 * half + 64; c0 += 16) {
-        uint32_t v[16];
-        asm volatile(
-            "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-            : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
-              "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-            : "r"(trow + 128u + (uint32_t)c0));
-        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-        for (int q4 = 0; q4 < 4; ++q4) {
-          const uint32_t jo = (uint32_t)(c0 + q4 * 4) * 4u;
-          const float4 bb = MlpTcPredV1::lds4(ab2 + jo);
-          const float h0 = tanh5(__uint_as_float(v[4 * q4]) + bb.x), h1 = tanh5(__uint_as_float(v[4 * q4 + 1]) + bb.y);
-          const float h2 = tanh5(__uint_as_float(v[4 * q4 + 2]) + bb.z), h3 = tanh5(__uint_as_float(v[4 * q4 + 3]) + bb.w);
-#pragma unroll
-          for (int k = 0; k < 5; ++k) {
-            const float4 w = MlpTcPredV1::lds4(aW3 + (uint32_t)k * 512u + jo);
-            y[k] = fmaf(h3, w.w, fmaf(h2, w.z, fmaf(h1, w.y, fmaf(h0, w.x, y[k]))));
-          }
-        }
-      }
+      for (int c0 = 64 * half; c0 < 64 * half + 64; c0 += 16) fold_l3_chunk<tanh5>(trow + 128u + (uint32_t)c0, c0, ab2, aW3, y);
     }
     // helper -> owner: five partial sums per row through quarter buffer 1 ([128 rows][8 floats])
     float* sy = reinterpret_cast<float*>(sA + kQBuf) + row * 8;
@@ -767,14 +476,7 @@ struct MlpTcPred {
       const float4 v0 = reinterpret_cast<const float4*>(sy)[0];
       y[0] += v0.x; y[1] += v0.y; y[2] += v0.z; y[3] += v0.w; y[4] += sy[4];
     }
-    z.om = y[0] + b3[0];
-    z.c = y[1] + b3[1];
-    z.s = y[2] + b3[2];
-    z.x = y[3] + b3[3];
-    z.v = y[4] + b3[4];
-    z.th = atan2f(z.s, z.c);
-    // the network's (cos, sin) outputs are not normalised: cos(atan2(s, c)) = c / hypot(s, c)
-    omc = 1.0f - z.c * rsqrtf(fmaf(z.c, z.c, z.s * z.s));
+    mlp_outputs_to_state(z, y, b3, omc);
   }
 };
 #endif  // __CUDACC__

@@ -21,28 +21,34 @@ static cudaError_t launch_mppi_p(int kind, bool log, int nblocks, int block, siz
   if (kind == 0) return log ? launch_mppi_t<Pred, 0, true>(nblocks, block, smem, st, a) : launch_mppi_t<Pred, 0, false>(nblocks, block, smem, st, a);
   return log ? launch_mppi_t<Pred, 1, true>(nblocks, block, smem, st, a) : launch_mppi_t<Pred, 1, false>(nblocks, block, smem, st, a);
 }
-cudaError_t launch_mppi_rollout(int pred, int kind, bool log, int nblocks, int block, size_t smem, cudaStream_t st, const MppiArgs& a) {
-  if (pred == 2) return launch_mppi_p<MlpTcPred>(kind, log, nblocks, block, smem, st, a);
-  if (pred == 6) return launch_mppi_p<MlpTcPredV1>(kind, log, nblocks, block, smem, st, a);
-  if (pred == 3) return launch_mppi_p<MlpTcBf16Pred>(kind, log, nblocks, block, smem, st, a);
-  if (pred == 4) return launch_mppi_p<MlpTcFastPred>(kind, log, nblocks, block, smem, st, a);
-  if (pred == 5) return launch_mppi_rollout_gru(kind, log, nblocks, block, smem, st, a);  // ctk_gru.cu
-  return pred == 0 ? launch_mppi_p<OdePred>(kind, log, nblocks, block, smem, st, a)
-                   : launch_mppi_p<MlpSimtPred>(kind, log, nblocks, block, smem, st, a);
+cudaError_t launch_mppi_rollout(PredKind pred, int kind, bool log, int nblocks, int block, size_t smem, cudaStream_t st, const MppiArgs& a) {
+  switch (pred) {
+    case PredKind::Ode: return launch_mppi_p<OdePred>(kind, log, nblocks, block, smem, st, a);
+    case PredKind::MlpSimt: return launch_mppi_p<MlpSimtPred>(kind, log, nblocks, block, smem, st, a);
+    case PredKind::MlpTc: return launch_mppi_p<MlpTcPred>(kind, log, nblocks, block, smem, st, a);
+    case PredKind::MlpTcBf16: return launch_mppi_p<MlpTcBf16Pred>(kind, log, nblocks, block, smem, st, a);
+    case PredKind::MlpTcFast: return launch_mppi_p<MlpTcFastPred>(kind, log, nblocks, block, smem, st, a);
+    case PredKind::Gru: return launch_mppi_rollout_gru(kind, log, nblocks, block, smem, st, a);  // ctk_gru.cu
+  }
+  return cudaErrorInvalidValue;
 }
-// pred: 0 ODE, 1 MLP on the FP32 pipe, 2 MLP with layer 2 on the tensor cores (tcgen05, bf16 x 3 split: fp32-level), 3 / 4 the opt-in
-// single-bf16-product engines (3: exact tanh, 4: MUFU.TANH)
-// 5: the recurrent (GRU) predictor on the FP32 pipe; 6: the round-1 structure of engine 2 (one tile in flight, CTK_TC_EXACT_V1=1: A/B runs)
-int mppi_max_block_threads(int pred) {
-  if (pred == 5) return GruSimtPred::kMaxThreads;
-  if (pred == 6) return MlpTcPredV1::kMaxThreads;
-  if (pred == 3 || pred == 4) return MlpTcBf16Pred::kMaxThreads;
-  return pred == 0 ? OdePred::kMaxThreads : (pred >= 2 ? MlpTcPred::kMaxThreads : MlpSimtPred::kMaxThreads);
+
+template <class Pred>
+static PredInfo pred_info_of(const char* name) {
+  PredInfo i{name, Pred::kMaxThreads, Pred::kRolloutsPerBlock, Pred::kBalanced, 0, &Pred::smem_floats};
+  if constexpr (Pred::kRolloutsPerBlock > 0) i.acc_smem_bytes = Pred::kAccSmemBytes;
+  return i;
 }
-size_t mppi_pred_smem_floats(int pred, const MlpDev& m) {
-  if (pred == 5) return GruSimtPred::smem_floats(m);
-  if (pred == 6) return MlpTcPredV1::smem_floats(m);
-  return pred == 0 ? 0 : (pred == 2 ? MlpTcPred::smem_floats(m) : (pred >= 3 ? MlpTcBf16Pred::smem_floats(m) : MlpSimtPred::smem_floats(m)));
+PredInfo pred_info(PredKind pred) {
+  switch (pred) {
+    case PredKind::Ode: return pred_info_of<OdePred>("OdePred");
+    case PredKind::MlpSimt: return pred_info_of<MlpSimtPred>("MlpSimtPred");
+    case PredKind::MlpTc: return pred_info_of<MlpTcPred>("MlpTcPred");
+    case PredKind::MlpTcBf16: return pred_info_of<MlpTcBf16Pred>("MlpTcBf16Pred");
+    case PredKind::MlpTcFast: return pred_info_of<MlpTcFastPred>("MlpTcFastPred");
+    case PredKind::Gru: return pred_info_of<GruSimtPred>("GruSimtPred");
+  }
+  return {};
 }
 
 #ifndef CTK_K1_MAXT2
@@ -169,12 +175,12 @@ __global__ void single_rollout_kernel(const float* s0, const float* Q, int H, co
   summed[0] = (sum - cost.shift) * (float)(H + 1);  // the device constants carry the 1/(H+1) of the trajectory mean
 }
 
-cudaError_t launch_single_rollout(int pred, const float* s0, const float* Q, int H, const DevConsts* kc, const MlpDev& mlp, const float* u_prev, float* traj, float* summed, cudaStream_t st) {
-  if (pred == 0) {
+cudaError_t launch_single_rollout(PredKind pred, const float* s0, const float* Q, int H, const DevConsts* kc, const MlpDev& mlp, const float* u_prev, float* traj, float* summed, cudaStream_t st) {
+  if (pred == PredKind::Ode) {
     single_rollout_kernel<OdePred><<<1, 32, 0, st>>>(s0, Q, H, kc, mlp, u_prev, traj, summed);
     return cudaGetLastError();
   }
-  if (pred == 5) return launch_single_rollout_gru(s0, Q, H, kc, mlp, u_prev, traj, summed, st);  // ctk_gru.cu
+  if (pred == PredKind::Gru) return launch_single_rollout_gru(s0, Q, H, kc, mlp, u_prev, traj, summed, st);  // ctk_gru.cu
   const size_t smem = sizeof(float) * MlpSimtPred::smem_floats(mlp);
   auto k = single_rollout_kernel<MlpSimtPred>;
   if (smem > 48 * 1024) {

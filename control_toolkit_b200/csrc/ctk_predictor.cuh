@@ -2,7 +2,7 @@
 // reference call sites optimizer_mppi.py:188, optimizer_cem_tf.py:57, optimizer_rpgd.py:300).
 //   OdePred     : CartPole Euler ODE, one thread per rollout, state in registers.
 //   MlpSimtPred : 6 -> hidden tanh -> hidden tanh -> 5 MLP on the FP32 pipe (one thread per rollout, weights in
-//                 shared memory).  Numerical anchor for the tcgen05 engine (ctk_mlp_tc.cuh).
+//                 shared memory).  Numerical anchor for the tcgen05 engines (ctk_mlp_tc.cuh).
 #pragma once
 #include "ctk_args.cuh"
 #include "ctk_device.cuh"
@@ -42,6 +42,20 @@ __device__ __forceinline__ float tanh_acc(float x) {
   const float x2 = x * x;
   const float ser = x * fmaf(x2, fmaf(x2, 0.13333334f, -0.33333334f), 1.0f);
   return (ax < 0.06f) ? ser : copysignf(r, x);
+}
+
+// network outputs y (before the output bias b3) -> next state [angleD, cos, sin, position, positionD]; angle = atan2(sin, cos)
+// (oracle/spec.py MLPPredictor.step).  b3 is a reference to the caller's member: an out-of-line step() re-reads it after each store
+// through z (which may alias the functor), so its code is that of the same statements written in place
+__device__ __forceinline__ void mlp_outputs_to_state(State& z, const float (&y)[5], const float* const& b3, float& omc) {
+  z.om = y[0] + b3[0];
+  z.c = y[1] + b3[1];
+  z.s = y[2] + b3[2];
+  z.x = y[3] + b3[3];
+  z.v = y[4] + b3[4];
+  z.th = atan2f(z.s, z.c);
+  // the network's (cos, sin) outputs are not normalised: cos(atan2(s, c)) = c / hypot(s, c)
+  omc = 1.0f - z.c * rsqrtf(fmaf(z.c, z.c, z.s * z.s));
 }
 
 struct MlpSimtPred {
@@ -114,14 +128,7 @@ struct MlpSimtPred {
         for (int k = 0; k < 5; ++k) y[k] = fmaf(h2, W3T[k * hid + j0 + jj], y[k]);
       }
     }
-    z.om = y[0] + b3[0];
-    z.c = y[1] + b3[1];
-    z.s = y[2] + b3[2];
-    z.x = y[3] + b3[3];
-    z.v = y[4] + b3[4];
-    z.th = atan2f(z.s, z.c);
-    // the network's (cos, sin) outputs are not normalised: cos(atan2(s, c)) = c / hypot(s, c)
-    omc = 1.0f - z.c * rsqrtf(fmaf(z.c, z.c, z.s * z.s));
+    mlp_outputs_to_state(z, y, b3, omc);
   }
 };
 
@@ -244,13 +251,7 @@ struct GruSimtPred {
         for (int k = 0; k < 5; ++k) y[k] = fmaf(a2[j], W3T[k * hid + j], y[k]);
       }
     }
-    z.om = y[0] + b3[0];
-    z.c = y[1] + b3[1];
-    z.s = y[2] + b3[2];
-    z.x = y[3] + b3[3];
-    z.v = y[4] + b3[4];
-    z.th = atan2f(z.s, z.c);
-    omc = 1.0f - z.c * rsqrtf(fmaf(z.c, z.c, z.s * z.s));
+    mlp_outputs_to_state(z, y, b3, omc);  // the same Dense read-out as the MLP
   }
 };
 

@@ -1,5 +1,5 @@
 #!/bin/bash
-# exact tcgen05 engine (round-2 structure) against its round-1 structure, and an A/B of the round-1 tree (_ab_r01, commit 9401463) against
+# exact tcgen05 engine (round-2 structure), and an A/B of the round-1 tree (_ab_r01, commit 9401463) against
 # the current one on the SAME box (default workload and the logging workload)
 set -u
 O=gpurun_out
@@ -7,7 +7,6 @@ P=/tmp/ctk_prof
 mkdir -p $O $P
 timeout 900 python -m pytest tests -m gpu -q --timeout 600 -k "tcgen05 or mlp or top_m" 2>&1 | tail -15 | tee $O/pytest_gpu_mlp.txt
 python bench.py --workload mppi_mlp_c4 --mlp-engine tcgen05 --steps 10 --warmup 3 > $O/bench_mlp_exact_v2.json 2> $O/bench_mlp_exact_v2.err
-CTK_TC_EXACT_V1=1 python bench.py --workload mppi_mlp_c4 --mlp-engine tcgen05 --steps 10 --warmup 3 > $O/bench_mlp_exact_v1.json 2> $O/bench_mlp_exact_v1.err
 for i in 1 2; do
   (cd _ab_r01 && python bench.py > ../$O/ab_r01_default_$i.json 2> ../$O/ab_r01_default_$i.err)
   python bench.py > $O/ab_r02_default_$i.json 2> $O/ab_r02_default_$i.err

@@ -532,7 +532,7 @@ __global__ void __launch_bounds__(kCemTickThreads) cem_tick_kernel(const CemTick
         } else {
           const float u = status ? __int_as_float(0x7fc00000) : first_q;
           if (!a.freeze_prev) a.u_prev[0] = u;
-          if (a.u_out != nullptr) a.u_out[0] = u;
+          if (a.u_out != nullptr) { a.u_out[0] = u; a.u_out[1] = (float)status; }
           if (a.host.p != nullptr) { host_put(a.host, 5, (float)status); host_put(a.host, 4, u); }
         }
         if (tid == H - 1) {

@@ -85,6 +85,9 @@ __device__ __forceinline__ int poll_records(RecPtr rec_ptr, int nrec, int P, uns
       if (!ld_tagged(rec_ptr(m) + c, seq, t0, &v)) lost = 1;
       if (dst != nullptr) dst[i] = v;
     }
+    // here a record's slots were stored by other threads than its owner (the fast path's thread m stores record m itself), and
+    // staged_combine reads every record's rho before its first barrier
+    if (dst != nullptr) __syncthreads();
   }
   return lost;
 }

@@ -217,7 +217,8 @@ int ctk_step_finish(ctk_handle *h, const float *gathered_dev, int num_shards, fl
 
 /* Asynchronous device-resident tick: s_dev [ns] and u_out_dev [2] (u, exchange status) stay on the device, nothing is
    synchronised.  With a connected exchange (below) every shard calls it once per tick; the whole tick -- rollouts,
-   softmin record, NVLink record exchange, u_nom update -- is ONE kernel launch.                                    */
+   softmin record, NVLink record exchange, u_nom update -- is ONE kernel launch.  The status word (0: ok) is written by the
+   CartPole MPPI tick and the one-launch CEM tick; the other ticks write u only (general environments: u_out_dev [nu]). */
 int ctk_step_device(ctk_handle *h, const float *s_dev, float *u_out_dev);
 
 /* n ticks back to back (states s_dev + i * s_stride floats, results [u, status] to u_out_dev + i * u_stride floats; u_out_dev may

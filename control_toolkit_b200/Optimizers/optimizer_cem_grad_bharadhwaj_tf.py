@@ -67,5 +67,5 @@ class optimizer_cem_grad_bharadhwaj_tf(optimizer_cem_naive_grad_tf):
 
     def adam_weights(self):
         """[iterations, m, v] like ``self.optim.get_weights()``; m, v are attached to the population rows."""
-        shape = (self.num_rollouts, self.mpc_horizon, 1)
+        shape = (self.num_rollouts, self.mpc_horizon, self.num_control_inputs)
         return [self._get_counter(L.COUNTER_ADAM_STEP), self._get_state(L.STATE_RPGD_M, shape), self._get_state(L.STATE_RPGD_V, shape)]

@@ -103,7 +103,7 @@ class optimizer_cem_naive_grad_tf(template_optimizer):
         if self.optimizer_logging:
             self.logging_values["Q_logged"] = self._get_log(L.LOG_Q, (N, H, nu))
             self.logging_values["J_logged"] = self._get_log(L.LOG_J, (N,))
-            self.logging_values["rollout_trajectories_logged"] = self._get_log(L.LOG_ROLLOUTS, (N, H + 1, 6))
+            self.logging_values["rollout_trajectories_logged"] = self._get_log(L.LOG_ROLLOUTS, (N, H + 1, int(self.num_states)))
             self.logging_values["u_logged"] = self.u
         self._last_iterations = iterations
         self.count += 1
@@ -118,11 +118,11 @@ class optimizer_cem_naive_grad_tf(template_optimizer):
     # reference attributes, read from the device on demand
     @property
     def dist_mue(self) -> np.ndarray:
-        return self._get_state(L.STATE_CEM_MU, (1, self.mpc_horizon, 1))
+        return self._get_state(L.STATE_CEM_MU, (1, self.mpc_horizon, self.num_control_inputs))
 
     @property
     def stdev(self) -> np.ndarray:
-        return self._get_state(L.STATE_CEM_STD, (1, self.mpc_horizon, 1))
+        return self._get_state(L.STATE_CEM_STD, (1, self.mpc_horizon, self.num_control_inputs))
 
     def elite_indices(self) -> np.ndarray:
         """[outer iterations of the last tick, cem_best_k] population indices, best first."""

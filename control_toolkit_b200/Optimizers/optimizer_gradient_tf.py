@@ -94,7 +94,7 @@ class optimizer_gradient_tf(template_optimizer):
         if self.optimizer_logging:
             self.logging_values["Q_logged"] = self._get_log(L.LOG_Q, (N, H, nu))
             self.logging_values["J_logged"] = self._get_log(L.LOG_J, (N,))
-            self.logging_values["rollout_trajectories_logged"] = self._get_log(L.LOG_ROLLOUTS, (N, H + 1, 6))
+            self.logging_values["rollout_trajectories_logged"] = self._get_log(L.LOG_ROLLOUTS, (N, H + 1, int(self.num_states)))
             self.logging_values["u_logged"] = self.u
         self.count += 1  # :141
         return self.u
@@ -109,11 +109,11 @@ class optimizer_gradient_tf(template_optimizer):
     # reference attributes, read from the device on demand
     @property
     def Q_tf(self) -> np.ndarray:
-        return self._get_state(L.STATE_RPGD_Q, (self.num_rollouts, self.mpc_horizon, 1))
+        return self._get_state(L.STATE_RPGD_Q, (self.num_rollouts, self.mpc_horizon, self.num_control_inputs))
 
     def adam_weights(self):
         """[iterations, m, v] like ``self.optim.get_weights()`` (:151)."""
-        shape = (self.num_rollouts, self.mpc_horizon, 1)
+        shape = (self.num_rollouts, self.mpc_horizon, self.num_control_inputs)
         return [self._get_counter(L.COUNTER_ADAM_STEP), self._get_state(L.STATE_RPGD_M, shape), self._get_state(L.STATE_RPGD_V, shape)]
 
     def best_index(self) -> int:

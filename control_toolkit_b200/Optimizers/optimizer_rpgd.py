@@ -64,8 +64,8 @@ class optimizer_rpgd(template_optimizer):
         self.sample_stdev = np.float32(sample_stdev)
         self.sample_mean = np.float32(sample_mean)
         self.sample_whole_control_space = bool(sample_whole_control_space)
-        if self.sample_whole_control_space:  # :199-205
-            self.sample_min, self.sample_max = np.float32(self.action_low[0]), np.float32(self.action_high[0])
+        if self.sample_whole_control_space:  # :199-205, per input
+            self.sample_min, self.sample_max = np.asarray(self.action_low, np.float32), np.asarray(self.action_high, np.float32)
         else:
             self.sample_min, self.sample_max = np.float32(uniform_dist_min), np.float32(uniform_dist_max)
         self.resamp_per = int(resamp_per)
@@ -102,6 +102,9 @@ class optimizer_rpgd(template_optimizer):
         self.number_of_interpolation_inducing_points = int(
             math.ceil((self.mpc_horizon - 1) / self.period_interpolation_inducing_points) + 1)
         self._create_backend(dt, predictor_specification)
+        if self.calculate_optimal_trajectory and self._env_info.env_id != L.ENV_CARTPOLE:
+            raise ValueError("calculate_optimal_trajectory: the nominal rollout (ctk_rollout_single) is implemented for the CartPole "
+                             f"environment only, not {self._environment()!r}")
         self.optimizer_reset()
 
     def _fill_config(self, cfg: L.ctk_config) -> None:
@@ -114,7 +117,9 @@ class optimizer_rpgd(template_optimizer):
         cfg.rpgd_distribution = L.DIST_NORMAL if self.SAMPLING_DISTRIBUTION == "normal" else L.DIST_UNIFORM
         cfg.rpgd_adam_form = L.ADAM_KERAS if self.adam_form == "keras" else L.ADAM_TORCH
         cfg.rpgd_sample_mean, cfg.rpgd_sample_stdev = float(self.sample_mean), float(self.sample_stdev)
-        cfg.rpgd_sample_min, cfg.rpgd_sample_max = float(self.sample_min), float(self.sample_max)
+        # the CartPole reads the scalar range; other environments sample each input over its own limits when the whole space is sampled
+        cfg.rpgd_sample_min, cfg.rpgd_sample_max = float(np.ravel(self.sample_min)[0]), float(np.ravel(self.sample_max)[0])
+        cfg.rpgd_sample_whole_space = int(self.sample_whole_control_space)
         cfg.rpgd_learning_rate = float(np.float32(self.learning_rate))
         cfg.rpgd_gradmax_clip = float(self.gradmax_clip)
         cfg.rpgd_beta_1, cfg.rpgd_beta_2, cfg.rpgd_epsilon = float(self.adam_beta_1), float(self.adam_beta_2), float(self.adam_epsilon)
@@ -133,7 +138,7 @@ class optimizer_rpgd(template_optimizer):
                                                         self.number_of_interpolation_inducing_points,
                                                         self.num_control_inputs))])
         H, nu, N = self.mpc_horizon, self.num_control_inputs, self.num_rollouts
-        u = self._tick(lib, s, L.STATE_U_NOM, H)  # u and Q[best] (:426) come back through the same host mirror
+        u = self._tick(lib, s, L.STATE_U_NOM, H * nu)  # u and Q[best] (:426) come back through the same host mirror
         self.u_nom = (self._state_buf.reshape(1, H, nu).copy() if self._state_buf is not None
                       else self._get_log(L.LOG_U_NOM, (1, H, nu)))
         if self.optimizer_logging:
@@ -158,7 +163,7 @@ class optimizer_rpgd(template_optimizer):
     # reference attributes, read from the device on demand
     @property
     def Q_tf(self) -> np.ndarray:
-        return self._get_state(L.STATE_RPGD_Q, (self.num_rollouts, self.mpc_horizon, 1))
+        return self._get_state(L.STATE_RPGD_Q, (self.num_rollouts, self.mpc_horizon, self.num_control_inputs))
 
     @property
     def trajectory_ages(self) -> np.ndarray:
@@ -166,7 +171,7 @@ class optimizer_rpgd(template_optimizer):
 
     def adam_weights(self):
         """[step, m, v] like ADAM.get_weights() (reference :84-99)."""
-        shape = (self.num_rollouts, self.mpc_horizon, 1)
+        shape = (self.num_rollouts, self.mpc_horizon, self.num_control_inputs)
         return [self._get_counter(L.COUNTER_ADAM_STEP), self._get_state(L.STATE_RPGD_M, shape), self._get_state(L.STATE_RPGD_V, shape)]
 
     def best_indices(self) -> np.ndarray:
@@ -178,14 +183,14 @@ class optimizer_rpgd(template_optimizer):
     def get_state(self) -> dict:
         step, m, v = self.adam_weights()
         return {"Q": self.Q_tf, "adam_step": step, "adam_m": m, "adam_v": v, "ages": self.trajectory_ages,
-                "count": self.count, "u": float(self._get_state(L.STATE_U_PREV, (1,))[0])}
+                "count": self.count, "u": self._get_state(L.STATE_U_PREV, (self.num_control_inputs,))}
 
     def set_state(self, state: dict) -> None:
         self._set_state(L.STATE_RPGD_Q, state["Q"])
         self._set_state(L.STATE_RPGD_M, state["adam_m"])
         self._set_state(L.STATE_RPGD_V, state["adam_v"])
         self._set_state(L.STATE_RPGD_AGES, state["ages"])
-        self._set_state(L.STATE_U_PREV, [state["u"]])
+        self._set_state(L.STATE_U_PREV, np.reshape(state["u"], (self.num_control_inputs,)))
         self._set_counter(L.COUNTER_ADAM_STEP, int(state["adam_step"]))
         self.count = int(state["count"])
         self._set_counter(L.COUNTER_COUNT, self.count)

@@ -70,7 +70,8 @@ class ctk_config(C.Structure):
         ("rpgd_sample_mean", C.c_float), ("rpgd_sample_stdev", C.c_float), ("rpgd_sample_min", C.c_float),
         ("rpgd_sample_max", C.c_float), ("rpgd_learning_rate", C.c_float), ("rpgd_gradmax_clip", C.c_float),
         ("rpgd_beta_1", C.c_double), ("rpgd_beta_2", C.c_double), ("rpgd_epsilon", C.c_double),
-        ("mlp_engine", C.c_int32), ("cem_uniform_actions", C.c_int32), ("rpgd_gradient_mode", C.c_int32), ("num_clients", C.c_int32), ("environment", C.c_int32), ("reserved", C.c_int32 * 3),
+        ("mlp_engine", C.c_int32), ("cem_uniform_actions", C.c_int32), ("rpgd_gradient_mode", C.c_int32), ("num_clients", C.c_int32), ("environment", C.c_int32),
+        ("rpgd_sample_whole_space", C.c_int32), ("reserved", C.c_int32 * 2),
     ]
 
 

@@ -19,7 +19,7 @@ CSRC = os.path.join(HERE, "csrc")
 INCLUDE = os.path.join(os.path.dirname(HERE), "include")
 OBJ = os.path.join(HERE, "build")
 LIB = os.path.join(HERE, "libctk_b200.so")
-UNITS = ["ctk_engine.cu", "ctk_mppi.cu", "ctk_cem.cu", "ctk_rpgd.cu", "ctk_batch.cu", "ctk_gru.cu", "ctk_env.cu"]
+UNITS = ["ctk_engine.cu", "ctk_mppi.cu", "ctk_cem.cu", "ctk_rpgd.cu", "ctk_batch.cu", "ctk_gru.cu", "ctk_env.cu", "ctk_env_rpgd.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC",
               "-I", INCLUDE, "-I", CSRC] + os.environ.get("CTK_NVCC_EXTRA", "").split()  # e.g. -DCTK_K1_MAXT2=1024
 

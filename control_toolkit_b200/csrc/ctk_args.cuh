@@ -393,6 +393,67 @@ struct EnvCemRefitArgs {
   int32_t* elite_idx_out;
 };
 
+// Gradient optimizers on a registered environment (ctk_kernels_env_rpgd.cuh).  Population arrays are [H][NU][N]: flat column
+// t * NU + c, one thread per trajectory reads coalesced.
+constexpr int kEnvRpgdBlock = 32;  // trajectories per block of the gradient kernel (= the largest population of the one-launch tick)
+constexpr size_t kEnvRpgdSmemMax = 227 * 1024 - 1024;  // the tape (dynamic shared memory); the fused select's arrays come on top
+struct EnvRpgdGradArgs {
+  int N, H, iters;
+  S0e s0;
+  const float* u_prev;   // [NU]
+  float *Q, *m, *v;      // [H][NU][N] in/out
+  float lo[kEnvMaxControls], hi[kEnvMaxControls];
+  float lr, gradmax_clip;
+  double beta1, beta2, eps;
+  long long adam_step0;
+  int adam_form;         // as RpgdGradArgs
+  EnvParams env;
+  float* J;              // [N] cost of the updated population
+  float* log_traj;       // [N][H+1][NS] or null
+  float* log_Q;          // [N][H][NU] or null
+  int n_host_adam;
+  float bc1_h[8], bc2_h[8], alpha_h[8];
+};
+struct EnvRpgdSelectArgs {
+  int N, H, k, period, n_ind;
+  int shift_previous, resample, tail_resample;  // as RpgdSelectArgs
+  const float* J;
+  const float *Q, *m, *v;  // [H][NU][N] current
+  const float* ages;
+  float *Qn, *mn, *vn;     // [H][NU][N] next
+  float* agesn;
+  NoiseSrc noise;          // resample: per_rollout = n_ind * NU (C order over [n_ind, NU]); tail redraw: per_rollout = NU
+  int dist;                // 0 normal, 1 uniform
+  float s_mean, s_std;
+  float s_min[kEnvMaxControls], s_max[kEnvMaxControls], lo[kEnvMaxControls], hi[kEnvMaxControls];
+  float* u_nom_out;        // [H][NU] Q[best] before the shift
+  float* u_prev;           // [NU]
+  float* u_out;            // [NU] or null
+  int freeze_prev;
+  int32_t* best_idx_out;   // [k]
+};
+struct EnvGradCemSampleArgs {
+  int H, ld, col0, cnt;
+  NoiseSrc noise;          // per_rollout = H * NU, draw index = column
+  const float *mu, *sd;    // [H][NU]
+  float lo[kEnvMaxControls], hi[kEnvMaxControls];
+  float* dst;              // [H][NU][ld]
+};
+struct EnvGradCemRefitArgs {
+  int N, H, k;
+  const float* J;
+  const float* Q;          // [H][NU][N]
+  float* Q_carry;          // [H][NU][N] or null
+  float *mu, *sd;          // [H][NU]
+  int last, u_from_mean;
+  float sd_min, sd_init;
+  float lo[kEnvMaxControls], hi[kEnvMaxControls];
+  float* u_prev;
+  float* u_out;
+  int freeze_prev;
+  int32_t* elite_idx_out;
+};
+
 constexpr int TOPK_THREADS = 1024;  // keys per top-k block
 
 }  // namespace ctk

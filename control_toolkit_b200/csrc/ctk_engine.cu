@@ -324,10 +324,9 @@ static int check_config(const ctk_config* cfg, const ctk_ode_params* ode, const 
   REQ(cfg->num_states == env_ns && cfg->num_control_inputs == env_nu,
       "num_states / num_control_inputs do not match the registered environment (CartPole: 6 / 1, Dubins car: 3 / 2)");
   if (cfg->environment != CTK_ENV_CARTPOLE)
-    REQ((cfg->optimizer == CTK_OPT_MPPI || cfg->optimizer == CTK_OPT_CEM) && cfg->predictor == CTK_PRED_ODE &&
-            cfg->num_rollouts == cfg->num_rollouts_global && cfg->num_clients <= 1 && !cfg->cem_uniform_actions,
-        "environments other than the CartPole: MPPI and CEM with the environment's ODE, unsharded, one client (RPGD's adjoint and the "
-        "network predictors are CartPole functors)");
+    REQ(cfg->predictor == CTK_PRED_ODE && cfg->num_rollouts == cfg->num_rollouts_global && cfg->num_clients <= 1 && !cfg->cem_uniform_actions,
+        "environments other than the CartPole: MPPI, CEM and the gradient optimizers with the environment's ODE, unsharded, one client "
+        "(the network predictors are CartPole functors)");
   REQ(cfg->num_rollouts >= 1 && cfg->mpc_horizon >= 1, "num_rollouts and mpc_horizon must be >= 1");
   REQ(cfg->num_rollouts_global >= cfg->num_rollouts && cfg->rollout_offset >= 0 &&
           cfg->rollout_offset + cfg->num_rollouts <= cfg->num_rollouts_global, "bad shard geometry");
@@ -343,7 +342,7 @@ static int check_config(const ctk_config* cfg, const ctk_ode_params* ode, const 
       "multi-client handles are implemented for MPPI with the ODE predictor, logging off, unsharded");
   const int N = cfg->num_rollouts, H = cfg->mpc_horizon, period = cfg->period_interpolation_inducing_points;
   if (cfg->optimizer != CTK_OPT_CEM && period < 1) return fail(CTK_EINVAL, "period_interpolation_inducing_points must be >= 1");
-  if (cfg->environment != CTK_ENV_CARTPOLE) {
+  if (cfg->environment != CTK_ENV_CARTPOLE && cfg->optimizer != CTK_OPT_RPGD) {
     if (cfg->optimizer == CTK_OPT_MPPI && (inducing_points(H, period) * env_nu > 32 || H * env_nu > 1024))
       return fail(CTK_EINVAL, "environment MPPI: n_ind * nu <= 32 and H * nu <= 1024");
     if (cfg->optimizer == CTK_OPT_CEM &&
@@ -360,6 +359,13 @@ static int check_config(const ctk_config* cfg, const ctk_ode_params* ode, const 
     if (cfg->rpgd_gradient_mode >= 2 && !(cfg->rpgd_gradient_mode <= 3 && cfg->cem_best_k >= 1 && cfg->cem_best_k <= N && cfg->cem_outer_it >= 1 &&
                                           period == 1 && elite_log_rows_max(*cfg) >= 1))
       return fail(CTK_EINVAL, "gradient-assisted CEM needs 1 <= cem_best_k <= num_rollouts, cem_outer_it >= 1 and inducing-point period 1");
+    // environments: the gradient kernel keeps states, q, g, m and v of every horizon step in shared memory (ctk_kernels_env_rpgd.cuh)
+    if (cfg->environment != CTK_ENV_CARTPOLE && env_rpgd_smem_bytes(cfg->environment, H) > kEnvRpgdSmemMax) {
+      int max_h = 1;
+      while (env_rpgd_smem_bytes(cfg->environment, max_h + 1) <= kEnvRpgdSmemMax) ++max_h;
+      return fail(CTK_EINVAL, "environment gradient optimizers: mpc_horizon too large for the shared-memory tape of H * (ns + 4 nu) floats "
+                              "per trajectory (max " + std::to_string(max_h) + ")");
+    }
   }
   return CTK_OK;
 }
@@ -488,11 +494,11 @@ extern "C" int ctk_create(const ctk_config* cfg, const ctk_ode_params* ode, cons
     A(h->d_cem_dist.alloc((size_t)2 * 512), "cem_dist");
   } else if (cfg->optimizer == CTK_OPT_RPGD) {
     for (int i = 0; i < 2; ++i) {
-      A(h->d_Q[i].alloc((size_t)N * H), "Q"); A(h->d_m[i].alloc((size_t)N * H), "m");
-      A(h->d_v[i].alloc((size_t)N * H), "v"); A(h->d_ages[i].alloc((size_t)N), "ages");
+      A(h->d_Q[i].alloc((size_t)N * H * nu), "Q"); A(h->d_m[i].alloc((size_t)N * H * nu), "m");
+      A(h->d_v[i].alloc((size_t)N * H * nu), "v"); A(h->d_ages[i].alloc((size_t)N), "ages");
     }
-    A(h->d_unom_log.alloc((size_t)H), "unom_log"); A(h->d_ages_log.alloc((size_t)N), "ages_log");
-    A(h->d_Q_log.alloc((size_t)N * H), "Q_log");
+    A(h->d_unom_log.alloc((size_t)H * nu), "unom_log"); A(h->d_ages_log.alloc((size_t)N), "ages_log");
+    A(h->d_Q_log.alloc((size_t)N * H * nu), "Q_log");
     A(h->d_best_idx.alloc((size_t)N), "best_idx");
   }
   if (rc == CTK_OK) A(upload_consts(h), "upload_consts");
@@ -670,6 +676,24 @@ static RpgdSelectArgs rpgd_sample_args(ctk_handle* h, NoiseSrc ns) {
   return a;
 }
 
+// The same for an environment: per-input limits; uniform draws over each input's own [low, high] when the whole control space is
+// sampled (optimizer_rpgd.py:199-205) and always for gradient-tf (optimizer_gradient_tf.py:171-177)
+static EnvRpgdSelectArgs env_rpgd_sample_args(ctk_handle* h, NoiseSrc ns) {
+  const ctk_config& c = h->cfg;
+  EnvRpgdSelectArgs a{};
+  a.N = h->N; a.H = h->H; a.k = c.rpgd_keep_k; a.period = h->period; a.n_ind = h->n_ind;
+  a.shift_previous = c.rpgd_shift_previous;
+  a.noise = ns; a.dist = c.rpgd_distribution;
+  a.s_mean = c.rpgd_sample_mean; a.s_std = c.rpgd_sample_stdev;
+  const bool whole = c.rpgd_sample_whole_space != 0 || c.rpgd_gradient_mode == 1;
+  for (int i = 0; i < kEnvMaxControls; ++i) {
+    a.lo[i] = h->lo_v[i]; a.hi[i] = h->hi_v[i];
+    a.s_min[i] = whole ? h->lo_v[i] : c.rpgd_sample_min;
+    a.s_max[i] = whole ? h->hi_v[i] : c.rpgd_sample_max;
+  }
+  return a;
+}
+
 // Mid-range warm start of `rows` control rows, per input (optimizer_mppi.py:227-231, optimizer_cem_tf.py:113-117), flat [rows][nu].
 // The CartPole's limits are the config's (ctk_set_control_limits).
 static std::vector<float> mid_range(const ctk_handle* h, size_t rows) {
@@ -695,18 +719,24 @@ extern "C" int ctk_reset(ctk_handle* h) {
   } else if (h->cfg.rpgd_gradient_mode >= 2) {
     // optimizer_cem_naive_grad_tf.py:116-119 / optimizer_cem_grad_bharadhwaj_tf.py:180-184: only the distribution (and count) is
     // reset; the Keras Adam slots of the bharadhwaj variant survive optimizer_reset()
-    CU(cudaMemcpyAsync(h->d_mu, mid.data(), sizeof(float) * h->H, cudaMemcpyHostToDevice, h->stream));
-    CU(cudaMemcpyAsync(h->d_sd, sd.data(), sizeof(float) * h->H, cudaMemcpyHostToDevice, h->stream));
+    CU(cudaMemcpyAsync(h->d_mu, mid.data(), sizeof(float) * h->H * h->nu, cudaMemcpyHostToDevice, h->stream));
+    CU(cudaMemcpyAsync(h->d_sd, sd.data(), sizeof(float) * h->H * h->nu, cudaMemcpyHostToDevice, h->stream));
     CU(cudaStreamSynchronize(h->stream));
   } else {
     NoiseSrc ns{};
-    int rcn = make_noise(h, STREAM_RPGD_INIT, h->n_ind, h->cfg.rpgd_distribution == CTK_DIST_UNIFORM, (size_t)h->N, &ns);
+    int rcn = make_noise(h, STREAM_RPGD_INIT, h->n_ind * h->nu, h->cfg.rpgd_distribution == CTK_DIST_UNIFORM, (size_t)h->N, &ns);
     if (rcn != CTK_OK) return rcn;
-    RpgdSelectArgs a = rpgd_sample_args(h, ns);
     h->cur = 0;
-    a.Qn = h->d_Q[0]; a.mn = h->d_m[0]; a.vn = h->d_v[0]; a.agesn = h->d_ages[0];
     h->launches++;
-    CU(launch_rpgd_init(a, h->stream));
+    if (h->env != 0) {
+      EnvRpgdSelectArgs a = env_rpgd_sample_args(h, ns);
+      a.Qn = h->d_Q[0]; a.mn = h->d_m[0]; a.vn = h->d_v[0]; a.agesn = h->d_ages[0];
+      CU(launch_env_rpgd_init(h->env, a, h->stream));
+    } else {
+      RpgdSelectArgs a = rpgd_sample_args(h, ns);
+      a.Qn = h->d_Q[0]; a.mn = h->d_m[0]; a.vn = h->d_v[0]; a.agesn = h->d_ages[0];
+      CU(launch_rpgd_init(a, h->stream));
+    }
     h->adam_step = 0;
   }
   CU(cudaStreamSynchronize(h->stream));
@@ -740,11 +770,13 @@ static S0e make_s0e(const ctk_handle* h, const float* s_dev, const float* s_host
   return s;
 }
 
+static int env_rpgd_tick(ctk_handle* h, const S0e& s0, float* u_out_dev);
 static int env_tick(ctk_handle* h, const S0e& s0, float* u_out_dev) {
   const ctk_config& c = h->cfg;
   if (!h->env_p_set) return fail(CTK_ESTATE, "environment parameters not set (ctk_set_env_params)");
   const int nu = h->nu;
   h->tick++;
+  if (c.optimizer == CTK_OPT_RPGD) return env_rpgd_tick(h, s0, u_out_dev);
   if (c.optimizer == CTK_OPT_MPPI) {
     EnvMppiArgs a{};
     int rcn = make_noise(h, STREAM_MPPI, h->n_ind * nu, 0, (size_t)h->NG, &a.noise);
@@ -1179,7 +1211,8 @@ static int cem_finish(ctk_handle* h, const uint64_t* cand, int cnt, float* u_out
 }
 
 // Adam bias corrections of the first gradient steps of a launch (RpgdGradArgs::bc1_h ...), float64 on the host, rounded once
-static void fill_host_adam(RpgdGradArgs& a) {
+template <class GradArgs>
+static void fill_host_adam(GradArgs& a) {
   a.n_host_adam = a.iters < 8 ? a.iters : 8;
   for (int i = 0; i < a.n_host_adam; ++i) {
     const double step = (double)(a.adam_step0 + i + 1);
@@ -1338,6 +1371,122 @@ static int rpgd_tick(ctk_handle* h, const float* s_dev, float* u_out_dev) {
   rc = rpgd_local(h, s_dev, &sel);
   if (rc != CTK_OK) return rc;
   rpgd_select_commit(h);
+  return CTK_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// gradient optimizers on environments (ctk_kernels_env_rpgd.cuh): the same tick structure as the CartPole's, population [H][nu][N]
+// ---------------------------------------------------------------------------------------------------------------
+static EnvRpgdGradArgs env_rpgd_grad_args(ctk_handle* h, const S0e& s0, int iters, float* Q, float* m, float* v, int adam_form) {
+  const ctk_config& c = h->cfg;
+  EnvRpgdGradArgs a{};
+  a.N = h->N; a.H = h->H; a.iters = iters; a.s0 = s0; a.u_prev = h->d_u_prev;
+  a.Q = Q; a.m = m; a.v = v;
+  for (int i = 0; i < kEnvMaxControls; ++i) { a.lo[i] = h->lo_v[i]; a.hi[i] = h->hi_v[i]; }
+  a.lr = c.rpgd_learning_rate; a.gradmax_clip = c.rpgd_gradmax_clip;
+  a.beta1 = c.rpgd_beta_1; a.beta2 = c.rpgd_beta_2; a.eps = c.rpgd_epsilon; a.adam_step0 = h->adam_step; a.adam_form = adam_form;
+  a.env = h->env_p; a.J = h->d_J; a.log_traj = h->d_log_traj_soa; a.log_Q = h->d_log_Q_soa;
+  fill_host_adam(a);
+  return a;
+}
+static std::string env_grad_kernel_name(const ctk_handle* h, bool fused) {
+  return std::string("env_rpgd_grad_kernel<DubinsEnv,") + (h->cfg.logging ? "1" : "0") + ">" + (fused ? " [fused select]" : "");
+}
+
+// gradient-assisted CEM (gradcem_tick over nu columns)
+static int env_gradcem_tick(ctk_handle* h, const S0e& s0, float* u_out_dev) {
+  const ctk_config& c = h->cfg;
+  const bool carry = c.rpgd_gradient_mode == 3;
+  const int N = h->N, H = h->H, k = c.cem_best_k, nu = h->nu;
+  const int iters = carry ? cem_tick_iters(h) : c.cem_outer_it;
+  const int kc = carry ? k : 0;
+  auto sample = [&](int col0, int cnt, uint32_t sub) -> int {
+    if (cnt <= 0) return CTK_OK;
+    EnvGradCemSampleArgs a{};
+    int rcn = make_noise(h, STREAM_CEM | (sub << 8), H * nu, 0, (size_t)cnt, &a.noise);
+    if (rcn != CTK_OK) return rcn;
+    a.H = H; a.ld = N; a.col0 = col0; a.cnt = cnt; a.mu = h->d_mu; a.sd = h->d_sd;
+    for (int i = 0; i < kEnvMaxControls; ++i) { a.lo[i] = h->lo_v[i]; a.hi[i] = h->hi_v[i]; }
+    a.dst = h->d_Q[h->cur];
+    h->launches++;
+    CU(launch_env_gradcem_sample(h->env, a, h->stream));
+    return CTK_OK;
+  };
+  int rc = carry ? sample(0, k, 0) : CTK_OK;  // bharadhwaj :159 the first "elites" are plain samples
+  if (rc != CTK_OK) return rc;
+  h->elite_log_rows = 0;
+  const size_t smem = env_rpgd_smem_bytes(h->env, H);
+  for (int it = 0; it < iters; ++it) {
+    rc = sample(kc, N - kc, (uint32_t)it + 1);
+    if (rc != CTK_OK) return rc;
+    const EnvRpgdGradArgs a = env_rpgd_grad_args(h, s0, 1, h->d_Q[h->cur], h->d_m[0], h->d_v[0], carry ? 0 : 2);
+    h->launches++;
+    {
+      KernelTimer kt(h);
+      CU(launch_env_rpgd_grad(h->env, c.logging != 0, smem, h->stream, a, nullptr));
+    }
+    h->last_kernel = env_grad_kernel_name(h, false);
+    if (carry) h->adam_step += 1;
+    const bool last = it == iters - 1;
+    EnvGradCemRefitArgs r{};
+    r.N = N; r.H = H; r.k = k; r.J = h->d_J; r.Q = h->d_Q[h->cur]; r.Q_carry = carry ? h->d_Q[h->cur ^ 1].get() : nullptr;
+    r.mu = h->d_mu; r.sd = h->d_sd; r.last = last ? 1 : 0; r.u_from_mean = carry ? 0 : 1;
+    r.sd_min = c.cem_stdev_min; r.sd_init = c.cem_initial_action_stdev;
+    for (int i = 0; i < kEnvMaxControls; ++i) { r.lo[i] = h->lo_v[i]; r.hi[i] = h->hi_v[i]; }
+    r.u_prev = h->d_u_prev; r.u_out = u_out_dev; r.freeze_prev = c.freeze_previous_input;
+    r.elite_idx_out = (it < h->elite_log_cap) ? h->d_elite_idx + (size_t)it * k : nullptr;
+    h->launches++;
+    CU(launch_env_gradcem_refit(h->env, r, h->stream));
+    if (r.elite_idx_out) h->elite_log_rows++;
+    if (carry) h->cur ^= 1;
+  }
+  h->count++;
+  return CTK_OK;
+}
+
+// RPGD / gradient-tf: one launch (gradient steps + fused K8) for a population of one block with logging off, else two
+static int env_rpgd_tick(ctk_handle* h, const S0e& s0, float* u_out_dev) {
+  const ctk_config& c = h->cfg;
+  if (c.rpgd_gradient_mode >= 2) return env_gradcem_tick(h, s0, u_out_dev);
+  const int N = h->N, nu = h->nu;
+  const int grad_mode = c.rpgd_gradient_mode == 1 ? 1 : 0;
+  const int resample = (!grad_mode && h->count % c.rpgd_resamp_per == 0) ? 1 : 0;  // optimizer_rpgd.py:449
+  NoiseSrc ns{};
+  if (grad_mode) {  // [N, 1, nu] uniform draws for the vacated last step (optimizer_gradient_tf.py:142-147)
+    int rcn = make_noise(h, STREAM_RPGD_RESAMPLE, nu, 1, (size_t)N, &ns);
+    if (rcn != CTK_OK) return rcn;
+  } else if (resample && N - c.rpgd_keep_k > 0) {
+    int rcn = make_noise(h, STREAM_RPGD_RESAMPLE, h->n_ind * nu, c.rpgd_distribution == CTK_DIST_UNIFORM, (size_t)(N - c.rpgd_keep_k), &ns);
+    if (rcn != CTK_OK) return rcn;
+  }
+  EnvRpgdSelectArgs sel = env_rpgd_sample_args(h, ns);
+  sel.resample = resample;
+  sel.tail_resample = grad_mode;
+  if (grad_mode) sel.dist = CTK_DIST_UNIFORM;
+  const int nx = h->cur ^ 1;
+  sel.J = h->d_J; sel.Q = h->d_Q[h->cur]; sel.m = h->d_m[h->cur]; sel.v = h->d_v[h->cur]; sel.ages = h->d_ages[h->cur];
+  sel.Qn = h->d_Q[nx]; sel.mn = h->d_m[nx]; sel.vn = h->d_v[nx]; sel.agesn = h->d_ages[nx];
+  sel.u_nom_out = h->d_unom_log; sel.u_prev = h->d_u_prev; sel.u_out = u_out_dev; sel.freeze_prev = c.freeze_previous_input;
+  sel.best_idx_out = h->d_best_idx;
+
+  const int iters = (h->count == 0) ? c.rpgd_first_iter_count : c.rpgd_outer_its;  // optimizer_rpgd.py:397-400
+  const EnvRpgdGradArgs a = env_rpgd_grad_args(h, s0, iters, h->d_Q[h->cur], h->d_m[h->cur], h->d_v[h->cur], c.rpgd_adam_form);
+  const bool fuse = N <= kEnvRpgdBlock && !c.logging;
+  h->launches++;
+  {
+    KernelTimer kt(h);
+    CU(launch_env_rpgd_grad(h->env, c.logging != 0, env_rpgd_smem_bytes(h->env, h->H), h->stream, a, fuse ? &sel : nullptr));
+  }
+  h->last_kernel = env_grad_kernel_name(h, fuse);
+  h->adam_step += iters;
+  if (!fuse) {
+    // trajectory_ages_logged: the ages BEFORE the warm-start update (:413-415); Q_logged is written by the gradient kernel
+    if (c.logging) CU(cudaMemcpyAsync(h->d_ages_log, h->d_ages[h->cur], sizeof(float) * N, cudaMemcpyDeviceToDevice, h->stream));
+    h->launches++;
+    CU(launch_env_rpgd_select(h->env, sel, h->stream));
+  }
+  h->cur = nx;
+  h->count++;
   return CTK_OK;
 }
 
@@ -1696,10 +1845,10 @@ static int state_ptr(ctk_handle* h, int which, float** p, size_t* n, bool* tmajo
     case CTK_STATE_U_NOM: *p = (h->cfg.optimizer == CTK_OPT_RPGD) ? h->d_unom_log : h->d_u_nom; *n = H * (size_t)h->nclients * h->nu; break;  // RPGD: Q[best] before the shift (:426)
     case CTK_STATE_CEM_MU: *p = h->d_mu; *n = H * h->nu; break;
     case CTK_STATE_CEM_STD: *p = h->d_sd; *n = H * h->nu; break;
-    case CTK_STATE_RPGD_Q: *p = h->d_Q[h->cur]; *n = N * H; *tmajor = true; break;
+    case CTK_STATE_RPGD_Q: *p = h->d_Q[h->cur]; *n = N * H * h->nu; *tmajor = true; break;
     // gradient-assisted CEM keeps its Adam moments attached to the population ROWS (never permuted): buffer 0
-    case CTK_STATE_RPGD_M: *p = h->d_m[h->cfg.rpgd_gradient_mode >= 2 ? 0 : h->cur]; *n = N * H; *tmajor = true; break;
-    case CTK_STATE_RPGD_V: *p = h->d_v[h->cfg.rpgd_gradient_mode >= 2 ? 0 : h->cur]; *n = N * H; *tmajor = true; break;
+    case CTK_STATE_RPGD_M: *p = h->d_m[h->cfg.rpgd_gradient_mode >= 2 ? 0 : h->cur]; *n = N * H * h->nu; *tmajor = true; break;
+    case CTK_STATE_RPGD_V: *p = h->d_v[h->cfg.rpgd_gradient_mode >= 2 ? 0 : h->cur]; *n = N * H * h->nu; *tmajor = true; break;
     case CTK_STATE_RPGD_AGES: *p = h->d_ages[h->cur]; *n = N; break;
     case CTK_STATE_U_PREV: *p = h->d_u_prev; *n = (size_t)(h->nclients > h->nu ? h->nclients : h->nu); break;
     case CTK_STATE_RNN_H: *p = h->d_rnn_h; *n = 2 * (size_t)h->mlp.hidden; break;
@@ -1719,7 +1868,7 @@ extern "C" int ctk_get_state(ctk_handle* h, int which, float* dst, size_t n) {
   if (tm) {
     Owned<float> tmp;
     CU(tmp.alloc(cnt, false));
-    rc = transpose_dev(h, p, tmp, h->H, h->N);  // [H][N] -> [N][H]
+    rc = transpose_dev(h, p, tmp, h->H * h->nu, h->N);  // [H][nu][N] -> [N][H][nu]
     if (rc != CTK_OK) return rc;
     CU(cudaMemcpyAsync(dst, tmp, cnt * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
     CU(cudaStreamSynchronize(h->stream));
@@ -1741,7 +1890,7 @@ extern "C" int ctk_set_state(ctk_handle* h, int which, const float* src, size_t 
     Owned<float> tmp;
     CU(tmp.alloc(cnt, false));
     CU(cudaMemcpyAsync(tmp, src, cnt * sizeof(float), cudaMemcpyHostToDevice, h->stream));
-    rc = transpose_dev(h, tmp, p, h->N, h->H);
+    rc = transpose_dev(h, tmp, p, h->N, h->H * h->nu);
     CU(cudaStreamSynchronize(h->stream));
     return rc;
   }

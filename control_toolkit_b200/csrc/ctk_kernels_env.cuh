@@ -7,12 +7,13 @@
 // [n_ind or H, nu]), the same top-k (K4) for CEM.  Multi-launch and unsharded: the latency work of the CartPole ticks is not repeated.
 #pragma once
 #include "ctk_device.cuh"
+#include "ctk_env_adjoint.h"
 #include "ctk_topk.cuh"
 
 namespace ctk {
 
-// ---- Dubins car: [x, y, yaw], [throttle, steer]; oracle/spec.py dubins_step / DubinsCost -------------------------------------
-struct DubinsEnv {
+// ---- Dubins car: [x, y, yaw], [throttle, steer]; oracle/spec.py dubins_step / DubinsCost; adjoint: ctk_env_adjoint.h -----------
+struct DubinsEnv : DubinsAdjoint {
   static constexpr int NS = 3, NU = 2;
   // p: 0 h  1 v_max  2 omega_max  3 dd_weight  4 obstacle_weight  5 cc_weight * R  6 ccrc_weight  7 terminal_weight
   //    8 target_x  9 target_y  10 obstacle_x  11 obstacle_y  12 obstacle_r^2  13 MAX_COST

@@ -68,6 +68,14 @@ cudaError_t launch_env_mppi(int env, bool log, const EnvMppiArgs& a, cudaStream_
 cudaError_t launch_env_cem_rollout(int env, bool log, const EnvCemArgs& a, cudaStream_t st);
 cudaError_t launch_env_cem_refit(const EnvCemRefitArgs& a, cudaStream_t st);
 void env_dims(int env, int* ns, int* nu);
+// gradient optimizers on environments (ctk_kernels_env_rpgd.cuh): grad kernel (+ fused K8 when fused_select != null: N <= 32),
+// K8, initial population, gradient-assisted CEM sample / refit; smem: the grad kernel's shared-memory tape at horizon H
+cudaError_t launch_env_rpgd_grad(int env, bool log, size_t smem, cudaStream_t st, const EnvRpgdGradArgs& a, const EnvRpgdSelectArgs* fused_select);
+size_t env_rpgd_smem_bytes(int env, int H);
+cudaError_t launch_env_rpgd_select(int env, const EnvRpgdSelectArgs& a, cudaStream_t st);
+cudaError_t launch_env_rpgd_init(int env, const EnvRpgdSelectArgs& a, cudaStream_t st);
+cudaError_t launch_env_gradcem_sample(int env, const EnvGradCemSampleArgs& a, cudaStream_t st);
+cudaError_t launch_env_gradcem_refit(int env, const EnvGradCemRefitArgs& a, cudaStream_t st);
 // recurrent predictor (ctk_gru.cu)
 cudaError_t launch_mppi_rollout_gru(int kind, bool log, int nblocks, int block, size_t smem, cudaStream_t st, const MppiArgs& a);
 cudaError_t launch_cem_rollout_gru(int kind, bool log, int nblocks, size_t smem, cudaStream_t st, const CemArgs& a);

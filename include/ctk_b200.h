@@ -50,14 +50,15 @@ enum { CTK_MLP_SIMT = 0, CTK_MLP_TCGEN05 = 1, CTK_MLP_TCGEN05_BF16 = 2, CTK_MLP_
 
 /* which = state arrays (get/set).  Layouts are the reference's: [1,H,nu] or [N,H,nu] row-major.                 */
 enum {
-  CTK_STATE_U_NOM = 0,      /* MPPI u_nom [H] ([num_clients][H] for a multi-client handle) (optimizer_mppi.py:227-231) */
+  CTK_STATE_U_NOM = 0,      /* MPPI u_nom [H,nu] ([num_clients][H] for a multi-client handle) (optimizer_mppi.py:227-231); RPGD:
+                               Q[best] before the shift [H,nu]                                                      */
   CTK_STATE_CEM_MU = 1,     /* CEM dist_mue [H]          (optimizer_cem_tf.py:114)                                */
   CTK_STATE_CEM_STD = 2,    /* CEM stdev [H]             (optimizer_cem_tf.py:115)                                */
-  CTK_STATE_RPGD_Q = 3,     /* RPGD Q_tf [N,H]           (optimizer_rpgd.py:540-544)                              */
-  CTK_STATE_RPGD_M = 4,     /* Adam m [N,H]              (optimizer_rpgd.py:84-131)                               */
-  CTK_STATE_RPGD_V = 5,     /* Adam v [N,H]                                                                       */
+  CTK_STATE_RPGD_Q = 3,     /* RPGD Q_tf [N,H,nu]        (optimizer_rpgd.py:540-544)                              */
+  CTK_STATE_RPGD_M = 4,     /* Adam m [N,H,nu]           (optimizer_rpgd.py:84-131)                               */
+  CTK_STATE_RPGD_V = 5,     /* Adam v [N,H,nu]                                                                    */
   CTK_STATE_RPGD_AGES = 6,  /* trajectory_ages [N]       (optimizer_rpgd.py:548)                                  */
-  CTK_STATE_U_PREV = 7,     /* self.u, the previous_input of the cost [1] (Optimizers/__init__.py:35)             */
+  CTK_STATE_U_PREV = 7,     /* self.u, the previous_input of the cost [nu] (Optimizers/__init__.py:35)            */
   CTK_STATE_RNN_H = 8       /* saved hidden state of the recurrent predictor [2 * hidden] (layer 1 | layer 2): what every rollout
                                starts from and predictor.update advances (optimizer_mppi.py:195-197)                  */
 };
@@ -152,7 +153,10 @@ typedef struct ctk_config {
                                      MPPI clients -- own warm-start sequence, previous input, costs and Philox tick counter each -- whose
                                      ticks ctk_step_batch runs in ONE launch (SURVEY 8f.4; MPPI + ODE predictor, logging off, unsharded) */
   int32_t environment;            /* CTK_ENV_*                                                                    */
-  int32_t reserved[3];
+  int32_t rpgd_sample_whole_space; /* environments other than the CartPole: 1 = uniform RPGD draws over each input's own [low, high]
+                                     (ctk_set_control_limits; reference sample_whole_control_space), 0 = over [rpgd_sample_min,
+                                     rpgd_sample_max] for every input.  The CartPole reads rpgd_sample_min / max                  */
+  int32_t reserved[2];
 } ctk_config;
 
 typedef struct ctk_handle ctk_handle;

@@ -105,13 +105,15 @@ class optimizer_cem_tf(template_optimizer):
     def last_elite_indices(self, iterations: int) -> np.ndarray:
         return self._get_log(L.LOG_ELITE_IDX, (iterations, self.cem_best_k), np.int32)
 
+    # dist_mue / stdev [1, H, nu]; u: a float for nu == 1, (nu,) otherwise (the shape step() returns)
     def get_state(self) -> dict:
-        return {"dist_mue": self.dist_mue, "stdev": self.stdev, "count": self.count,
-                "u": float(self._get_state(L.STATE_U_PREV, (1,))[0])}
+        nu = int(self.num_control_inputs)
+        u = self._get_state(L.STATE_U_PREV, (nu,))
+        return {"dist_mue": self.dist_mue, "stdev": self.stdev, "count": self.count, "u": float(u[0]) if nu == 1 else u}
 
     def set_state(self, state: dict) -> None:
         self._set_state(L.STATE_CEM_MU, state["dist_mue"])
         self._set_state(L.STATE_CEM_STD, state["stdev"])
-        self._set_state(L.STATE_U_PREV, [state["u"]])
+        self._set_state(L.STATE_U_PREV, np.reshape(state["u"], (int(self.num_control_inputs),)))
         self.count = int(state["count"])
         self._set_counter(L.COUNTER_COUNT, self.count)

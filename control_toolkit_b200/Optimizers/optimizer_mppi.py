@@ -126,10 +126,14 @@ class optimizer_mppi(template_optimizer):
         self.u_nom = self._get_state(L.STATE_U_NOM, (self.num_clients, self.mpc_horizon, self.num_control_inputs))
 
     # state access (part of the parity contract: "optimizer state within 1e-5")
+    # u_nom [1, H, nu]; u: a float for nu == 1, (nu,) otherwise (the shape step() returns)
     def get_state(self) -> dict:
-        return {"u_nom": self._get_state(L.STATE_U_NOM, (1, self.mpc_horizon, 1)), "u": float(self._get_state(L.STATE_U_PREV, (1,))[0])}
+        nu = int(self.num_control_inputs)
+        u = self._get_state(L.STATE_U_PREV, (nu,))
+        return {"u_nom": self._get_state(L.STATE_U_NOM, (1, self.mpc_horizon, nu)), "u": float(u[0]) if nu == 1 else u}
 
     def set_state(self, state: dict) -> None:
+        nu = int(self.num_control_inputs)
         self._set_state(L.STATE_U_NOM, state["u_nom"])
-        self._set_state(L.STATE_U_PREV, [state["u"]])
-        self.u_nom = np.asarray(state["u_nom"], np.float32).reshape(1, self.mpc_horizon, 1)
+        self._set_state(L.STATE_U_PREV, np.reshape(state["u"], (nu,)))
+        self.u_nom = np.asarray(state["u_nom"], np.float32).reshape(1, self.mpc_horizon, nu)

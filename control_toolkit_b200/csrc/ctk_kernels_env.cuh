@@ -49,6 +49,20 @@ __device__ __forceinline__ void env_log_state(float* log_traj, int n, int t, int
   for (int i = 0; i < Env::NS; ++i) log_traj[((size_t)n * (H + 1) + t) * Env::NS + i] = s[i];
 }
 
+// Compensated (Kahan) sum.  The MPPI correction adds 3 H NU terms into one total that enters the softmin unscaled: at H NU = 1024 a
+// plain fp32 running sum is ~4e-4 off (totals ~60), which moves the weights exp(-(S - rho) / LBD) at LBD = 1 and put u_nom 4.6e-5 from
+// float64 where the reference's fp32 evaluation is 1e-6 away (tests/test_gpu_env_ticks.py, H = 512).  The _rn intrinsics keep the
+// compiler from contracting or reassociating the compensation.
+struct KahanSum {
+  float s = 0.0f, c = 0.0f;
+  __device__ __forceinline__ void add(float x) {
+    const float y = __fsub_rn(x, c);
+    const float t = __fadd_rn(s, y);
+    c = __fsub_rn(__fsub_rn(t, s), y);
+    s = t;
+  }
+};
+
 // ---- MPPI: sample -> rollout -> cost (reference optimizer_mppi.py:170-193 up to the total cost S) ----------------------------
 template <class Env, bool LOG>
 __global__ void __launch_bounds__(128) env_mppi_rollout_kernel(const EnvMppiArgs a) {
@@ -61,7 +75,8 @@ __global__ void __launch_bounds__(128) env_mppi_rollout_kernel(const EnvMppiArgs
   for (int i = 0; i < NS; ++i) s[i] = a.s0.p != nullptr ? a.s0.p[i] : a.s0.v[i];
 #pragma unroll
   for (int c = 0; c < NU; ++c) up[c] = a.u_prev[c];
-  float jsum = 0.0f, corr = 0.0f;
+  float jsum = 0.0f;
+  KahanSum corr;
   float y0[NU], y1[NU];
   for (int t = 0; t < a.H; ++t) {
     const int seg = t / a.period, j = t - seg * a.period;
@@ -81,9 +96,9 @@ __global__ void __launch_bounds__(128) env_mppi_rollout_kernel(const EnvMppiArgs
       const float un = a.u_nom[(size_t)min(t + 1, a.H - 1) * NU + c];                          // :184 shift on read
       u[c] = fminf(fmaxf(__fadd_rn(un, du), a.lo[c]), a.hi[c]);                                // :186-187
       // :154-155  cc_weight * (0.5 (1 - 1/NU) R du^2 + R u du + 0.5 R u^2)
-      corr = fmaf(du * du, a.k_du2, corr);
-      corr = fmaf(u[c] * du, a.k_udu, corr);
-      corr = fmaf(u[c] * u[c], a.k_uu, corr);
+      corr.add(__fmul_rn(__fmul_rn(du, du), a.k_du2));
+      corr.add(__fmul_rn(__fmul_rn(u[c], du), a.k_udu));
+      corr.add(__fmul_rn(__fmul_rn(u[c], u[c]), a.k_uu));
       if (LOG) a.log_Q[((size_t)n * a.H + t) * NU + c] = u[c];
     }
     if (LOG) env_log_state<Env>(a.log_traj, n, t, a.H, s);
@@ -94,7 +109,7 @@ __global__ void __launch_bounds__(128) env_mppi_rollout_kernel(const EnvMppiArgs
   }
   if (LOG) env_log_state<Env>(a.log_traj, n, a.H, a.H, s);
   // Cost_Functions/__init__.py:90-92 (mean over H+1 incl. the terminal cost) + the MPPI correction (optimizer_mppi.py:160)
-  a.J[n] = __fadd_rn((jsum + Env::terminal_cost(s, a.env)) / (float)(a.H + 1), corr);
+  a.J[n] = __fadd_rn((jsum + Env::terminal_cost(s, a.env)) / (float)(a.H + 1), corr.s);
 }
 
 // ---- MPPI: softmin weights, weighted perturbation average on the inducing points, u_nom update (optimizer_mppi.py:163-168,190-191).

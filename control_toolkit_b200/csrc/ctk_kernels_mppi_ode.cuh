@@ -5,7 +5,7 @@
 //
 // What is different from the generic kernel (all measured with ncu, profiles/):
 //  * scaled state variables (OdeHot): T = angle/sqrt(2), W = beta*angleD, V = (cF/g)*positionD remove 6 multiplies per
-//    step; every constant multiplier is a kernel parameter that ptxas keeps in a uniform register, so all but four FMAs
+//    step; every constant multiplier is a kernel parameter that ptxas keeps in a uniform register, so all but five FMAs
 //    per step read at most two vector registers (the sm_100 register file feeds 3-source FFMAs at ~2/3 rate);
 //  * the control terms of the stage cost and of the MPPI correction collapse to u*(kA u + kB u_prev + kC du); the
 //    du^2 term of the correction has a closed form per inducing-point segment and leaves the step loop entirely;
@@ -13,6 +13,9 @@
 //    du = fma(dy, w_j, y0) is one instruction;
 //  * ILP rollouts per thread are advanced in lock step (independent dependency chains): the last warps of an SM
 //    sub-partition still fill the FMA pipe, which removes the tail the hi-wid-first warp arbiter otherwise produces;
+//    with ILP = 2 they are ONE roll of f2 lanes (ctk_ode_scaled.cuh): every add, multiply and fma of the step is one packed
+//    FADD2 / FMUL2 / FFMA2 for both rollouts, bit-identical per lane to the float build.  The kernel is issue-bound, and a pair
+//    takes one issue slot where two scalar instructions took two (tests/test_k1_packed_sass.py, DESIGN.md 5.1);
 //  * the state-independent part of the prologue (the Philox draws of the first rollout group) runs BEFORE griddepcontrol.wait: in a
 //    back-to-back chain of ticks (programmatic dependent launch) it overlaps the previous tick's finish / exchange / launch gap;
 //    the global reads of the prologue (s0, u_prev, u_nom) follow the wait and were prefetched into L2 before the draws;
@@ -22,19 +25,33 @@
 //    on three sub-partitions, round 1) the ideal 26.4 units per sub-partition at C5 became 28; with 28 warps and the units dealt out
 //    one by one it is 27.
 #pragma once
+#include <type_traits>
+
 #include "ctk_device.cuh"
 #include "ctk_kernels_mppi.cuh"
 #include "ctk_ode_scaled.cuh"
 
 namespace ctk {
 
-struct Roll : ScaledState {  // one rollout's registers
-  float ul, acc, y0, dy, y1;
+// The registers of a thread's rollouts: L = float for one rollout per thread, f2 for two advanced in lock step (ctk_ode_scaled.cuh).
+template <class L>
+struct Roll : ScaledStateT<L> {
+  L ul, acc, y0, dy, y1;
 #ifdef CTK_K1_DSUM
-  double dtot;
+  double dtot[sizeof(L) / sizeof(float)];
 #endif
-  float tot, comp;  // running total of the per-segment cost sums (+ its compensation term under CTK_K1_KAHAN; see fold_segment)
+  L tot, comp;  // running total of the per-segment cost sums (+ its compensation term under CTK_K1_KAHAN; see fold_segment)
 };
+template <int ILP>
+using Lanes = typename std::conditional<ILP == 2, f2, float>::type;
+
+// a thread's draw i of its ILP rollouts: lane q at p[q * T_], p = sh_z + i * ILP * T_ + tid
+template <class L>
+__device__ L ld_lanes(const float* p, int T_);
+template <>
+__device__ __forceinline__ float ld_lanes<float>(const float* p, int) { return p[0]; }
+template <>
+__device__ __forceinline__ f2 ld_lanes<f2>(const float* p, int T_) { return f2(p[0], p[T_]); }
 
 // The total cost S ~ 5e3 enters the softmin as exp(-(S - rho) / lambda) with lambda = 100: one ulp of S (4.9e-4) is 5e-6 relative
 // in the weight, and a 100-term sequential fp32 sum wanders by ~3 ulp rms -- more than the reference's torch.mean over [H + 1]
@@ -42,32 +59,37 @@ struct Roll : ScaledState {  // one rollout's registers
 // magnitude below S) and the segment sums enter the total through a compensated (Kahan) addition: 4 FADD per SEGMENT, ~0.5 ulp.
 // (-DCTK_K1_PLAIN_SUM adds the segment sums up plainly, ~0.9 ulp rms: the pinned C1 ticks then miss the 1e-5 bound -- measured,
 // tests/test_gpu_production_pinning.py c1 / c1_ilp2 -- so the compensation stays.)
-__device__ __forceinline__ void fold_segment(Roll& r) {
+template <class L>
+__device__ __forceinline__ void fold_segment(Roll<L>& r) {
 #if defined(CTK_K1_DSUM)
-  r.dtot += (double)r.acc;  // (experiment) second level in double: exact, one conversion + one DADD per segment
+  for (int q = 0; q < (int)(sizeof(L) / sizeof(float)); ++q)
+    r.dtot[q] += (double)lane_of(r.acc, q);  // (experiment) second level in double: exact, one conversion + one DADD per segment
 #elif !defined(CTK_K1_PLAIN_SUM)
-  const float y = r.acc - r.comp;
-  const float t = r.tot + y;
+  const L y = r.acc - r.comp;
+  const L t = r.tot + y;
   r.comp = (t - r.tot) - y;
   r.tot = t;
 #else
-  r.tot += r.acc;
+  r.tot = r.tot + r.acc;
 #endif
   r.acc = 0.0f;
 }
 
-// One rollout step.  wj = j/period (immediate when PERIOD is a template constant).
-template <int KIND, bool LOG>
-__device__ __forceinline__ void ode_mppi_step(const MppiOdeArgs& a, const OdeHot& k, Roll& r, float unom_t, float wj, bool first,
-                                              int t, int n, bool active) {
+// One step of a thread's rollouts (lane q: rollout n[q]).  wj = j/period (immediate when PERIOD is a template constant).
+template <int KIND, bool LOG, class L>
+__device__ __forceinline__ void ode_mppi_step(const MppiOdeArgs& a, const OdeHot& k, Roll<L>& r, float unom_t, float wj, bool first,
+                                              int t, const int* n, const bool* active) {
   // Interpolator.py:97-106 (two non-zero weights): du = y0 (1 - wj) + y1 wj = y0 + (y1 - y0) wj
-  const float du = first ? r.y0 : fmaf(r.dy, wj, r.y0);
-  const float u = fminf(fmaxf(unom_t + du, k.lo), k.hi);  // optimizer_mppi.py:186-187
-  if (LOG && active) {
-    float* p = a.log_traj_soa + (size_t)t * 6 * a.N + n;
-    p[0] = r.T * kSqrt2; p[a.N] = r.W * k.inv_beta; p[2 * (size_t)a.N] = r.c; p[3 * (size_t)a.N] = r.s;
-    p[4 * (size_t)a.N] = r.x; p[5 * (size_t)a.N] = r.V * k.inv_cFg;
-    a.log_Q_soa[(size_t)t * a.N + n] = u;
+  const L du = first ? r.y0 : fmaf(r.dy, wj, r.y0);
+  const L u = fminf(fmaxf(unom_t + du, k.lo), k.hi);  // optimizer_mppi.py:186-187
+#pragma unroll
+  for (int q = 0; q < (int)(sizeof(L) / sizeof(float)); ++q) {
+    if (LOG && active[q]) {
+      float* p = a.log_traj_soa + (size_t)t * 6 * a.N + n[q];
+      p[0] = lane_of(r.T, q) * kSqrt2; p[a.N] = lane_of(r.W, q) * k.inv_beta; p[2 * (size_t)a.N] = lane_of(r.c, q); p[3 * (size_t)a.N] = lane_of(r.s, q);
+      p[4 * (size_t)a.N] = lane_of(r.x, q); p[5 * (size_t)a.N] = lane_of(r.V, q) * k.inv_cFg;
+      a.log_Q_soa[(size_t)t * a.N + n[q]] = lane_of(u, q);
+    }
   }
   // stage cost / (H+1) (spec: DESIGN.md section 3; Cost_Functions/__init__.py:49-64) merged with the MPPI correction
   // (optimizer_mppi.py:154-155), then the Euler step in scaled variables (ctk_ode_scaled.cuh)
@@ -177,8 +199,11 @@ __device__ __forceinline__ void mppi_ode_body(const MppiOdeArgs& a) {
   float rho_t = INFINITY, a_t = 0.0f;  // per-thread online softmin (optimizer_mppi.py:163-168, exact combine later)
   float* sa = sh_acc + tid;
 
+  static_assert(ILP == 1 || ILP == 2, "one rollout per thread (float lanes) or two (f2 lanes)");
+  using L = Lanes<ILP>;
+  const float* sz = sh_z + tid;  // draw i of lane q: sz[(i * ILP + q) * T_]
   for (int base = boff; base - lane < r_end; base += stride) {  // (warp-uniform bound; no block barrier inside the loop)
-    Roll r[ILP];
+    Roll<L> r;
     int n[ILP];
     bool active[ILP];
     if (base != boff) gen_noise(base);  // the first group's draws were generated in the prologue
@@ -186,17 +211,16 @@ __device__ __forceinline__ void mppi_ode_body(const MppiOdeArgs& a) {
     for (int q = 0; q < ILP; ++q) {
       n[q] = base + q * 32;
       active[q] = n[q] < r_end;
-      const float* sz = sh_z + q * T_ + tid;
-      r[q].T = T0; r[q].W = W0; r[q].c = c0; r[q].s = sn0; r[q].x = x0; r[q].V = V0; r[q].omc = omc0;
-      r[q].ul = upv;
-      r[q].acc = (k.k_ccrc * upv) * upv;  // telescoped ccrc term of u_{-1}
-      r[q].tot = 0.0f; r[q].comp = 0.0f;
-#ifdef CTK_K1_DSUM
-      r[q].dtot = 0.0;
-#endif
-      r[q].y0 = 0.0f; r[q].dy = 0.0f;
-      r[q].y1 = sz[0] * k.stdev;  // y0 of segment 0   (:173-175 normal * stdev before interpolation)
     }
+    r.T = T0; r.W = W0; r.c = c0; r.s = sn0; r.x = x0; r.V = V0; r.omc = omc0;
+    r.ul = upv;
+    r.acc = (k.k_ccrc * upv) * upv;  // telescoped ccrc term of u_{-1}
+    r.tot = 0.0f; r.comp = 0.0f;
+#ifdef CTK_K1_DSUM
+    for (int q = 0; q < ILP; ++q) r.dtot[q] = 0.0;
+#endif
+    r.y0 = 0.0f; r.dy = 0.0f;
+    r.y1 = ld_lanes<L>(sz, T_) * k.stdev;  // y0 of segment 0   (:173-175 normal * stdev before interpolation)
     // ---- rollout: segments between inducing points ----
     int t = 0;
     for (int seg = 0; t < a.H; ++seg) {
@@ -205,55 +229,44 @@ __device__ __forceinline__ void mppi_ode_body(const MppiOdeArgs& a) {
       const float cntf = (float)cnt;
       const float w1x2 = full ? segW1x2_full : cntf * (cntf - 1.0f) / pf;
       const float w2 = full ? segW2_full : (cntf - 1.0f) * cntf * (2.0f * cntf - 1.0f) / (6.0f * pf * pf);
-#pragma unroll
-      for (int q = 0; q < ILP; ++q) {
-        const float* sz = sh_z + q * T_ + tid;
-        float y0 = r[q].y1;
-        if (seg == a.n_ind - 1) y0 *= interp_last_point_weight(period);  // reference quirk: last point weighs 1/period (ctk_device.cuh)
-        const float y1 = (seg + 1 < a.n_ind) ? sz[(size_t)(seg + 1) * ILP * T_] * k.stdev : 0.0f;
-        r[q].y0 = y0;
-        r[q].y1 = y1;
-        r[q].dy = y1 - y0;
-        // optimizer_mppi.py:154-155, du^2 term: cc_weight 0.5 (1 - 1/NU) R sum_j du_j^2
-        const float sq = fmaf(r[q].dy, fmaf(w2, r[q].dy, w1x2 * y0), cntf * (y0 * y0));
-        r[q].acc = fmaf(sq, k.k_du2, r[q].acc);
-      }
+      L y0 = r.y1;
+      if (seg == a.n_ind - 1) y0 = y0 * interp_last_point_weight(period);  // reference quirk: last point weighs 1/period (ctk_device.cuh)
+      const L y1 = (seg + 1 < a.n_ind) ? ld_lanes<L>(sz + (size_t)(seg + 1) * ILP * T_, T_) * k.stdev : L(0.0f);
+      r.y0 = y0;
+      r.y1 = y1;
+      r.dy = y1 - y0;
+      // optimizer_mppi.py:154-155, du^2 term: cc_weight 0.5 (1 - 1/NU) R sum_j du_j^2
+      const L sq = fmaf(r.dy, fmaf(w2, r.dy, w1x2 * y0), cntf * (y0 * y0));
+      r.acc = fmaf(sq, k.k_du2, r.acc);
       if (PERIOD > 0 && full) {
 #pragma unroll
         for (int j = 0; j < (PERIOD > 0 ? PERIOD : 1); ++j) {
-          const float un = sh_unom[t + j];
-#pragma unroll
-          for (int q = 0; q < ILP; ++q)
-            ode_mppi_step<KIND, LOG>(a, k, r[q], un, (float)j / (float)(PERIOD > 0 ? PERIOD : 1), j == 0, t + j, n[q], active[q]);
+          ode_mppi_step<KIND, LOG>(a, k, r, sh_unom[t + j], (float)j / (float)(PERIOD > 0 ? PERIOD : 1), j == 0, t + j, n, active);
         }
       } else {
 #pragma unroll 2
         for (int j = 0; j < cnt; ++j) {
-          const float un = sh_unom[t + j];
-          const float wj = sh_w[j].y;
-#pragma unroll
-          for (int q = 0; q < ILP; ++q) ode_mppi_step<KIND, LOG>(a, k, r[q], un, wj, false, t + j, n[q], active[q]);
+          ode_mppi_step<KIND, LOG>(a, k, r, sh_unom[t + j], sh_w[j].y, false, t + j, n, active);
         }
       }
       t += cnt;
-#pragma unroll
-      for (int q = 0; q < ILP; ++q) fold_segment(r[q]);
+      fold_segment(r);
     }
 
     // ---- per-rollout total + per-thread online softmin ----
 #pragma unroll
     for (int q = 0; q < ILP; ++q) {
-      const float th = r[q].T * kSqrt2;
+      const ScaledState rq = lane_of(r, q);
       if (LOG && active[q]) {
         float* p = a.log_traj_soa + (size_t)a.H * 6 * a.N + n[q];
-        p[0] = th; p[a.N] = r[q].W * k.inv_beta; p[2 * (size_t)a.N] = r[q].c; p[3 * (size_t)a.N] = r[q].s;
-        p[4 * (size_t)a.N] = r[q].x; p[5 * (size_t)a.N] = r[q].V * k.inv_cFg;
+        p[0] = rq.T * kSqrt2; p[a.N] = rq.W * k.inv_beta; p[2 * (size_t)a.N] = rq.c; p[3 * (size_t)a.N] = rq.s;
+        p[4 * (size_t)a.N] = rq.x; p[5 * (size_t)a.N] = rq.V * k.inv_cFg;
       }
       // Cost_Functions/__init__.py:90-92 (mean over H+1 incl. the terminal cost); optimizer_mppi.py:160
 #ifdef CTK_K1_DSUM
-      const float S = finish_cost_scaled((float)r[q].dtot, r[q], r[q].ul, k);
+      const float S = finish_cost_scaled((float)r.dtot[q], rq, lane_of(r.ul, q), k);
 #else
-      const float S = finish_cost_scaled(r[q].tot - r[q].comp, r[q], r[q].ul, k);
+      const float S = finish_cost_scaled(lane_of(r.tot, q) - lane_of(r.comp, q), rq, lane_of(r.ul, q), k);
 #endif
       if (active[q]) {
         a.J[n[q]] = S;
@@ -263,10 +276,10 @@ __device__ __forceinline__ void mppi_ode_body(const MppiOdeArgs& a) {
           const float sn = __expf((S - rho_n) * k.neg_inv_lbd);
           a_t = fmaf(a_t, so, sn);
           rho_t = rho_n;
-          const float* sz = sh_z + q * T_ + tid;
+          const float* szq = sz + q * T_;
           for (int i = 0; i < a.n_ind; ++i) {
             const size_t o = (size_t)i * T_;
-            sa[o] = fmaf(sa[o], so, sn * sz[(size_t)i * ILP * T_]);
+            sa[o] = fmaf(sa[o], so, sn * szq[(size_t)i * ILP * T_]);
           }
         }
       }

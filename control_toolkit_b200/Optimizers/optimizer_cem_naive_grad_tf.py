@@ -5,8 +5,9 @@
 Every outer iteration: Q ~ clip(N(dist_mue, stdev)) for the whole population, ONE plain gradient-descent step on every sample
 (``Q - learning_rate * clip_by_norm(dJ/dQ)``, box clip), rollout + cost of the updated samples, top-k refit of mean / population
 std.  After the loop the stdev is clipped to [cem_stdev_min, 10] and both arrays shift by one step; u is the first element of the
-refit MEAN (:105).  On the device: ``gradcem_sample_kernel`` -> ``rpgd_grad_kernel`` (forward tape + hand-derived adjoint, plain
-GD form) -> ``gradcem_refit_kernel`` (bitonic argsort with ties to the lower index, elite gather, refit, shift).
+refit MEAN (:105).  On the device: ``gradcem_sample_kernel<nu>`` -> ``rpgd_grad_kernel`` or ``env_rpgd_grad_kernel`` (forward tape +
+hand-derived adjoint, plain GD form) -> ``gradcem_refit_kernel<nu>`` (bitonic argsort with ties to the lower index, elite gather,
+refit, shift).
 """
 from __future__ import annotations
 

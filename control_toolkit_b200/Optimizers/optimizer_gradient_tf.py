@@ -6,8 +6,8 @@ Every tick: ``gradient_steps`` (first tick: ``warmup_iterations`` if ``warmup``)
 the rollout (per-trajectory ``clip_by_norm``, Keras Adam, box clip), one more rollout for the costs, u = first control of the
 cheapest sequence; then every sequence and both Adam moments shift by one step, the vacated last control is redrawn from
 U[action_low, action_high) and the moments are zero-filled.  On the device this is the RPGD machinery
-(``rpgd_grad_kernel`` + ``rpgd_select_kernel``) with inducing-point period 1, no ranking-based resampling and the
-tail redraw (ctk_config.rpgd_gradient_mode).
+(``rpgd_grad_kernel`` or ``env_rpgd_grad_kernel`` + ``rpgd_select_kernel<nu>``) with inducing-point period 1, no ranking-based
+resampling and the tail redraw (ctk_config.rpgd_gradient_mode).
 """
 from __future__ import annotations
 

@@ -301,54 +301,59 @@ struct RpgdGradArgs {
   float bc1_h[8], bc2_h[8], alpha_h[8];
 };
 
+constexpr int kEnvMaxStates = 8, kEnvMaxControls = 4;  // states / control inputs of any environment (the CartPole: 6 / 1)
+
+// Population steps of the gradient optimizers (ctk_kernels_rpgd_select.cuh), for the CartPole and every registered environment:
+// populations are [H][nu][N] (flat column t * nu + c), limits per input.
 struct RpgdSelectArgs {
   int N, H, k, period, n_ind;
   int shift_previous;
   int resample;            // count % resamp_per == 0
-  int tail_resample;       // gradient mode: no reordering, the LAST control of every row is redrawn (noise rows 0..N-1, one draw each)
+  int tail_resample;       // gradient mode: no reordering, the LAST control of every row is redrawn (noise rows 0..N-1, nu draws each)
   const float* J;          // [N]
-  const float *Q, *m, *v;  // [H][N] current
+  const float *Q, *m, *v;  // [H][nu][N] current
   const float* ages;       // [N]
-  float *Qn, *mn, *vn;     // [H][N] next
+  float *Qn, *mn, *vn;     // [H][nu][N] next
   float* agesn;            // [N]
-  NoiseSrc noise;          // resample draws, per_rollout = n_ind, rows 0..N-k-1
+  NoiseSrc noise;          // resample: per_rollout = n_ind * nu (C order over [n_ind, nu]), rows 0..N-k-1; tail redraw: per_rollout = nu
   int dist;                // 0 normal, 1 uniform
-  float s_mean, s_std, s_min, s_max, lo, hi;
-  float* u_nom_out;        // [H] Q[best_idx[0]] BEFORE the shift (optimal_control_sequence, :426)
-  float* u_prev;           // [1]
-  float* u_out;            // [1] or null
+  float s_mean, s_std;
+  float s_min[kEnvMaxControls], s_max[kEnvMaxControls], lo[kEnvMaxControls], hi[kEnvMaxControls];
+  float* u_nom_out;        // [H][nu] Q[best_idx[0]] BEFORE the shift (optimal_control_sequence, :426)
+  float* u_prev;           // [nu]
+  float* u_out;            // [nu] or null
   int freeze_prev;
   int32_t* best_idx_out;   // [k]
-  HostMirror host;         // u and u_nom_out[H] mirrored to the host caller
+  HostMirror host;         // u of input 0 and u_nom_out mirrored to the host caller (CartPole host-facing ticks), or null
 };
 
 // Gradient-assisted CEM (reference optimizer_cem_naive_grad_tf.py, optimizer_cem_grad_bharadhwaj_tf.py): population stored like RPGD
 struct GradCemSampleArgs {
-  int H, ld, col0, cnt;    // dst[t * ld + col0 + r] for r < cnt, t < H
-  const float *mu, *sd;    // [H]
-  NoiseSrc noise;          // rows 0..cnt-1, per_rollout = H
-  float lo, hi;
-  float* dst;
+  int H, ld, col0, cnt;    // dst[col * ld + col0 + r] for r < cnt, col < H * nu
+  const float *mu, *sd;    // [H][nu]
+  NoiseSrc noise;          // rows 0..cnt-1, per_rollout = H * nu, draw index = column
+  float lo[kEnvMaxControls], hi[kEnvMaxControls];
+  float* dst;              // [H][nu][ld]
 };
 
 struct GradCemRefitArgs {
   int N, H, k;
   const float* J;          // [N] costs of the population AFTER its gradient step
-  const float* Q;          // [H][N] that population
-  float* Q_carry;          // [H][N] next buffer: the k elites are written to columns 0..k-1 (rank order), or null
-  float *mu, *sd;          // [H] out
-  int last;                // 1: post-loop clip / shift
+  const float* Q;          // [H][nu][N] that population
+  float* Q_carry;          // [H][nu][N] next buffer: the k elites are written to columns 0..k-1 (rank order), or null
+  float *mu, *sd;          // [H][nu] out
+  int last;                // 1: post-loop clip / shift, the vacated last step refilled with mid-range means
   int u_from_mean;         // 1: u = refit mean[0] (naive-grad :105), 0: u = best sample's first control (bharadhwaj :168)
-  float sd_min, sd_init, mid;
-  float* u_prev;
-  float* u_out;
+  float sd_min, sd_init;
+  float lo[kEnvMaxControls], hi[kEnvMaxControls];
+  float* u_prev;           // [nu]
+  float* u_out;            // [nu] or null
   int freeze_prev;
   int32_t* elite_idx_out;  // [k] or null
   HostMirror host;         // last iteration: u mirrored to the host caller
 };
 
 // ---- environments registered through the functor registry (ctk_kernels_env.cuh) ----------------------------------------------
-constexpr int kEnvMaxStates = 8, kEnvMaxControls = 4;
 struct EnvParams { float p[24]; };           // environment-specific constants (layout: the Env struct in ctk_kernels_env.cuh)
 struct S0e { const float* p; float v[kEnvMaxStates]; };  // initial state: device pointer, or the values inside the kernel parameters
 struct EnvMppiArgs {
@@ -413,45 +418,6 @@ struct EnvRpgdGradArgs {
   float* log_Q;          // [N][H][NU] or null
   int n_host_adam;
   float bc1_h[8], bc2_h[8], alpha_h[8];
-};
-struct EnvRpgdSelectArgs {
-  int N, H, k, period, n_ind;
-  int shift_previous, resample, tail_resample;  // as RpgdSelectArgs
-  const float* J;
-  const float *Q, *m, *v;  // [H][NU][N] current
-  const float* ages;
-  float *Qn, *mn, *vn;     // [H][NU][N] next
-  float* agesn;
-  NoiseSrc noise;          // resample: per_rollout = n_ind * NU (C order over [n_ind, NU]); tail redraw: per_rollout = NU
-  int dist;                // 0 normal, 1 uniform
-  float s_mean, s_std;
-  float s_min[kEnvMaxControls], s_max[kEnvMaxControls], lo[kEnvMaxControls], hi[kEnvMaxControls];
-  float* u_nom_out;        // [H][NU] Q[best] before the shift
-  float* u_prev;           // [NU]
-  float* u_out;            // [NU] or null
-  int freeze_prev;
-  int32_t* best_idx_out;   // [k]
-};
-struct EnvGradCemSampleArgs {
-  int H, ld, col0, cnt;
-  NoiseSrc noise;          // per_rollout = H * NU, draw index = column
-  const float *mu, *sd;    // [H][NU]
-  float lo[kEnvMaxControls], hi[kEnvMaxControls];
-  float* dst;              // [H][NU][ld]
-};
-struct EnvGradCemRefitArgs {
-  int N, H, k;
-  const float* J;
-  const float* Q;          // [H][NU][N]
-  float* Q_carry;          // [H][NU][N] or null
-  float *mu, *sd;          // [H][NU]
-  int last, u_from_mean;
-  float sd_min, sd_init;
-  float lo[kEnvMaxControls], hi[kEnvMaxControls];
-  float* u_prev;
-  float* u_out;
-  int freeze_prev;
-  int32_t* elite_idx_out;
 };
 
 constexpr int TOPK_THREADS = 1024;  // keys per top-k block

@@ -665,27 +665,18 @@ extern "C" int ctk_clear_injected_noise(ctk_handle* h) {
 // ---------------------------------------------------------------------------------------------------------------
 // reset
 // ---------------------------------------------------------------------------------------------------------------
+// Sampling arguments of the initial population and of K8, with per-input limits.  The CartPole draws over [rpgd_sample_min,
+// rpgd_sample_max] (the gradient-tf tail redraw of K8 over the action limits: rpgd_select_prepare); other environments draw uniformly
+// over each input's own [low, high] when the whole control space is sampled (optimizer_rpgd.py:199-205) and always for gradient-tf
+// (optimizer_gradient_tf.py:171-177)
 static RpgdSelectArgs rpgd_sample_args(ctk_handle* h, NoiseSrc ns) {
-  RpgdSelectArgs a{};
-  a.N = h->N; a.H = h->H; a.k = h->cfg.rpgd_keep_k; a.period = h->period; a.n_ind = h->n_ind;
-  a.shift_previous = h->cfg.rpgd_shift_previous;
-  a.noise = ns; a.dist = h->cfg.rpgd_distribution;
-  a.s_mean = h->cfg.rpgd_sample_mean; a.s_std = h->cfg.rpgd_sample_stdev;
-  a.s_min = h->cfg.rpgd_sample_min; a.s_max = h->cfg.rpgd_sample_max;
-  a.lo = h->cfg.action_low; a.hi = h->cfg.action_high;
-  return a;
-}
-
-// The same for an environment: per-input limits; uniform draws over each input's own [low, high] when the whole control space is
-// sampled (optimizer_rpgd.py:199-205) and always for gradient-tf (optimizer_gradient_tf.py:171-177)
-static EnvRpgdSelectArgs env_rpgd_sample_args(ctk_handle* h, NoiseSrc ns) {
   const ctk_config& c = h->cfg;
-  EnvRpgdSelectArgs a{};
+  RpgdSelectArgs a{};
   a.N = h->N; a.H = h->H; a.k = c.rpgd_keep_k; a.period = h->period; a.n_ind = h->n_ind;
   a.shift_previous = c.rpgd_shift_previous;
   a.noise = ns; a.dist = c.rpgd_distribution;
   a.s_mean = c.rpgd_sample_mean; a.s_std = c.rpgd_sample_stdev;
-  const bool whole = c.rpgd_sample_whole_space != 0 || c.rpgd_gradient_mode == 1;
+  const bool whole = h->env != 0 && (c.rpgd_sample_whole_space != 0 || c.rpgd_gradient_mode == 1);
   for (int i = 0; i < kEnvMaxControls; ++i) {
     a.lo[i] = h->lo_v[i]; a.hi[i] = h->hi_v[i];
     a.s_min[i] = whole ? h->lo_v[i] : c.rpgd_sample_min;
@@ -728,15 +719,9 @@ extern "C" int ctk_reset(ctk_handle* h) {
     if (rcn != CTK_OK) return rcn;
     h->cur = 0;
     h->launches++;
-    if (h->env != 0) {
-      EnvRpgdSelectArgs a = env_rpgd_sample_args(h, ns);
-      a.Qn = h->d_Q[0]; a.mn = h->d_m[0]; a.vn = h->d_v[0]; a.agesn = h->d_ages[0];
-      CU(launch_env_rpgd_init(h->env, a, h->stream));
-    } else {
-      RpgdSelectArgs a = rpgd_sample_args(h, ns);
-      a.Qn = h->d_Q[0]; a.mn = h->d_m[0]; a.vn = h->d_v[0]; a.agesn = h->d_ages[0];
-      CU(launch_rpgd_init(a, h->stream));
-    }
+    RpgdSelectArgs a = rpgd_sample_args(h, ns);
+    a.Qn = h->d_Q[0]; a.mn = h->d_m[0]; a.vn = h->d_v[0]; a.agesn = h->d_ages[0];
+    CU(launch_rpgd_init(h->nu, a, h->stream));
     h->adam_step = 0;
   }
   CU(cudaStreamSynchronize(h->stream));
@@ -1222,22 +1207,41 @@ static void fill_host_adam(GradArgs& a) {
   }
 }
 
+// Gradient step on an environment other than the CartPole (ctk_kernels_env_rpgd.cuh), population [H][nu][N]
+static EnvRpgdGradArgs env_rpgd_grad_args(ctk_handle* h, const S0e& s0, int iters, float* Q, float* m, float* v, int adam_form) {
+  const ctk_config& c = h->cfg;
+  EnvRpgdGradArgs a{};
+  a.N = h->N; a.H = h->H; a.iters = iters; a.s0 = s0; a.u_prev = h->d_u_prev;
+  a.Q = Q; a.m = m; a.v = v;
+  for (int i = 0; i < kEnvMaxControls; ++i) { a.lo[i] = h->lo_v[i]; a.hi[i] = h->hi_v[i]; }
+  a.lr = c.rpgd_learning_rate; a.gradmax_clip = c.rpgd_gradmax_clip;
+  a.beta1 = c.rpgd_beta_1; a.beta2 = c.rpgd_beta_2; a.eps = c.rpgd_epsilon; a.adam_step0 = h->adam_step; a.adam_form = adam_form;
+  a.env = h->env_p; a.J = h->d_J; a.log_traj = h->d_log_traj_soa; a.log_Q = h->d_log_Q_soa;
+  fill_host_adam(a);
+  return a;
+}
+static std::string env_grad_kernel_name(const ctk_handle* h, bool fused) {
+  return std::string("env_rpgd_grad_kernel<DubinsEnv,") + (h->cfg.logging ? "1" : "0") + ">" + (fused ? " [fused select]" : "");
+}
+
 // Gradient-assisted CEM tick (rpgd_gradient_mode 2: optimizer_cem_naive_grad_tf.py:90-114, 3: optimizer_cem_grad_bharadhwaj_tf.py:151-178)
-static int gradcem_tick(ctk_handle* h, const float* s_dev, float* u_out_dev) {
+// over nu columns.  The state: s_dev (or h_pin) for the CartPole's gradient kernel, s0e for another environment's.
+static int gradcem_tick(ctk_handle* h, const float* s_dev, const S0e& s0e, float* u_out_dev) {
   const ctk_config& c = h->cfg;
   const bool carry = c.rpgd_gradient_mode == 3;
-  const int N = h->N, H = h->H, k = c.cem_best_k;
+  const int N = h->N, H = h->H, k = c.cem_best_k, nu = h->nu;
   const int iters = carry ? cem_tick_iters(h) : c.cem_outer_it;
   const int kc = carry ? k : 0;
   auto sample = [&](int col0, int cnt, uint32_t sub) -> int {
     if (cnt <= 0) return CTK_OK;
     GradCemSampleArgs a{};
-    int rcn = make_noise(h, STREAM_CEM | (sub << 8), H, 0, (size_t)cnt, &a.noise);
+    int rcn = make_noise(h, STREAM_CEM | (sub << 8), H * nu, 0, (size_t)cnt, &a.noise);
     if (rcn != CTK_OK) return rcn;
-    a.H = H; a.ld = N; a.col0 = col0; a.cnt = cnt; a.mu = h->d_mu; a.sd = h->d_sd; a.lo = c.action_low; a.hi = c.action_high;
+    a.H = H; a.ld = N; a.col0 = col0; a.cnt = cnt; a.mu = h->d_mu; a.sd = h->d_sd;
+    for (int i = 0; i < kEnvMaxControls; ++i) { a.lo[i] = h->lo_v[i]; a.hi[i] = h->hi_v[i]; }
     a.dst = h->d_Q[h->cur];
     h->launches++;
-    CU(launch_gradcem_sample(a, h->stream));
+    CU(launch_gradcem_sample(nu, a, h->stream));
     return CTK_OK;
   };
   int rc = carry ? sample(0, k, 0) : CTK_OK;  // bharadhwaj :159 the first "elites" are plain samples
@@ -1246,35 +1250,47 @@ static int gradcem_tick(ctk_handle* h, const float* s_dev, float* u_out_dev) {
   for (int it = 0; it < iters; ++it) {
     rc = sample(kc, N - kc, (uint32_t)it + 1);
     if (rc != CTK_OK) return rc;
-    RpgdGradArgs a{};
-    a.N = N; a.H = H; a.iters = 1; a.s0 = make_s0(h, s_dev); a.u_prev = h->d_u_prev;
-    a.Q = h->d_Q[h->cur]; a.m = h->d_m[0]; a.v = h->d_v[0];
-    a.lo = c.action_low; a.hi = c.action_high; a.lr = c.rpgd_learning_rate; a.gradmax_clip = c.rpgd_gradmax_clip;
-    a.beta1 = c.rpgd_beta_1; a.beta2 = c.rpgd_beta_2; a.eps = c.rpgd_epsilon; a.adam_step0 = h->adam_step;
-    a.adam_form = carry ? 0 : 2;
-    fill_host_adam(a);
-    a.kc = h->d_kc; a.ode = h->ode; a.fwd = h->fwd; a.cost = h->cost; a.J = h->d_J; a.log_traj_soa = h->d_log_traj_soa;
-    const int B = 32;
-    const bool coef = sizeof(float) * (size_t)H * B * 12 <= 227 * 1024;  // coefficient tape: q, g, m, v and 8 coefficients per step
-    const size_t smem = sizeof(float) * (size_t)H * B * (coef ? 12 : 8);
-    if (smem > 227 * 1024) return fail(CTK_EINVAL, "mpc_horizon too large for the shared-memory tape (max 227)");
-    h->launches++;
-    {
-      KernelTimer kt(h);
-      CU(launch_rpgd_grad(h->cost.kind, c.logging != 0, coef, (N + B - 1) / B, B, smem, h->stream, a));
+    const bool last = it == iters - 1;
+    if (h->env != 0) {
+      const EnvRpgdGradArgs a = env_rpgd_grad_args(h, s0e, 1, h->d_Q[h->cur], h->d_m[0], h->d_v[0], carry ? 0 : 2);
+      h->launches++;
+      {
+        KernelTimer kt(h);
+        CU(launch_env_rpgd_grad(h->env, c.logging != 0, env_rpgd_smem_bytes(h->env, H), h->stream, a, nullptr));
+      }
+      h->last_kernel = env_grad_kernel_name(h, false);
+    } else {
+      RpgdGradArgs a{};
+      a.N = N; a.H = H; a.iters = 1; a.s0 = make_s0(h, s_dev); a.u_prev = h->d_u_prev;
+      a.Q = h->d_Q[h->cur]; a.m = h->d_m[0]; a.v = h->d_v[0];
+      a.lo = c.action_low; a.hi = c.action_high; a.lr = c.rpgd_learning_rate; a.gradmax_clip = c.rpgd_gradmax_clip;
+      a.beta1 = c.rpgd_beta_1; a.beta2 = c.rpgd_beta_2; a.eps = c.rpgd_epsilon; a.adam_step0 = h->adam_step;
+      a.adam_form = carry ? 0 : 2;
+      fill_host_adam(a);
+      a.kc = h->d_kc; a.ode = h->ode; a.fwd = h->fwd; a.cost = h->cost; a.J = h->d_J; a.log_traj_soa = h->d_log_traj_soa;
+      const int B = 32;
+      const bool coef = sizeof(float) * (size_t)H * B * 12 <= 227 * 1024;  // coefficient tape: q, g, m, v and 8 coefficients per step
+      const size_t smem = sizeof(float) * (size_t)H * B * (coef ? 12 : 8);
+      if (smem > 227 * 1024) return fail(CTK_EINVAL, "mpc_horizon too large for the shared-memory tape (max 227)");
+      h->launches++;
+      {
+        KernelTimer kt(h);
+        CU(launch_rpgd_grad(h->cost.kind, c.logging != 0, coef, (N + B - 1) / B, B, smem, h->stream, a));
+      }
+      // Q_logged of the last population (the environment kernel writes log_Q itself)
+      if (last && c.logging) CU(cudaMemcpyAsync(h->d_Q_log, h->d_Q[h->cur], sizeof(float) * N * H, cudaMemcpyDeviceToDevice, h->stream));
     }
     if (carry) h->adam_step += 1;
-    const bool last = it == iters - 1;
-    if (last && c.logging) CU(cudaMemcpyAsync(h->d_Q_log, h->d_Q[h->cur], sizeof(float) * N * H, cudaMemcpyDeviceToDevice, h->stream));
     GradCemRefitArgs r{};
     r.N = N; r.H = H; r.k = k; r.J = h->d_J; r.Q = h->d_Q[h->cur]; r.Q_carry = carry ? h->d_Q[h->cur ^ 1].get() : nullptr;
     r.mu = h->d_mu; r.sd = h->d_sd; r.last = last ? 1 : 0; r.u_from_mean = carry ? 0 : 1;
-    r.sd_min = c.cem_stdev_min; r.sd_init = c.cem_initial_action_stdev; r.mid = 0.5f * (c.action_low + c.action_high);
+    r.sd_min = c.cem_stdev_min; r.sd_init = c.cem_initial_action_stdev;
+    for (int i = 0; i < kEnvMaxControls; ++i) { r.lo[i] = h->lo_v[i]; r.hi[i] = h->hi_v[i]; }
     r.u_prev = h->d_u_prev; r.u_out = u_out_dev; r.freeze_prev = c.freeze_previous_input;
     r.elite_idx_out = (it < h->elite_log_cap) ? h->d_elite_idx + (size_t)it * k : nullptr;
     if (last) r.host = h->mirror;
     h->launches++;
-    CU(launch_gradcem_refit(r, h->stream));
+    CU(launch_gradcem_refit(nu, r, h->stream));
     if (r.elite_idx_out) h->elite_log_rows++;
     if (carry) h->cur ^= 1;
   }
@@ -1314,17 +1330,20 @@ static int rpgd_select_prepare(ctk_handle* h, float* u_out_dev, RpgdSelectArgs* 
   const int grad_mode = c.rpgd_gradient_mode == 1 ? 1 : 0;
   const int resample = (!grad_mode && h->count % c.rpgd_resamp_per == 0) ? 1 : 0;  // optimizer_rpgd.py:449
   NoiseSrc ns{};
-  if (grad_mode) {  // one uniform draw per row for the vacated last step (optimizer_gradient_tf.py:142-147)
-    int rcn = make_noise(h, STREAM_RPGD_RESAMPLE, 1, 1, (size_t)h->N, &ns);
+  if (grad_mode) {  // [N, 1, nu] uniform draws for the vacated last step (optimizer_gradient_tf.py:142-147)
+    int rcn = make_noise(h, STREAM_RPGD_RESAMPLE, h->nu, 1, (size_t)h->N, &ns);
     if (rcn != CTK_OK) return rcn;
   } else if (resample && h->N - c.rpgd_keep_k > 0) {
-    int rcn = make_noise(h, STREAM_RPGD_RESAMPLE, h->n_ind, c.rpgd_distribution == CTK_DIST_UNIFORM, (size_t)(h->N - c.rpgd_keep_k), &ns);
+    int rcn = make_noise(h, STREAM_RPGD_RESAMPLE, h->n_ind * h->nu, c.rpgd_distribution == CTK_DIST_UNIFORM, (size_t)(h->N - c.rpgd_keep_k), &ns);
     if (rcn != CTK_OK) return rcn;
   }
   RpgdSelectArgs a = rpgd_sample_args(h, ns);
   a.resample = resample;
   a.tail_resample = grad_mode;
-  if (grad_mode) { a.dist = CTK_DIST_UNIFORM; a.s_min = c.action_low; a.s_max = c.action_high; }
+  if (grad_mode) {  // the tail redraw is uniform over the action limits
+    a.dist = CTK_DIST_UNIFORM;
+    for (int i = 0; i < kEnvMaxControls; ++i) { a.s_min[i] = h->lo_v[i]; a.s_max[i] = h->hi_v[i]; }
+  }
   a.J = h->d_J; a.Q = h->d_Q[h->cur]; a.m = h->d_m[h->cur]; a.v = h->d_v[h->cur]; a.ages = h->d_ages[h->cur];
   const int nx = h->cur ^ 1;
   a.Qn = h->d_Q[nx]; a.mn = h->d_m[nx]; a.vn = h->d_v[nx]; a.agesn = h->d_ages[nx];
@@ -1341,7 +1360,7 @@ static void rpgd_select_commit(ctk_handle* h) {
 
 static int rpgd_finish(ctk_handle* h, float* u_out_dev) {
   const ctk_config& c = h->cfg;
-  if (c.rpgd_gradient_mode >= 2) return gradcem_tick(h, h->pending_s, u_out_dev);
+  if (c.rpgd_gradient_mode >= 2) return gradcem_tick(h, h->pending_s, S0e{}, u_out_dev);
   RpgdSelectArgs a{};
   int rc = rpgd_select_prepare(h, u_out_dev, &a);
   if (rc != CTK_OK) return rc;
@@ -1350,7 +1369,7 @@ static int rpgd_finish(ctk_handle* h, float* u_out_dev) {
     CU(cudaMemcpyAsync(h->d_ages_log, h->d_ages[h->cur], sizeof(float) * h->N, cudaMemcpyDeviceToDevice, h->stream));
   }
   h->launches++;
-  CU(launch_rpgd_select(a, h->stream));
+  CU(launch_rpgd_select(h->nu, a, h->stream));
   rpgd_select_commit(h);
   return CTK_OK;
 }
@@ -1374,104 +1393,17 @@ static int rpgd_tick(ctk_handle* h, const float* s_dev, float* u_out_dev) {
   return CTK_OK;
 }
 
-// ---------------------------------------------------------------------------------------------------------------
-// gradient optimizers on environments (ctk_kernels_env_rpgd.cuh): the same tick structure as the CartPole's, population [H][nu][N]
-// ---------------------------------------------------------------------------------------------------------------
-static EnvRpgdGradArgs env_rpgd_grad_args(ctk_handle* h, const S0e& s0, int iters, float* Q, float* m, float* v, int adam_form) {
-  const ctk_config& c = h->cfg;
-  EnvRpgdGradArgs a{};
-  a.N = h->N; a.H = h->H; a.iters = iters; a.s0 = s0; a.u_prev = h->d_u_prev;
-  a.Q = Q; a.m = m; a.v = v;
-  for (int i = 0; i < kEnvMaxControls; ++i) { a.lo[i] = h->lo_v[i]; a.hi[i] = h->hi_v[i]; }
-  a.lr = c.rpgd_learning_rate; a.gradmax_clip = c.rpgd_gradmax_clip;
-  a.beta1 = c.rpgd_beta_1; a.beta2 = c.rpgd_beta_2; a.eps = c.rpgd_epsilon; a.adam_step0 = h->adam_step; a.adam_form = adam_form;
-  a.env = h->env_p; a.J = h->d_J; a.log_traj = h->d_log_traj_soa; a.log_Q = h->d_log_Q_soa;
-  fill_host_adam(a);
-  return a;
-}
-static std::string env_grad_kernel_name(const ctk_handle* h, bool fused) {
-  return std::string("env_rpgd_grad_kernel<DubinsEnv,") + (h->cfg.logging ? "1" : "0") + ">" + (fused ? " [fused select]" : "");
-}
-
-// gradient-assisted CEM (gradcem_tick over nu columns)
-static int env_gradcem_tick(ctk_handle* h, const S0e& s0, float* u_out_dev) {
-  const ctk_config& c = h->cfg;
-  const bool carry = c.rpgd_gradient_mode == 3;
-  const int N = h->N, H = h->H, k = c.cem_best_k, nu = h->nu;
-  const int iters = carry ? cem_tick_iters(h) : c.cem_outer_it;
-  const int kc = carry ? k : 0;
-  auto sample = [&](int col0, int cnt, uint32_t sub) -> int {
-    if (cnt <= 0) return CTK_OK;
-    EnvGradCemSampleArgs a{};
-    int rcn = make_noise(h, STREAM_CEM | (sub << 8), H * nu, 0, (size_t)cnt, &a.noise);
-    if (rcn != CTK_OK) return rcn;
-    a.H = H; a.ld = N; a.col0 = col0; a.cnt = cnt; a.mu = h->d_mu; a.sd = h->d_sd;
-    for (int i = 0; i < kEnvMaxControls; ++i) { a.lo[i] = h->lo_v[i]; a.hi[i] = h->hi_v[i]; }
-    a.dst = h->d_Q[h->cur];
-    h->launches++;
-    CU(launch_env_gradcem_sample(h->env, a, h->stream));
-    return CTK_OK;
-  };
-  int rc = carry ? sample(0, k, 0) : CTK_OK;  // bharadhwaj :159 the first "elites" are plain samples
-  if (rc != CTK_OK) return rc;
-  h->elite_log_rows = 0;
-  const size_t smem = env_rpgd_smem_bytes(h->env, H);
-  for (int it = 0; it < iters; ++it) {
-    rc = sample(kc, N - kc, (uint32_t)it + 1);
-    if (rc != CTK_OK) return rc;
-    const EnvRpgdGradArgs a = env_rpgd_grad_args(h, s0, 1, h->d_Q[h->cur], h->d_m[0], h->d_v[0], carry ? 0 : 2);
-    h->launches++;
-    {
-      KernelTimer kt(h);
-      CU(launch_env_rpgd_grad(h->env, c.logging != 0, smem, h->stream, a, nullptr));
-    }
-    h->last_kernel = env_grad_kernel_name(h, false);
-    if (carry) h->adam_step += 1;
-    const bool last = it == iters - 1;
-    EnvGradCemRefitArgs r{};
-    r.N = N; r.H = H; r.k = k; r.J = h->d_J; r.Q = h->d_Q[h->cur]; r.Q_carry = carry ? h->d_Q[h->cur ^ 1].get() : nullptr;
-    r.mu = h->d_mu; r.sd = h->d_sd; r.last = last ? 1 : 0; r.u_from_mean = carry ? 0 : 1;
-    r.sd_min = c.cem_stdev_min; r.sd_init = c.cem_initial_action_stdev;
-    for (int i = 0; i < kEnvMaxControls; ++i) { r.lo[i] = h->lo_v[i]; r.hi[i] = h->hi_v[i]; }
-    r.u_prev = h->d_u_prev; r.u_out = u_out_dev; r.freeze_prev = c.freeze_previous_input;
-    r.elite_idx_out = (it < h->elite_log_cap) ? h->d_elite_idx + (size_t)it * k : nullptr;
-    h->launches++;
-    CU(launch_env_gradcem_refit(h->env, r, h->stream));
-    if (r.elite_idx_out) h->elite_log_rows++;
-    if (carry) h->cur ^= 1;
-  }
-  h->count++;
-  return CTK_OK;
-}
-
-// RPGD / gradient-tf: one launch (gradient steps + fused K8) for a population of one block with logging off, else two
+// RPGD / gradient-tf on an environment other than the CartPole: one launch (gradient steps + fused K8) for a population of one block
+// with logging off, else two
 static int env_rpgd_tick(ctk_handle* h, const S0e& s0, float* u_out_dev) {
   const ctk_config& c = h->cfg;
-  if (c.rpgd_gradient_mode >= 2) return env_gradcem_tick(h, s0, u_out_dev);
-  const int N = h->N, nu = h->nu;
-  const int grad_mode = c.rpgd_gradient_mode == 1 ? 1 : 0;
-  const int resample = (!grad_mode && h->count % c.rpgd_resamp_per == 0) ? 1 : 0;  // optimizer_rpgd.py:449
-  NoiseSrc ns{};
-  if (grad_mode) {  // [N, 1, nu] uniform draws for the vacated last step (optimizer_gradient_tf.py:142-147)
-    int rcn = make_noise(h, STREAM_RPGD_RESAMPLE, nu, 1, (size_t)N, &ns);
-    if (rcn != CTK_OK) return rcn;
-  } else if (resample && N - c.rpgd_keep_k > 0) {
-    int rcn = make_noise(h, STREAM_RPGD_RESAMPLE, h->n_ind * nu, c.rpgd_distribution == CTK_DIST_UNIFORM, (size_t)(N - c.rpgd_keep_k), &ns);
-    if (rcn != CTK_OK) return rcn;
-  }
-  EnvRpgdSelectArgs sel = env_rpgd_sample_args(h, ns);
-  sel.resample = resample;
-  sel.tail_resample = grad_mode;
-  if (grad_mode) sel.dist = CTK_DIST_UNIFORM;
-  const int nx = h->cur ^ 1;
-  sel.J = h->d_J; sel.Q = h->d_Q[h->cur]; sel.m = h->d_m[h->cur]; sel.v = h->d_v[h->cur]; sel.ages = h->d_ages[h->cur];
-  sel.Qn = h->d_Q[nx]; sel.mn = h->d_m[nx]; sel.vn = h->d_v[nx]; sel.agesn = h->d_ages[nx];
-  sel.u_nom_out = h->d_unom_log; sel.u_prev = h->d_u_prev; sel.u_out = u_out_dev; sel.freeze_prev = c.freeze_previous_input;
-  sel.best_idx_out = h->d_best_idx;
-
+  if (c.rpgd_gradient_mode >= 2) return gradcem_tick(h, nullptr, s0, u_out_dev);
+  RpgdSelectArgs sel{};
+  int rc = rpgd_select_prepare(h, u_out_dev, &sel);
+  if (rc != CTK_OK) return rc;
   const int iters = (h->count == 0) ? c.rpgd_first_iter_count : c.rpgd_outer_its;  // optimizer_rpgd.py:397-400
   const EnvRpgdGradArgs a = env_rpgd_grad_args(h, s0, iters, h->d_Q[h->cur], h->d_m[h->cur], h->d_v[h->cur], c.rpgd_adam_form);
-  const bool fuse = N <= kEnvRpgdBlock && !c.logging;
+  const bool fuse = h->N <= kEnvRpgdBlock && !c.logging;
   h->launches++;
   {
     KernelTimer kt(h);
@@ -1481,12 +1413,11 @@ static int env_rpgd_tick(ctk_handle* h, const S0e& s0, float* u_out_dev) {
   h->adam_step += iters;
   if (!fuse) {
     // trajectory_ages_logged: the ages BEFORE the warm-start update (:413-415); Q_logged is written by the gradient kernel
-    if (c.logging) CU(cudaMemcpyAsync(h->d_ages_log, h->d_ages[h->cur], sizeof(float) * N, cudaMemcpyDeviceToDevice, h->stream));
+    if (c.logging) CU(cudaMemcpyAsync(h->d_ages_log, h->d_ages[h->cur], sizeof(float) * h->N, cudaMemcpyDeviceToDevice, h->stream));
     h->launches++;
-    CU(launch_env_rpgd_select(h->env, sel, h->stream));
+    CU(launch_rpgd_select(h->nu, sel, h->stream));
   }
-  h->cur = nx;
-  h->count++;
+  rpgd_select_commit(h);
   return CTK_OK;
 }
 

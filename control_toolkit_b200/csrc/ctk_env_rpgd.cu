@@ -1,19 +1,19 @@
-// ctk_env_rpgd.cu -- translation unit owning the gradient-optimizer kernels of the general environments (ctk_kernels_env_rpgd.cuh).
+// ctk_env_rpgd.cu -- translation unit owning the gradient kernel of the general environments (ctk_kernels_env_rpgd.cuh).
 // A unit of its own: the shared-memory kernels here would otherwise change the reserved shared memory of ctk_env.cu's kernels.
 #include "ctk_kernels_env_rpgd.cuh"
 #include "ctk_launch.h"
 
 namespace ctk {
 
-cudaError_t launch_env_rpgd_grad(int env, bool log, size_t smem, cudaStream_t st, const EnvRpgdGradArgs& a, const EnvRpgdSelectArgs* fused_select) {
+cudaError_t launch_env_rpgd_grad(int env, bool log, size_t smem, cudaStream_t st, const EnvRpgdGradArgs& a, const RpgdSelectArgs* fused_select) {
   if (env != 1) return cudaErrorInvalidValue;
-  void (*k)(const EnvRpgdGradArgs, const EnvRpgdSelectArgs, const int) =
+  void (*k)(const EnvRpgdGradArgs, const RpgdSelectArgs, const int) =
       log ? env_rpgd_grad_kernel<DubinsEnv, true> : env_rpgd_grad_kernel<DubinsEnv, false>;
   if (smem > 48 * 1024) {
     cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
   }
-  const EnvRpgdSelectArgs none{};
+  const RpgdSelectArgs none{};
   k<<<(a.N + kEnvRpgdBlock - 1) / kEnvRpgdBlock, kEnvRpgdBlock, smem, st>>>(a, fused_select ? *fused_select : none, fused_select ? 1 : 0);
   return cudaGetLastError();
 }
@@ -21,25 +21,5 @@ size_t env_rpgd_smem_bytes(int env, int H) {
   int ns, nu;
   env_dims(env, &ns, &nu);
   return sizeof(float) * (size_t)H * kEnvRpgdBlock * env_rpgd_tape_floats(ns, nu);
-}
-cudaError_t launch_env_rpgd_select(int env, const EnvRpgdSelectArgs& a, cudaStream_t st) {
-  if (env != 1) return cudaErrorInvalidValue;
-  env_rpgd_select_kernel<DubinsEnv::NU><<<1, TOPK_THREADS, 0, st>>>(a);
-  return cudaGetLastError();
-}
-cudaError_t launch_env_rpgd_init(int env, const EnvRpgdSelectArgs& a, cudaStream_t st) {
-  if (env != 1) return cudaErrorInvalidValue;
-  env_rpgd_init_kernel<DubinsEnv::NU><<<(a.N * a.H * DubinsEnv::NU + 255) / 256, 256, 0, st>>>(a);
-  return cudaGetLastError();
-}
-cudaError_t launch_env_gradcem_sample(int env, const EnvGradCemSampleArgs& a, cudaStream_t st) {
-  if (env != 1) return cudaErrorInvalidValue;
-  env_gradcem_sample_kernel<DubinsEnv::NU><<<(a.cnt * a.H * DubinsEnv::NU + 255) / 256, 256, 0, st>>>(a);
-  return cudaGetLastError();
-}
-cudaError_t launch_env_gradcem_refit(int env, const EnvGradCemRefitArgs& a, cudaStream_t st) {
-  if (env != 1) return cudaErrorInvalidValue;
-  env_gradcem_refit_kernel<DubinsEnv::NU><<<1, TOPK_THREADS, 0, st>>>(a);
-  return cudaGetLastError();
 }
 }  // namespace ctk

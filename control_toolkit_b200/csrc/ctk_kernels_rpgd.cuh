@@ -1,10 +1,10 @@
-// ctk_kernels_rpgd.cuh -- K6/K7 forward tape + reverse-mode adjoint + Adam, K8 select / shift / resample.
-// Replaces reference optimizer_rpgd.py:306-338 (grad_step), :340-380 (get_action) and :443-516 (warm start /
-// resampling / Adam-moment bookkeeping) for one tick.  Population arrays are stored t-major ([H][N]) on the device so
-// that one-thread-per-trajectory access is coalesced; the C-ABI transposes to the reference's [N,H,nu].
+// ctk_kernels_rpgd.cuh -- K6/K7 forward tape + reverse-mode adjoint + Adam for the CartPole; K8 select / shift / resample
+// (rpgd_select_body<1>, ctk_kernels_rpgd_select.cuh) fused into the coefficient-form kernel.
+// Replaces reference optimizer_rpgd.py:306-338 (grad_step) and :340-380 (get_action) for one tick.  Population arrays are stored
+// t-major ([H][N]) on the device so that one-thread-per-trajectory access is coalesced; the C-ABI transposes to the reference's [N,H,nu].
 #pragma once
 #include "ctk_device.cuh"
-#include "ctk_topk.cuh"
+#include "ctk_kernels_rpgd_select.cuh"
 
 namespace ctk {
 
@@ -107,81 +107,6 @@ __global__ void __launch_bounds__(32) rpgd_grad_kernel(const RpgdGradArgs a) {
     p[0] = z.th; p[a.N] = z.om; p[2 * a.N] = z.c; p[3 * a.N] = z.s; p[4 * (size_t)a.N] = z.x; p[5 * (size_t)a.N] = z.v;
   }
   a.J[n] = (jsum + terminal_cost(z, a.cost)) - a.cost.shift;
-}
-
-// sample_actions (:275-296) for one new row at horizon step t: clip(z*scale+offset) on inducing points, interpolate
-__device__ __forceinline__ float rpgd_sample_point(const RpgdSelectArgs& a, uint32_t row, int i) {
-  const float z = noise1(a.noise, row, i);
-  const float y = a.dist == 0 ? __fadd_rn(__fmul_rn(z, a.s_std), a.s_mean) : __fadd_rn(__fmul_rn(z, a.s_max - a.s_min), a.s_min);
-  return fminf(fmaxf(y, a.lo), a.hi);
-}
-
-// K8 body: any block size >= the padded population (callers: rpgd_select_kernel, and rpgd_grad_coef_kernel when the whole
-// population is one block -- then the tick is ONE launch)
-__device__ __forceinline__ void rpgd_select_body(const RpgdSelectArgs& a, uint64_t* sh, int* sh_best) {
-  const int tid = threadIdx.x;
-  uint64_t key = (tid < a.N) ? make_key(a.J[tid], (uint32_t)tid) : KEY_MAX;
-  int n_sort = 32;
-  while (n_sort < a.N) n_sort <<= 1;
-  key = block_bitonic_sort(key, sh, n_sort);  // argsort (:345), stable by index; C3's 32 costs stay inside one warp's shuffles
-  if (tid < a.k) {
-    sh_best[tid] = (int)(key & 0xffffffffu);
-    a.best_idx_out[tid] = sh_best[tid];
-  }
-  __syncthreads();
-  const int best = sh_best[0];
-  for (int t = tid; t < a.H; t += blockDim.x) {
-    const float q = a.Q[(size_t)t * a.N + best];
-    a.u_nom_out[t] = q;  // :426
-    if (a.host.p != nullptr) host_put(a.host, 8 + t, q);
-  }
-  if (tid == 0) {
-    const float u = a.Q[best];
-    if (!a.freeze_prev) a.u_prev[0] = u;
-    if (a.u_out != nullptr) a.u_out[0] = u;
-    if (a.host.p != nullptr) { host_put(a.host, 5, 0.0f); host_put(a.host, 4, u); }
-  }
-  const int nnew = a.resample ? a.N - a.k : 0;
-#pragma unroll 4
-  for (int idx = tid; idx < a.N * a.H; idx += blockDim.x) {
-    const int t = idx / a.N, n = idx - t * a.N;
-    float q, mm, vv;
-    if (n < nnew) {
-      // fresh sample (:451-453): interpolate clipped inducing points (Interpolator.py:97-106)
-      const int seg = t / a.period, j = t - seg * a.period;
-      float w0, w1;
-      interp_weights(seg, j, a.period, a.n_ind, &w0, &w1);
-      const float y0 = rpgd_sample_point(a, (uint32_t)n, seg);
-      const float y1 = (j > 0) ? rpgd_sample_point(a, (uint32_t)n, seg + 1) : 0.0f;
-      q = fmaf(y1, w1, __fmul_rn(y0, w0));
-      mm = 0.0f;
-      vv = 0.0f;
-    } else {
-      const int src = a.resample ? sh_best[n - nnew] : n;  // gather in best order (:454) or identity
-      const int ts = min(t + a.shift_previous, a.H - 1);   // :376-379 shift, repeat the last
-      q = a.Q[(size_t)ts * a.N + src];
-      // optimizer_gradient_tf.py:142-149: the vacated last step gets a fresh uniform control instead of a repeat
-      if (a.tail_resample && t == a.H - 1) q = rpgd_sample_point(a, (uint32_t)n, 0);
-      // Adam moments: always shifted by ONE with zero fill (:462-513)
-      mm = (t + 1 < a.H) ? a.m[(size_t)(t + 1) * a.N + src] : 0.0f;
-      vv = (t + 1 < a.H) ? a.v[(size_t)(t + 1) * a.N + src] : 0.0f;
-    }
-    a.Qn[idx] = q;
-    a.mn[idx] = mm;
-    a.vn[idx] = vv;
-  }
-  for (int n = tid; n < a.N; n += blockDim.x) {
-    const float age = (n < nnew) ? 0.0f : a.ages[a.resample ? sh_best[n - nnew] : n];
-    a.agesn[n] = age + 1.0f;  // :514
-  }
-}
-
-__global__ void __launch_bounds__(TOPK_THREADS) rpgd_select_kernel(const RpgdSelectArgs a) {
-  __shared__ uint64_t sh[TOPK_THREADS];
-  __shared__ int sh_best[TOPK_THREADS];
-  pdl_wait();
-  pdl_trigger();
-  rpgd_select_body(a, sh, sh_best);
 }
 
 // The same tick with the adjoint in COEFFICIENT form (ctk_math.cuh adjoint_coefficients / adjoint_apply): the forward pass folds
@@ -355,94 +280,9 @@ __global__ void __launch_bounds__(32 * kRpgdWarps) rpgd_grad_coef_kernel(const R
     __shared__ uint64_t sh_sel[32 * kRpgdWarps];
     __shared__ int sh_best[32 * kRpgdWarps];
     __syncthreads();  // J, Q, m, v of every trajectory are written (same block: visible after the barrier)
-    rpgd_select_body(sel, sh_sel, sh_best);
+    rpgd_select_body<1>(sel, sh_sel, sh_best);
   }
   trace();
-}
-
-// initial population (optimizer_reset :540): all N rows sampled; Adam state zeroed
-__global__ void rpgd_init_kernel(const RpgdSelectArgs a) {
-  for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < a.N * a.H; idx += gridDim.x * blockDim.x) {
-    const int t = idx / a.N, n = idx - t * a.N;
-    const int seg = t / a.period, j = t - seg * a.period;
-    float w0, w1;
-    interp_weights(seg, j, a.period, a.n_ind, &w0, &w1);
-    const float y0 = rpgd_sample_point(a, (uint32_t)n, seg);
-    const float y1 = (j > 0) ? rpgd_sample_point(a, (uint32_t)n, seg + 1) : 0.0f;
-    a.Qn[idx] = fmaf(y1, w1, __fmul_rn(y0, w0));
-    a.mn[idx] = 0.0f;
-    a.vn[idx] = 0.0f;
-    if (t == 0) a.agesn[n] = 0.0f;
-  }
-}
-
-// ---------------------------------------------------------------------------------------------------------------
-// Gradient-assisted CEM (reference optimizer_cem_naive_grad_tf.py:58-87, optimizer_cem_grad_bharadhwaj_tf.py:93-132)
-// ---------------------------------------------------------------------------------------------------------------
-// Q[t][col0 + r] = clip(mu_t + z_{r,t} * sd_t)  (multiply and add separately rounded, as the reference's tf ops)
-__global__ void gradcem_sample_kernel(const GradCemSampleArgs a) {
-  pdl_wait();
-  pdl_trigger();
-  for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < a.cnt * a.H; idx += gridDim.x * blockDim.x) {
-    const int t = idx / a.cnt, r = idx - t * a.cnt;
-    const float z = noise1(a.noise, (uint32_t)r, t);
-    a.dst[(size_t)t * a.ld + a.col0 + r] = fminf(fmaxf(__fadd_rn(a.mu[t], __fmul_rn(z, a.sd[t])), a.lo), a.hi);
-  }
-}
-
-// argsort of the N <= 1024 costs (ties to the lower index), elite gather in rank order, mean / population std per horizon step,
-// elites carried into the next population buffer, and on the last outer iteration the clip / shift / u of ``step``
-__global__ void __launch_bounds__(TOPK_THREADS) gradcem_refit_kernel(const GradCemRefitArgs a) {
-  __shared__ uint64_t sh[TOPK_THREADS];
-  __shared__ int sh_best[TOPK_THREADS];
-  const int tid = threadIdx.x;
-  pdl_wait();
-  pdl_trigger();
-  uint64_t key = (tid < a.N) ? make_key(a.J[tid], (uint32_t)tid) : KEY_MAX;
-  int n_sort = 32;
-  while (n_sort < a.N) n_sort <<= 1;
-  key = block_bitonic_sort(key, sh, n_sort);
-  if (tid < a.k) {
-    sh_best[tid] = (int)(key & 0xffffffffu);
-    if (a.elite_idx_out != nullptr) a.elite_idx_out[tid] = sh_best[tid];
-  }
-  __syncthreads();
-  for (int t = tid; t < a.H; t += blockDim.x) {
-    const float* row = a.Q + (size_t)t * a.N;
-    float acc = 0.0f;
-    for (int e = 0; e < a.k; ++e) acc += row[sh_best[e]];
-    const float new_mu = acc / (float)a.k;
-    float var = 0.0f;
-    for (int e = 0; e < a.k; ++e) {
-      const float q = row[sh_best[e]];
-      const float d = q - new_mu;
-      var = fmaf(d, d, var);
-      if (a.Q_carry != nullptr) a.Q_carry[(size_t)t * a.N + e] = q;
-    }
-    const float new_sd = sqrtf(var / (float)a.k);
-    if (!a.last) {
-      a.mu[t] = new_mu;
-      a.sd[t] = new_sd;
-    } else {
-      const float sdc = fminf(fmaxf(new_sd, a.sd_min), 10.0f);  // naive :103 / bharadhwaj :139
-      if (t > 0) {
-        a.mu[t - 1] = new_mu;
-        a.sd[t - 1] = sdc;
-      } else {
-        const float u = a.u_from_mean ? new_mu : row[sh_best[0]];
-        if (!a.freeze_prev) a.u_prev[0] = u;
-        if (a.u_out != nullptr) a.u_out[0] = u;
-        if (a.host.p != nullptr) { host_put(a.host, 5, 0.0f); host_put(a.host, 4, u); }
-      }
-    }
-  }
-  if (a.last) {
-    __syncthreads();  // column H-1 is written by the thread of column H (none) -> fill after every shifted store is issued
-    if (tid == 0) {
-      a.mu[a.H - 1] = a.mid;
-      a.sd[a.H - 1] = a.sd_init;
-    }
-  }
 }
 
 }  // namespace ctk

@@ -68,14 +68,10 @@ cudaError_t launch_env_mppi(int env, bool log, const EnvMppiArgs& a, cudaStream_
 cudaError_t launch_env_cem_rollout(int env, bool log, const EnvCemArgs& a, cudaStream_t st);
 cudaError_t launch_env_cem_refit(const EnvCemRefitArgs& a, cudaStream_t st);
 void env_dims(int env, int* ns, int* nu);
-// gradient optimizers on environments (ctk_kernels_env_rpgd.cuh): grad kernel (+ fused K8 when fused_select != null: N <= 32),
-// K8, initial population, gradient-assisted CEM sample / refit; smem: the grad kernel's shared-memory tape at horizon H
-cudaError_t launch_env_rpgd_grad(int env, bool log, size_t smem, cudaStream_t st, const EnvRpgdGradArgs& a, const EnvRpgdSelectArgs* fused_select);
+// gradient kernel on environments (ctk_kernels_env_rpgd.cuh), + fused K8 when fused_select != null (N <= 32); smem: its shared-memory
+// tape at horizon H
+cudaError_t launch_env_rpgd_grad(int env, bool log, size_t smem, cudaStream_t st, const EnvRpgdGradArgs& a, const RpgdSelectArgs* fused_select);
 size_t env_rpgd_smem_bytes(int env, int H);
-cudaError_t launch_env_rpgd_select(int env, const EnvRpgdSelectArgs& a, cudaStream_t st);
-cudaError_t launch_env_rpgd_init(int env, const EnvRpgdSelectArgs& a, cudaStream_t st);
-cudaError_t launch_env_gradcem_sample(int env, const EnvGradCemSampleArgs& a, cudaStream_t st);
-cudaError_t launch_env_gradcem_refit(int env, const EnvGradCemRefitArgs& a, cudaStream_t st);
 // recurrent predictor (ctk_gru.cu)
 cudaError_t launch_mppi_rollout_gru(int kind, bool log, int nblocks, int block, size_t smem, cudaStream_t st, const MppiArgs& a);
 cudaError_t launch_cem_rollout_gru(int kind, bool log, int nblocks, size_t smem, cudaStream_t st, const CemArgs& a);
@@ -96,10 +92,12 @@ cudaError_t launch_cem_refit(const CemRefitArgs& a, cudaStream_t st);
 // fused_select != null (coef only, one block): the select / resample step (K8) runs at the end of the same launch
 cudaError_t launch_rpgd_grad(int kind, bool log, bool coef, int nblocks, int block, size_t smem, cudaStream_t st, const RpgdGradArgs& a,
                              const RpgdSelectArgs* fused_select = nullptr);
-cudaError_t launch_rpgd_select(const RpgdSelectArgs& a, cudaStream_t st);
-cudaError_t launch_rpgd_init(const RpgdSelectArgs& a, cudaStream_t st);
-cudaError_t launch_gradcem_sample(const GradCemSampleArgs& a, cudaStream_t st);
-cudaError_t launch_gradcem_refit(const GradCemRefitArgs& a, cudaStream_t st);
+// population steps of every gradient optimizer over nu control inputs (ctk_kernels_rpgd_select.cuh): K8, initial population,
+// gradient-assisted CEM sample / refit; nu outside {1, 2} -> cudaErrorInvalidValue
+cudaError_t launch_rpgd_select(int nu, const RpgdSelectArgs& a, cudaStream_t st);
+cudaError_t launch_rpgd_init(int nu, const RpgdSelectArgs& a, cudaStream_t st);
+cudaError_t launch_gradcem_sample(int nu, const GradCemSampleArgs& a, cudaStream_t st);
+cudaError_t launch_gradcem_refit(int nu, const GradCemRefitArgs& a, cudaStream_t st);
 
 // ODE -> OdePred, GRU -> the GRU kernel, every MLP engine -> MlpSimtPred (one rollout: no tile to fill)
 cudaError_t launch_single_rollout(PredKind pred, const float* s0, const float* Q, int H, const DevConsts* kc, const MlpDev& mlp, const float* u_prev, float* traj, float* summed, cudaStream_t st);

@@ -1,4 +1,5 @@
-// ctk_rpgd.cu -- translation unit owning the RPGD kernels (K6/K7 grad steps, K8 select/resample, init) and utilities.
+// ctk_rpgd.cu -- translation unit owning the CartPole RPGD gradient kernels (K6/K7), the population steps every environment shares
+// (K8 select / resample, init, grad-CEM sample / refit) and utilities.
 #include "ctk_kernels_rpgd.cuh"
 #include "ctk_launch.h"
 
@@ -26,19 +27,24 @@ cudaError_t launch_rpgd_grad(int kind, bool log, bool coef, int nblocks, int blo
   }
   return launch_pdl(k, dim3(nblocks), dim3(block), smem, st, a);
 }
-cudaError_t launch_rpgd_select(const RpgdSelectArgs& a, cudaStream_t st) {
-  return launch_pdl(rpgd_select_kernel, dim3(1), dim3(TOPK_THREADS), 0, st, a);
-}
-cudaError_t launch_rpgd_init(const RpgdSelectArgs& a, cudaStream_t st) {
-  rpgd_init_kernel<<<(a.N * a.H + 255) / 256, 256, 0, st>>>(a);
-  return cudaGetLastError();
-}
 
-cudaError_t launch_gradcem_sample(const GradCemSampleArgs& a, cudaStream_t st) {
-  return launch_pdl(gradcem_sample_kernel, dim3((a.cnt * a.H + 255) / 256), dim3(256), 0, st, a);
+// the population steps are instantiated for nu = 1 (the CartPole) and nu = 2 (the Dubins car)
+template <class A>
+static cudaError_t launch_nu(int nu, void (*k1)(A), void (*k2)(A), unsigned grid, unsigned block, cudaStream_t st, const A& a) {
+  if (nu != 1 && nu != 2) return cudaErrorInvalidValue;
+  return launch_pdl(nu == 1 ? k1 : k2, dim3(grid), dim3(block), 0, st, a);
 }
-cudaError_t launch_gradcem_refit(const GradCemRefitArgs& a, cudaStream_t st) {
-  return launch_pdl(gradcem_refit_kernel, dim3(1), dim3(TOPK_THREADS), 0, st, a);
+cudaError_t launch_rpgd_select(int nu, const RpgdSelectArgs& a, cudaStream_t st) {
+  return launch_nu(nu, rpgd_select_kernel<1>, rpgd_select_kernel<2>, 1, TOPK_THREADS, st, a);
+}
+cudaError_t launch_rpgd_init(int nu, const RpgdSelectArgs& a, cudaStream_t st) {
+  return launch_nu(nu, rpgd_init_kernel<1>, rpgd_init_kernel<2>, (a.N * a.H * nu + 255) / 256, 256, st, a);
+}
+cudaError_t launch_gradcem_sample(int nu, const GradCemSampleArgs& a, cudaStream_t st) {
+  return launch_nu(nu, gradcem_sample_kernel<1>, gradcem_sample_kernel<2>, (a.cnt * a.H * nu + 255) / 256, 256, st, a);
+}
+cudaError_t launch_gradcem_refit(int nu, const GradCemRefitArgs& a, cudaStream_t st) {
+  return launch_nu(nu, gradcem_refit_kernel<1>, gradcem_refit_kernel<2>, 1, TOPK_THREADS, st, a);
 }
 
 // FP32 FMA-chain microbenchmark: 8 independent chains per thread, 16x unrolled

@@ -250,11 +250,11 @@ def test_gradcem_oracles_nu2_refit_per_column(cls):
 # ---- machine code of the shipped gradient kernel ---------------------------------------------------------------------------
 LIB = os.path.join(REPO, "control_toolkit_b200", "libctk_b200.so")
 CUOBJDUMP = shutil.which("cuobjdump") or "/usr/local/cuda/bin/cuobjdump"
-KERNEL = "_ZN3ctk20env_rpgd_grad_kernelINS_9DubinsEnvELb0EEEvNS_15EnvRpgdGradArgsENS_17EnvRpgdSelectArgsEi"
+KERNEL = "_ZN3ctk20env_rpgd_grad_kernelINS_9DubinsEnvELb0EEEvNS_15EnvRpgdGradArgsENS_14RpgdSelectArgsEi"
 
 
 @pytest.mark.skipif(not (os.path.exists(LIB) and os.path.exists(CUOBJDUMP)), reason="needs the built library and cuobjdump")
-def test_env_gradient_kernel_has_no_spill_and_no_local_memory_traffic_but_the_trig_slow_path():
+def test_env_gradient_kernel_spills_nothing_and_uses_local_memory_only_in_the_trig_slow_path():
     """Nothing spills.  The only local memory of the kernel is the argument-reduction buffer of the slow path of sincosf / cosf / sinf
     (|yaw| > 105615, never taken: the yaw is wrapped to (-pi, pi]) -- the same 32-byte frame the env MPPI / CEM rollout kernels
     have from the same DubinsEnv::step.  Every LDL / STL must therefore belong to such a reduction: it follows a load of the 2/pi
